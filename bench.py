@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the scoring hot path of DeepRecommendation on B200, measured per BASELINE.json.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload all|attention|graph|basic]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload all|attention|graph|basic] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Prints ONE JSON line (rank 0).  Headline = BASELINE.json configs[1]: AttentionNCF scoring on the MovieLens-latest-small
@@ -136,9 +136,10 @@ def _max_over_ranks(dist, ms, dev):
     return float(t.item())
 
 
-def timed_steps(step_fn, steps, warmup, dist, dev):
+def timed_steps(step_fn, steps, warmup, dist, dev, keep=None):
     """W untimed steps, then exactly K steps between CUDA events on the launching stream, barrier + synchronize on both
-    sides, max over ranks.  Returns (ms_total, launches)."""
+    sides, max over ranks.  Returns (ms_total, launches).  `keep`, a list, receives host copies of what step_fn returned
+    in the last timed step (a tensor or a list / tuple of tensors), taken after the timed region."""
     from deeprecommendation_b200 import ops
     for i in range(warmup):
         step_fn(i)
@@ -146,11 +147,15 @@ def timed_steps(step_fn, steps, warmup, dist, dev):
     l0 = ops.launch_count()
     a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     a.record()
+    out = None
     for i in range(steps):
-        step_fn(warmup + i)
+        out = step_fn(warmup + i)
     b.record()
     _barrier(dist)
-    return _max_over_ranks(dist, a.elapsed_time(b), dev), ops.launch_count() - l0
+    launches = ops.launch_count() - l0
+    if keep is not None:
+        keep.extend(t.detach().cpu() for t in (out if isinstance(out, (list, tuple)) else [out]))
+    return _max_over_ranks(dist, a.elapsed_time(b), dev), launches
 
 
 def op_breakdown(step_fn, steps, start_index):
@@ -261,12 +266,10 @@ def run_attention(w, steps, warmup, dist, dev, peaks):
     def step(i):
         # ONE timed step = all `nb` rotating batches (nb x 512 pairs, ~105 MB of inputs each: the working set of a step is far
         # larger than L2, and K steps make a timed region of tens of milliseconds)
-        out = None
-        for k in range(nb):
-            out = step_eager(k) if graphs is None else graphs[k].replay()
-        return out
+        return [step_eager(k) if graphs is None else graphs[k].replay() for k in range(nb)]
 
-    ms, launches = timed_steps(step, steps, warmup, dist, dev)
+    dump = [] if w.get('dump') else None
+    ms, launches = timed_steps(step, steps, warmup, dist, dev, dump)
     if graphs is not None:                                   # replays do not pass through the launch counter
         resident = [tuple(g.static_in) for g in graphs]
         l0 = ops.launch_count()
@@ -517,7 +520,7 @@ def run_attention(w, steps, warmup, dist, dev, peaks):
     if len(roofs) > 1:
         roof['other_kernels'] = roofs[1:]
     return dict(ms=ms, launches=launches, e2e_ms=e2e_ms, h2d=h2d, d2h=BATCH * 4 * nb, roofline=roof, I_mean=I_mean, out0=out0, nb=nb,
-                nnz_mean=float(np.mean(w['nnz'])), e2e_res=e2e_res, e2e_ids=e2e_ids, train=train, serving=serving,
+                nnz_mean=float(np.mean(w['nnz'])), e2e_res=e2e_res, e2e_ids=e2e_ids, train=train, serving=serving, dump=dump,
                 launch_mode='cuda_graph' if graphs is not None else 'eager: ' + w.get('graph_capture_error', 'requested'))
 
 
@@ -665,7 +668,8 @@ def run_graph(w, steps, warmup, dist, dev, peaks):
             return step_eager(i)
         return graphed(*ids[i % len(ids)])
 
-    ms, launches = timed_steps(step, steps, warmup, dist, dev)
+    dump = [] if w.get('dump') else None
+    ms, launches = timed_steps(step, steps, warmup, dist, dev, dump)
     if graphed is not None:                                  # replays do not pass through the launch counter
         l0 = __import__('deeprecommendation_b200.ops', fromlist=['x']).launch_count()
         step_eager(0)
@@ -750,7 +754,7 @@ def run_graph(w, steps, warmup, dist, dev, peaks):
             roof['fp32_view'] = {'algorithmic_flops': int(flops), 'peak': fp32, 'unit': 'TFLOP/s', 'roofline_ms': round(t_fp32, 4),
                                  'frac': round(t_fp32 / kms, 4), 'what': 'cuBLAS fp32 SIMT rate of this GPU (profiles/tf32_peak.json); the kernel itself '
                                  'is bound by the L1 data path (ncu l1tex 81 %), see DESIGN.md'}
-    return dict(ms=ms, launches=launches, e2e_ms=e2e_ms, h2d=2 * BATCH * 8, d2h=BATCH * 4, roofline=roof, train=train, trace=trace,
+    return dict(ms=ms, launches=launches, e2e_ms=e2e_ms, h2d=2 * BATCH * 8, d2h=BATCH * 4, roofline=roof, train=train, trace=trace, dump=dump,
                 launch_mode='cuda_graph' if graphed is not None else 'eager: ' + w.get('graph_capture_error', 'requested'))
 
 
@@ -968,7 +972,9 @@ def run_basic(w, steps, warmup, dist, dev, peaks):
             out = step_eager(k) if graphed is None else graphed(*resident[k])
         return out
 
-    ms, launches = timed_steps(step, steps, warmup, dist, dev)
+    # the captured forward overwrites its one output buffer per batch: a step leaves the scores of its last batch
+    dump = [] if w.get('dump') else None
+    ms, launches = timed_steps(step, steps, warmup, dist, dev, dump)
     if graphed is not None:
         l0 = ops.launch_count()
         step_eager(0)
@@ -1089,7 +1095,7 @@ def run_basic(w, steps, warmup, dist, dev, peaks):
             'peak': peaks['hbm_gbs'], 'unit': 'GB/s', 'frac': round(achieved / peaks['hbm_gbs'], 4), 'traffic': _traffic('basic'),
             'peak_source': peaks['src'], 'kernel_ms': round(kms, 4), 'algorithmic_bytes': int(alg_bytes),
             'op_ms_per_step': {f'{n}{list(m)}': round(v[0] * v[1], 4) for (n, m), v in sorted(ops_ms.items(), key=lambda kv: -kv[1][0] * kv[1][1])}}
-    return dict(ms=ms, launches=launches, e2e_ms=e2e_ms, h2d=2 * BATCH * F * 4 * nb, d2h=BATCH * 4 * nb, roofline=roof, train_ms=train_ms, train_mode=train_mode, out0=out0, nb=nb, res_legs=res_legs,
+    return dict(ms=ms, launches=launches, e2e_ms=e2e_ms, h2d=2 * BATCH * F * 4 * nb, d2h=BATCH * 4 * nb, roofline=roof, train_ms=train_ms, train_mode=train_mode, out0=out0, nb=nb, res_legs=res_legs, dump=dump,
                 launch_mode='cuda_graph' if graphed is not None else 'eager: ' + w.get('graph_capture_error', 'requested'))
 
 
@@ -1157,7 +1163,8 @@ def run_allpairs(w, steps, warmup, dist, dev, peaks, precision='fp32'):
     def step(i):
         return model.recommend(users[i % 2], items, k=AP_K, precision=precision)
 
-    ms, launches = timed_steps(step, steps, warmup, dist, dev)
+    dump = [] if w.get('dump') else None
+    ms, launches = timed_steps(step, steps, warmup, dist, dev, dump)
 
     def step_e2e(i):
         xu = w['users_host'][i % 2].to(dev, non_blocking=True)
@@ -1187,7 +1194,7 @@ def run_allpairs(w, steps, warmup, dist, dev, peaks, precision='fp32'):
             'traffic': _traffic('allpairs'), 'peak_source': peaks['src'] + ' bf16_tflops (burst: kernel timed alone)', 'kernel_ms': round(kms, 4),
             'algorithmic_flops': int(flop),
             'op_ms_per_step': {f'{n}{list(m)}': round(v[0] * v[1], 4) for (n, m), v in sorted(ops_ms.items(), key=lambda kv: -kv[1][0] * kv[1][1])}}
-    return dict(ms=ms, launches=launches, e2e_ms=e2e_ms, h2d=AP_USERS * F * 4, d2h=AP_USERS * AP_K * 12, roofline=roof, pairs=pairs)
+    return dict(ms=ms, launches=launches, e2e_ms=e2e_ms, h2d=AP_USERS * F * 4, d2h=AP_USERS * AP_K * 12, roofline=roof, pairs=pairs, dump=dump)
 
 
 def cpu_allpairs(w, n_users=16, n_items=2000):
@@ -1629,9 +1636,11 @@ PARALLELISM = {
 
 
 def graph_leg(args, dev, rank, world, dist, peaks):
-    """GraphNCF propagation, BASELINE configs[2] (strong scaling).  Returns (entry, compact scaling summary)."""
+    """GraphNCF propagation, BASELINE configs[2] (strong scaling).  Returns (entry, compact scaling summary, {name: outputs of the
+    last timed step} for --dump-outputs)."""
     w = build_graph(dev, args.graph_scale, 1, args.graph_scheme)
     w['eager'] = args.eager
+    w['dump'] = bool(args.dump_outputs)
     single_ms = None
     if world > 1:
         # the 1-GPU step of the SAME graph in the SAME job, BEFORE the graph is partitioned: every rank holds the whole graph and times the
@@ -1656,6 +1665,7 @@ def graph_leg(args, dev, rank, world, dist, peaks):
              'roofline': r['roofline'],
              'e2e': {'value': msgs / (r['e2e_ms'] * 1e-3), 'unit': 'edges/s', 'h2d_bytes_per_step': r['h2d'], 'd2h_bytes_per_step': r['d2h']},
              'gpu_launches': r['launches']}
+    outputs = {'graph_scores': r['dump'][0]} if r['dump'] else {}
     if r.get('trace'):
         traces = [None] * world
         if dist is not None:
@@ -1679,6 +1689,8 @@ def graph_leg(args, dev, rank, world, dist, peaks):
             n_steps = max(3, args.steps // 2)
             rb = run_graph(w, n_steps, 3, dist, dev, peaks)
             bf16_ms = rb['ms'] / n_steps
+            if rb['dump']:
+                outputs['graph_bf16_scores'] = rb['dump'][0]
             entry['bf16_mode'] = {'value': 2.0 * w['E'] * w['L'] * n_steps / (rb['ms'] * 1e-3), 'ms_per_step': rb['ms'] / n_steps, 'steps': n_steps,
                                   'dtype': 'bf16 messages, fp32 accumulate', 'roofline': rb['roofline'],
                                   'e2e': {'value': 2.0 * w['E'] * w['L'] * n_steps / (rb['e2e_ms'] * 1e-3), 'unit': 'edges/s',
@@ -1700,18 +1712,35 @@ def graph_leg(args, dev, rank, world, dist, peaks):
     if bf16_ms:
         scaling['bf16_messages'] = {'ms_per_step': round(bf16_ms, 4), 'value': 2.0 * w['E'] * w['L'] / (bf16_ms * 1e-3)}
     entry['speedup_vs_1gpu'] = scaling['speedup_vs_1gpu']
-    return entry, scaling
+    return entry, scaling, outputs
 
 
 ATT_WORKLOAD = ('configs[1]: AttentionNCF scoring, synthetic MovieLens-latest-small shape (610 users, 9724 items, 100836 ratings, '
                 'F=2094 profiles, 128/128/128 + MLP [256,128]), batches of 512 pairs through forward(candidate_items, rated_items, '
                 'user_matrix)')
 
+DUMP_LIMIT = 64 << 20
+
+
+def write_outputs(path, outputs):
+    """--dump-outputs: one DIR/<name>.npy per array; float32 (float64 where the source is float64 or an integer array, which
+    float64 holds exactly below 2^53)"""
+    arrays = {k: (v.float() if v.is_floating_point() and v.element_size() <= 4 else v.double()).numpy() for k, v in outputs.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f'--dump-outputs: {total} bytes of outputs, more than the {DUMP_LIMIT} allowed')
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + '.npy'), a)
+
 
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=20)
+    ap.add_argument('--steps', type=int, default=20,
+                    help='timed steps K of the headline (attention), basic, graph and sparse legs; the other timed legs run a count derived from '
+                         'K: allpairs max(3, K/4), graph bf16 mode max(3, K/2), attention '
+                         'train max(3, K/2), graph train max(3, K/4), basic train 4K single batches, graph5 max(3, min(K, 10))')
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--workload', default='all', choices=['all', 'attention', 'graph', 'basic', 'allpairs', 'k3hbm', 'k2hbm', 'graph5', 'allpairs_full', 'sparse'])
@@ -1728,7 +1757,14 @@ def main():
                          "memory (deeprecommendation_b200/peer.py); 'reduce' / 'gather' = the same partitions with NCCL collectives issued "
                          "from Python (deeprecommendation_b200/parallel.py), kept as the comparison baseline")
     ap.add_argument('--eager', action='store_true', help='do not capture the steps into CUDA graphs')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the attention, basic, allpairs and graph legs returned in their last timed step '
+                         'as DIR/<name>.npy (float32, integer arrays as float64): all batches of an attention step, the last batch of a basic '
+                         'step (its captured forward reuses one output buffer per batch), the top-k of an allpairs step, the scores of a graph '
+                         'step; the inputs are seeded, so two builds can be compared')
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != 'b200' or args.workload not in ('all', 'attention', 'basic', 'allpairs', 'graph')):
+        ap.error('--dump-outputs covers the attention, basic, allpairs and graph legs of --impl b200')
     args.warmup = max(args.warmup, 3) if args.impl == 'b200' else args.warmup
 
     if args.impl == 'reference':
@@ -1750,7 +1786,7 @@ def main():
         dist_mod.init_process_group('nccl', device_id=dev)
         dist = dist_mod
     peaks = _peaks()
-    result, also = None, []
+    result, also, outputs = None, [], {}
     from deeprecommendation_b200 import ops as _ops
     _ops.set_gemm_engine(args.gemm)
 
@@ -1760,7 +1796,10 @@ def main():
             w['gemm'] = args.gemm
             w['no_train'] = world > 1 or args.no_train_step              # the train-step leg is single-GPU (no gradient all-reduce: out of scope, SURVEY.md §8e)
             w['eager'] = args.eager
+            w['dump'] = bool(args.dump_outputs)
             r = run_attention(w, args.steps, args.warmup, dist, dev, peaks)
+            if r['dump']:
+                outputs['attention_scores'] = torch.stack(r['dump'])        # (batches per step, 512, 1)
             pairs = BATCH * r['nb'] * args.steps * world
             result = {'metric': 'scored user-item pairs/sec (NCF fwd)', 'value': pairs / (r['ms'] * 1e-3), 'unit': 'pairs/s',
                       'n_gpus': world, 'steps': args.steps, 'warmup': args.warmup, 'ms_per_step': r['ms'] / args.steps,
@@ -1818,7 +1857,10 @@ def main():
         if args.workload in ('all', 'basic'):
             w = build_basic(dev, rank)
             w['eager'] = args.eager
+            w['dump'] = bool(args.dump_outputs)
             r = run_basic(w, args.steps, args.warmup, dist, dev, peaks)
+            if r['dump']:
+                outputs['basic_scores'] = r['dump'][0]
             pairs = BATCH * r['nb'] * args.steps * world
             entry = {'metric': 'scored user-item pairs/sec (BasicNCF fwd)', 'value': pairs / (r['ms'] * 1e-3), 'unit': 'pairs/s',
                      'ms_per_step': r['ms'] / args.steps, 'scaling': 'weak', 'dtype': 'f32',
@@ -1855,9 +1897,12 @@ def main():
             torch.cuda.empty_cache()
         if args.workload in ('all', 'allpairs'):
             w = build_allpairs(dev, rank)
+            w['dump'] = bool(args.dump_outputs)
             entry = None
             for precision in ('fp32', 'bf16'):
                 r = run_allpairs(w, max(3, args.steps // 4), 3, dist, dev, peaks, precision)
+                if r['dump']:
+                    outputs[f'allpairs_{precision}_topk_scores'], outputs[f'allpairs_{precision}_topk_items'] = r['dump']
                 n_steps = max(3, args.steps // 4)
                 e = {'metric': f'scored user-item pairs/sec (BasicNCF all-pairs + top-{AP_K})', 'value': r['pairs'] * n_steps * world / (r['ms'] * 1e-3),
                      'unit': 'pairs/s', 'ms_per_step': r['ms'] / n_steps, 'steps': n_steps, 'scaling': 'weak',
@@ -1915,7 +1960,8 @@ def main():
     graph_scaling = None
     if args.workload in ('all', 'graph'):                  # LAST, so that the tail of the line carries the strong-scaling leg
         with ClockSampler(local) as gclocks:
-            entry, graph_scaling = graph_leg(args, dev, rank, world, dist, peaks)
+            entry, graph_scaling, graph_outputs = graph_leg(args, dev, rank, world, dist, peaks)
+        outputs.update(graph_outputs)
         if args.workload == 'graph':
             clocks = gclocks
         else:
@@ -1938,6 +1984,8 @@ def main():
         result['also'] = also
     if graph_scaling is not None:
         result['graph_scaling'] = graph_scaling            # compact copy of the strong-scaling leg at the very end of the line
+    if rank == 0 and args.dump_outputs:
+        write_outputs(args.dump_outputs, outputs)
     if rank == 0:
         print(json.dumps(result), flush=True)
     if dist is not None:

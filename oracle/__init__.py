@@ -8,9 +8,9 @@ loudly when the CUDA library is missing instead of falling back to anything here
 Contents
   restatement.py   torch-CPU / numpy restatement of the reference algorithm, function by function,
                    each citing the reference file:line it follows.  Travels to the GPU box.
-  ref_loader.py    imports the UNMODIFIED reference modules from /root/reference/src (this container
-                   only; the GPU box has no /root/reference) with `pyg_shim/` standing in for the
-                   uninstallable torch_geometric 2.0.4.
+  ref_loader.py    imports the UNMODIFIED reference modules from the src/ of a checkout of the original
+                   project named by B200REC_REFERENCE_ROOT (not part of this repository) with `pyg_shim/`
+                   standing in for the uninstallable torch_geometric 2.0.4.
   pyg_shim/        restatement of the five PyG symbols the reference touches.
   make_golden.py   runs the real reference (through ref_loader) on seeded synthetic inputs and writes
                    the fixtures under tests/golden/.  Committed together with the fixtures.

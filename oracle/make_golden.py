@@ -1,7 +1,7 @@
 """Generate tests/golden/*.npz by running the UNMODIFIED reference (container only).
 
 TEST INFRASTRUCTURE (oracle/__init__.py).  Usage:  python -m oracle.make_golden
-Requires /root/reference.  The reference ships no golden vectors of its own (SURVEY.md §4), so these
+Requires a checkout of the original project (B200REC_REFERENCE_ROOT).  The reference ships no golden vectors of its own (SURVEY.md §4), so these
 fixtures — outputs of the reference's own classes on seeded inputs — are what pins the restatement
 (oracle/restatement.py) and, through it, the CUDA path.  GraphNCF cases execute the reference's
 gnn_ncf.py on top of oracle/pyg_shim (PyG 2.0.4 itself is not installable): "parity unpinned" at that

@@ -1,24 +1,24 @@
-"""Import the UNMODIFIED reference modules (container only).  TEST INFRASTRUCTURE (oracle/__init__.py).
+"""Import the UNMODIFIED reference modules.  TEST INFRASTRUCTURE (oracle/__init__.py).
 
-`/root/reference` is read-only and absent on the GPU box: only `make_golden.py` and the
-`-m "not gpu"` tests that are explicitly skipped when the directory is missing use this.
+The reference (the original DeepRecommendation project) is not part of this repository: B200REC_REFERENCE_ROOT names a
+checkout of it.  Only `make_golden.py` and the tests marked `reference` use this; those tests skip when it is not set.
 """
 import importlib
 import os
 import sys
 
-REFERENCE_ROOT = os.environ.get('B200REC_REFERENCE_ROOT', '/root/reference')
+REFERENCE_ROOT = os.environ.get('B200REC_REFERENCE_ROOT', '')
 _SRC = os.path.join(REFERENCE_ROOT, 'src')
 _SHIM = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'pyg_shim')
 
 
 def available() -> bool:
-    return os.path.isdir(os.path.join(_SRC, 'neural_collaborative_filtering'))
+    return bool(REFERENCE_ROOT) and os.path.isdir(os.path.join(_SRC, 'neural_collaborative_filtering'))
 
 
 def _ensure_path():
     if not available():
-        raise RuntimeError(f'reference not found under {REFERENCE_ROOT}')
+        raise RuntimeError(f'reference not found: set B200REC_REFERENCE_ROOT to a checkout of the original project (now {REFERENCE_ROOT!r})')
     try:
         import torch_geometric  # noqa: F401  (a real install wins over the shim)
     except ImportError:

@@ -10,7 +10,7 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line('markers', 'gpu: needs a CUDA device (B200); run with -m gpu on the GPU box')
-    config.addinivalue_line('markers', 'reference: needs /root/reference (container only); skipped when absent')
+    config.addinivalue_line('markers', 'reference: needs a checkout of the original project named by B200REC_REFERENCE_ROOT; skipped without it')
 
 
 def pytest_collection_modifyitems(config, items):

@@ -1,6 +1,6 @@
 """The oracle's restatement vs golden outputs of the UNMODIFIED reference (CPU; no GPU needed).
 
-tests/golden/*.npz were produced by oracle/make_golden.py running /root/reference's own classes.
+tests/golden/*.npz were produced by oracle/make_golden.py running the original project's own classes.
 A restatement that disagrees with them is not an oracle.
 """
 import numpy as np
@@ -150,7 +150,7 @@ def test_csr_by_destination_is_stable():
 
 
 @pytest.mark.reference
-@pytest.mark.skipif(not ref_loader.available(), reason='/root/reference absent (GPU box)')
+@pytest.mark.skipif(not ref_loader.available(), reason='B200REC_REFERENCE_ROOT does not name a checkout of the original project')
 def test_restatement_vs_live_reference_shipped_checkpoint():
     """Shipped AttentionNCF checkpoint (real trained weights) through the live reference and the restatement."""
     import os

@@ -1,5 +1,5 @@
 import sys, os, time
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch, numpy as np
 import bench
 from torch.profiler import profile, ProfilerActivity
