@@ -2,17 +2,19 @@
 from __future__ import annotations
 
 import os
+import weakref
 
 import torch
 from torch import nn
 
 from ... import _lib as L
 from ... import ops
-from ..util import build_MLP_layers, run_mlp
+from ..util import build_MLP_layers, mlp_parameters, run_mlp
 from .base import NCF, _named_like
 
 
 _SIDE_STREAMS = {}
+RECOMMEND_SLAB_BYTES = 1 << 30      # default budget of one chunk's h1 slab in `AttentionNCF.recommend` (users per chunk = budget / (nI·H1P·4))
 
 
 def _side_stream(device):
@@ -306,3 +308,149 @@ class AttentionNCF(NCF):
         mask = att_top > thr
         return {'items': cand_rows[top], 'scores': val.view(-1),
                 'because': [rated_sorted[m] for m in mask], 'attention': [a[m] for a, m in zip(att_top, mask)]}
+
+    # ------------------------------------------------------------------------------------------------------------------
+    def _recommend_tables(self, item_profiles):
+        """Catalogue tables of `recommend`, one GEMM over the (nI, F) profiles per weight version.  The candidate and rated sides are the
+        same catalogue, and the user-embedding half of the first MLP Linear is folded into the pooled table (W1 = [W1e | W1u], item first,
+        attention_ncf.py:219; user_emb = Σ α·um·Q + b_U):
+
+            h1_pre[b] = Ai[b] + Σ_i α_bi·um_i·Q'[i],   Ai = Ec·W1eᵀ + (b1 + W1u·b_U),   Q' = Q·W1uᵀ = R·(W1u·W_U)ᵀ
+
+        so no per-pair (U x H1) GEMM is left.  Composites are formed in float64 and rounded once, like `_composite_projection`.
+        Returns (Pc, Pr, mode, a2, a20, Ai, Qp, H1) with Ai / Qp zero-padded to H1P in {32, 64, 128, 256} columns; cached on the profile
+        tensor (identity, `_version`, shape) and the parameter versions."""
+        weights, biases, _ = mlp_parameters(self.MLP)
+        if len(weights) < 2:
+            raise NotImplementedError('recommend(): the MLP needs at least one hidden layer (the kernel ends at the first hidden ReLU)')
+        H1 = weights[0].shape[0]
+        if H1 > 256:
+            raise NotImplementedError(f'recommend(): first MLP layer of width {H1} > 256 is not supported')
+        H1P = max(32, 1 << (H1 - 1).bit_length())
+        E = self.ItemEmbeddings[0].weight.shape[0]
+        if self.use_cos_sim_instead:                                   # width of the score tables K8 stages in shared memory
+            H = (E + 3) // 4 * 4
+        else:
+            H = (self.AttentionNet[0].weight.shape[0] + 3) // 4 * 4 if len(self.AttentionNet) > 1 else 4
+        if H > 256:
+            raise NotImplementedError(f'recommend(): attention width {H} > 256 is not supported')
+        params = tuple(self.parameters())
+        key = (tuple(item_profiles.shape), item_profiles._version, item_profiles.device) + tuple((p.data_ptr(), p._version) for p in params)
+        cached = getattr(self, '_rec_cache', None)
+        if cached is not None and cached[0] == key and cached[1]() is item_profiles:
+            return cached[2]
+        item, user = self.ItemEmbeddings[0], self.UserEmbeddings[0]
+        R = item_profiles if item_profiles.dtype == torch.float32 else item_profiles.float()
+        with torch.no_grad():
+            WI, bI, WU, bU = (t.detach().double() for t in (item.weight, item.bias, user.weight, user.bias))
+            W1, b1 = weights[0].detach().double(), biases[0].detach().double()
+            W1e, W1u = W1[:, :E], W1[:, E:]
+            pad = H1P - H1
+            Wa = torch.nn.functional.pad(W1e @ WI, (0, 0, 0, pad))                         # (H1P, F)
+            ba = torch.nn.functional.pad(W1e @ bI + b1 + W1u @ bU, (0, pad))
+            Wq = torch.nn.functional.pad(W1u @ WU, (0, 0, 0, pad))
+            bq = torch.zeros(H1P, dtype=torch.float64, device=Wq.device)
+            halves = self._attention_halves()
+            if halves is not None:                                                         # AttentionNet, att_dense % 4 == 0: composites
+                A1c, A1r, a1, a2, a20 = halves
+                H = A1r.shape[0]
+                A1c, A1r = A1c.double(), A1r.double()
+                W = torch.cat((Wa, A1c @ WI, A1r @ WI, Wq), 0)
+                b = torch.cat((ba, A1c @ bI + a1.double(), A1r @ bI, bq), 0)
+                T = ops.linear_raw(R, W.float().contiguous(), b.float().contiguous())
+                Ai, Pc, Pr, Qp = T[:, :H1P], T[:, H1P:H1P + H], T[:, H1P + H:H1P + 2 * H], T[:, H1P + 2 * H:]
+                mode = L.ATT_NET
+            else:                                                                          # cosine, att_dense=None, att_dense % 4 != 0
+                Ep = (E + 3) // 4 * 4
+                W = torch.cat((torch.nn.functional.pad(WI, (0, 0, 0, Ep - E)), Wa, Wq), 0)
+                b = torch.cat((torch.nn.functional.pad(bI, (0, Ep - E)), ba, bq), 0)
+                T = ops.linear_raw(R, W.float().contiguous(), b.float().contiguous())
+                Ec, Ai, Qp = T[:, :E], T[:, Ep:Ep + H1P], T[:, Ep + H1P:]
+                Pc, Pr, mode, a2, a20 = self._score_tables(Ec, Ec)
+                Pc, Pr = Pc.detach().contiguous(), Pr.detach().contiguous()
+        out = (Pc, Pr, mode, a2, a20, Ai, Qp, H1)
+        self._rec_cache = (key, weakref.ref(item_profiles), out)
+        return out
+
+    def recommend(self, item_profiles, list_ptr, list_item, list_val, k=10, users=None, ignore_seen=True, return_scores=False, chunk_users=None):
+        """Top-k catalogue items for many users at once: the reference's serving call (src/webapp/backend.py:78-121, one user x every
+        catalogue item, attention_ncf.py:136-224) batched over users.
+
+        item_profiles (nI, F) CUDA fp32 — the catalogue, every row a candidate.  The rating lists use K6's resident format (a
+        `DeviceCollateProvider` feeds it directly: `prov.table, prov.d_list_ptr, prov.d_list_item, prov.d_list_val`): list_ptr int64
+        (rows+1), list_item int32 catalogue rows ascending per user, list_val fp32 ALREADY centred (an entry of exactly 0.0 gets no
+        attention).  `users` int64 list rows (default: every row; duplicates allowed).  `ignore_seen` leaves a user's own list items out.
+        Users are processed `chunk_users` at a time (default: an h1 slab of about RECOMMEND_SLAB_BYTES): the working memory is bounded by
+        the chunk, whatever the number of users; the whole (nU, nI) score matrix is only allocated with `return_scores=True`.
+
+        Pipeline per chunk: K8 (csrc/attention_recommend.cu: attention pooling over the shared list, h1 slab) on the cached catalogue tables
+        (`_recommend_tables`), the remaining MLP layers on the slab (K1a), seen pairs set to NaN, `ops.topk_rows`.
+        Returns (top_scores (nU, k) fp32, top_items (nU, k) int64 catalogue rows, padded with (-inf, -1)[, scores (nU, nI)])."""
+        if self.training:
+            raise RuntimeError('recommend() is an inference call: model.eval() first')
+        ops._require_cuda(item_profiles, list_ptr, list_item, list_val, users)
+        if list_ptr.dtype != torch.int64 or list_item.dtype != torch.int32 or list_val.dtype != torch.float32:
+            raise ValueError('recommend(): list_ptr must be int64, list_item int32 and list_val float32')
+        if not 1 <= k <= 64:
+            raise ValueError('recommend(): need 1 <= k <= 64')
+        dev = item_profiles.device
+        nI = item_profiles.shape[0]
+        n_rows = list_ptr.numel() - 1
+        users = torch.arange(max(n_rows, 0), device=dev) if users is None else users.to(dev).long().contiguous()
+        nU = users.numel()
+        self._check_lists(list_ptr, list_item, list_val, users, nI)
+        weights, biases, _ = mlp_parameters(self.MLP)
+        with torch.no_grad():
+            Pc, Pr, mode, a2, a20, Ai, Qp, H1 = self._recommend_tables(item_profiles)
+            H1P = Ai.shape[1]
+            if chunk_users is None:
+                chunk_users = max(1, RECOMMEND_SLAB_BYTES // max(1, nI * H1P * 4))
+            chunk_users = int(max(1, min(chunk_users, 65535)))
+            val = torch.full((nU, k), float('-inf'), dtype=torch.float32, device=dev)
+            idx = torch.full((nU, k), -1, dtype=torch.int64, device=dev)
+            scores = torch.empty((nU, nI), dtype=torch.float32, device=dev) if return_scores else None
+            last = len(weights) - 1
+            for s in range(0, nU if nI > 0 else 0, chunk_users):
+                uc = users[s:s + chunk_users]
+                n = uc.numel()
+                sc = scores[s:s + n] if scores is not None else torch.empty((n, nI), dtype=torch.float32, device=dev)
+                x = ops.attention_recommend_raw(Pc, Pr, Ai, Qp, mode=mode, a2=a2, a20=a20, list_ptr=list_ptr, list_item=list_item,
+                                                list_val=list_val, users=uc)[:, :H1]
+                for li in range(1, last):
+                    x = ops.linear_raw(x, weights[li], biases[li], relu=True)
+                ops.linear_raw(x, weights[last], biases[last], out=sc.view(n * nI, 1))
+                del x
+                if ignore_seen:                                        # item_features.drop(...) (backend.py:85): never selected by the top-k
+                    self._mask_seen(sc, uc, list_ptr, list_item)
+                val[s:s + n], idx[s:s + n] = ops.topk_rows(sc, k)
+        return (val, idx, scores) if return_scores else (val, idx)
+
+    @staticmethod
+    def _check_lists(list_ptr, list_item, list_val, users, nI):
+        """Host-side range checks of the rating lists and user rows (one device read-back): K8 reads `list_ptr[users]` and the table rows
+        `list_item[...]` without bounds checks."""
+        n_rows = list_ptr.numel() - 1
+        if n_rows < 0:
+            raise ValueError('recommend(): list_ptr needs at least one element')
+        z = torch.zeros((), dtype=torch.bool, device=list_ptr.device)
+        flags = torch.stack((
+            ((users < 0) | (users >= n_rows)).any() if users.numel() else z,
+            (list_ptr[0] != 0) | (list_ptr[-1] > min(list_item.numel(), list_val.numel())) | ((list_ptr[1:] < list_ptr[:-1]).any() if n_rows else z),
+            ((list_item < 0) | (list_item >= nI)).any() if list_item.numel() else z)).tolist()
+        if flags[0]:
+            raise ValueError(f'recommend(): `users` must be list rows in [0, {n_rows})')
+        if flags[1]:
+            raise ValueError('recommend(): list_ptr must start at 0, be non-decreasing and end within list_item / list_val')
+        if flags[2]:
+            raise ValueError(f'recommend(): list_item must hold catalogue rows in [0, {nI})')
+
+    @staticmethod
+    def _mask_seen(scores, users, list_ptr, list_item):
+        """scores[r, list_item of users[r]] = NaN for every list entry of every row r"""
+        start, lens = list_ptr[users], list_ptr[users + 1] - list_ptr[users]
+        total = int(lens.sum())
+        if total:
+            dev = scores.device
+            rows = torch.repeat_interleave(torch.arange(users.numel(), device=dev), lens, output_size=total)
+            first = torch.repeat_interleave(start - (torch.cumsum(lens, 0) - lens), lens, output_size=total)
+            scores[rows, list_item[first + torch.arange(total, device=dev)].long()] = float('nan')

@@ -35,7 +35,7 @@ class NCF(nn.Module):
     # ---- derived copies of the weights (packed MMA tiles, composite / transposed matrices, cached embeddings) -----------------------
     # They are keyed on (address, tensor `_version`).  Loading a state dict, moving / casting the module, or editing parameters through
     # `.data` (which does NOT bump `_version`) must drop them: the first two are hooked here, the third is what `invalidate_caches()` is for.
-    _DERIVED = ('_proj_cache', '_comp_cache', '_att_cache', '_cache', '_peer_layer0', '_emb_cache')
+    _DERIVED = ('_proj_cache', '_comp_cache', '_att_cache', '_cache', '_peer_layer0', '_emb_cache', '_rec_cache')
 
     def invalidate_caches(self):
         from ... import ops

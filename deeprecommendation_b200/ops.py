@@ -1084,6 +1084,50 @@ def attention_pool(Pc, Pr, Q, *, mode, a2, a20, bU, user_matrix, return_attentio
 
 
 # ------------------------------------------------------------------------------------------------------------------
+# K8 whole-catalogue attention pooling (attention_ncf.py:136-224 for every catalogue item of many users, backend.py:78-121)
+# ------------------------------------------------------------------------------------------------------------------
+def _check_rows(t, what):
+    if t.dim() != 2 or t.dtype != torch.float32 or t.stride(1) != 1 or t.stride(0) % 4 or t.data_ptr() % 16:
+        raise ValueError(f'attention_recommend: {what} must be a 2-D fp32 table with unit column stride, 16-byte aligned rows')
+    return t.stride(0) if t.shape[0] > 1 else max(t.stride(0), (t.shape[1] + 3) // 4 * 4)
+
+
+def attention_recommend_raw(Pc, Pr, Ai, Qp, *, mode, a2, a20, list_ptr, list_item, list_val, users, out=None):
+    """h1 = ReLU(Ai[b] + Σ_i softmax_i(s_bi)·val_i·Qp[i]) for every (user of `users`, catalogue row b) — b200rec_attention_recommend.
+    Pc / Pr (nI, H) score tables (mode ATT_NET: s = a2·ReLU(Pc[b] + Pr[i]) + a20; ATT_DOT: s = <Pc[b], Pr[i]>); Ai / Qp (nI, H1P) with
+    H1P in {32, 64, 128, 256}; the rating lists in K6's resident format (list_ptr int64, list_item int32, list_val fp32 centred); `users`
+    int64 list rows.  Returns (len(users)·nI, H1P) fp32, row u·nI + b (or fills `out` of that shape)."""
+    _require_cuda(Pc, Pr, Ai, Qp, a2, a20, list_ptr, list_item, list_val, users, out)
+    if list_ptr.dtype != torch.int64 or users.dtype != torch.int64:
+        raise ValueError('attention_recommend: list_ptr and users must be int64')
+    if list_item.dtype != torch.int32:
+        raise ValueError('attention_recommend: list_item must be int32')
+    if list_val.dtype != torch.float32:
+        raise ValueError('attention_recommend: list_val must be float32')
+    nI, H = Pc.shape
+    H1P = Ai.shape[1]
+    if Pr.shape != (nI, H) or Ai.shape[0] != nI or Qp.shape != (nI, H1P):
+        raise ValueError('attention_recommend: table shapes disagree')
+    ld_pc, ld_pr, ld_ai, ld_q = _check_rows(Pc, 'Pc'), _check_rows(Pr, 'Pr'), _check_rows(Ai, 'Ai'), _check_rows(Qp, 'Qp')
+    list_ptr, list_item, list_val, users = list_ptr.contiguous(), list_item.contiguous(), list_val.contiguous(), users.contiguous()
+    if a2 is not None:
+        a2 = a2.detach().contiguous().float()
+    if a20 is not None:
+        a20 = a20.detach().contiguous().float()
+    nU = users.numel()
+    if out is None:
+        out = torch.empty((nU * nI, H1P), dtype=torch.float32, device=Pc.device)
+    elif out.shape != (nU * nI, H1P) or out.dtype != torch.float32 or out.stride(1) != 1:
+        raise ValueError('attention_recommend: bad `out`')
+    ldo = out.stride(0) if out.shape[0] > 1 else H1P
+    with _on(Pc.device), _timed('attention_recommend', (nU, nI, H, H1P)):
+        L.check(L.lib().b200rec_attention_recommend(_ptr(Pc), ld_pc, _ptr(Pr), ld_pr, H, int(mode), _ptr(a2), _ptr(a20), _ptr(Ai), ld_ai, _ptr(Qp), ld_q,
+                                                    H1P, nI, _ptr(list_ptr), _ptr(list_item), _ptr(list_val), _ptr(users), nU, _ptr(out), ldo,
+                                                    _stream()), 'attention_recommend')
+    return out
+
+
+# ------------------------------------------------------------------------------------------------------------------
 # top-k
 # ------------------------------------------------------------------------------------------------------------------
 def topk_rows(scores, k):

@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define B200REC_VERSION 202
+#define B200REC_VERSION 203
 
 typedef void* b200rec_stream_t; /* cudaStream_t */
 
@@ -226,6 +226,23 @@ typedef struct {
 size_t b200rec_attention_pool_workspace(int64_t B, int64_t I, int U, int dense);
 size_t b200rec_attention_pool_workspace_csr(int64_t B, int64_t I, int U, int64_t max_row_nnz, int64_t nnz);
 int b200rec_attention_pool(const b200rec_attention_t* a, b200rec_stream_t stream);
+/* ---- K8  AttentionNCF whole-catalogue recommendation: attention pooling over one shared rated list per user ------------------
+ * Replaces, for every catalogue item b as a candidate of user u, attention_ncf.py:136-224 up to the first hidden layer of the MLP — the
+ * per-user scoring loop of src/webapp/backend.py:78-121 run for many users at once (csrc/attention_recommend.cu).  With the user-embedding
+ * half of the first MLP Linear folded into the pooled table (W1 = [W1e | W1u], item first, :219):
+ *   s_bi = a2·ReLU(Pc[b] + Pr[i]) + a20 (mode NET) or <Pc[b], Pr[i]> (mode DOT);  α = softmax_i over the list entries with val != 0
+ *   (exact 0.0 = "unrated", :158,192; none -> α = 0, :208-209);  h1[u, b] = ReLU(Ai[b] + Σ_i α_bi·val_i·Qp[i])
+ *   where Ai = Ec·W1eᵀ + b1 + W1u·b_U (nI, H1P) and Qp = Q·W1uᵀ (nI, H1P), columns past H1 zero.
+ * Tables: Pc, Pr (n_items, H) fp32, H % 4 == 0, H <= 256; a2 (H) and a20 (device scalar or NULL) for mode NET.  H1P in {32, 64, 128, 256}.
+ * Rating lists (the resident format of b200rec_collate_interacted): list_ptr int64 (rows+1), list_item int32 catalogue rows, list_val fp32
+ * centred ratings.  users (n_users int64, list rows; duplicates allowed, n_users <= 65535 per call).  h1 (n_users·n_items, ld_h1 >= H1P) fp32:
+ * row u·n_items + b; b200rec_attention_recommend_workspace gives its size in bytes for ld_h1 = H1P.  All leading dimensions % 4 == 0,
+ * tables and h1 16-byte aligned.  No atomics: bit-identical results run to run. */
+size_t b200rec_attention_recommend_workspace(int64_t n_users, int64_t n_items, int H1P);
+int b200rec_attention_recommend(const float* Pc, int64_t ld_pc, const float* Pr, int64_t ld_pr, int H, int mode, const float* a2, const float* a20,
+                                const float* Ai, int64_t ld_ai, const float* Qp, int64_t ld_q, int H1P, int64_t n_items, const int64_t* list_ptr,
+                                const int32_t* list_item, const float* list_val, const int64_t* users, int64_t n_users, float* h1, int64_t ld_h1,
+                                b200rec_stream_t stream);
 /* The same op with AttentionNet's inner Dropout applied in training mode: hidden = ReLU(Pc[b] + Pr[i]) ∘ m / keep, m ~ Bernoulli(keep), keep =
  * round((1 - dropout_p)·65536) / 65536, one Philox2x32-10 call (counter = (i, b·64 + hidden group), key = seed) per 4 hidden units
  * (csrc/common.cuh).  A separately compiled copy of the kernels (csrc/attention_pool_drop.cu): the scoring build above is untouched. */
