@@ -12,7 +12,7 @@ OK, ERR_CUDA, ERR_BAD_ARG, ERR_UNSUPPORTED, ERR_WORKSPACE = 0, 1, 2, 3, 4
 F32, BF16 = 0, 1
 ATT_NET, ATT_DOT = 0, 1
 TC_TF32X3, TC_BF16, TC_BF16X3 = 0, 1, 2
-ABI_VERSION = 203          # B200REC_VERSION of include/b200rec.h these bindings were written against (checked when the library is loaded)
+ABI_VERSION = 204          # B200REC_VERSION of include/b200rec.h these bindings were written against (checked when the library is loaded)
 AP_BF16, AP_BF16X2 = 0, 1
 MLP_MAX_LAYERS = 8
 PEER_MAX, PEER_CHANNELS, PEER_HANDLE_BYTES = 16, 16, 64
@@ -31,7 +31,7 @@ class AttentionDesc(C.Structure):
                 ('B', c_i64), ('I', c_i64), ('H', c_int), ('U', c_int), ('out', c_vp), ('ldo', c_i64), ('att_weights', c_vp),
                 ('train_cand_emb', c_vp), ('train_rated_emb', c_vp), ('E', c_int), ('atol', c_f), ('rtol', c_f),
                 ('drop_zero_scores', c_int), ('score_scale', c_f), ('ld_pr', c_i64), ('ld_q', c_i64), ('workspace', c_vp), ('workspace_bytes', c_sz),
-                ('max_row_nnz', c_i64), ('nnz', c_i64), ('prepared', c_int), ('ld_pc', c_i64), ('dropout_p', c_f), ('dropout_seed', C.c_uint64), ('dropout_seed_dev', c_vp)]
+                ('max_row_nnz', c_i64), ('nnz', c_i64), ('ld_pc', c_i64), ('dropout_p', c_f), ('dropout_seed', C.c_uint64), ('dropout_seed_dev', c_vp)]
 
 
 class AttentionBwdDesc(C.Structure):
@@ -102,7 +102,6 @@ SIGNATURES = {
     'b200rec_attention_pool': (c_int, [C.POINTER(AttentionDesc), c_vp]),
     'b200rec_attention_pool_dropout': (c_int, [C.POINTER(AttentionDesc), c_vp]),
     'b200rec_attention_pool_set_path': (c_int, [c_int]),
-    'b200rec_attention_pool_prepare': (c_int, [C.POINTER(AttentionDesc), c_vp]),
     'b200rec_attention_pool_backward': (c_int, [C.POINTER(AttentionBwdDesc), c_vp]),
     'b200rec_attention_recommend_workspace': (c_sz, [c_i64, c_i64, c_int]),
     'b200rec_attention_recommend': (c_int, [c_vp, c_i64, c_vp, c_i64, c_int, c_int, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_int, c_i64, c_vp, c_vp, c_vp,

@@ -24,7 +24,6 @@
 // the reference's dense (B, I) `user_matrix` on the fly through a per-warp shared-memory queue (drop-in entry;
 // exact 0.0 means "unrated", attention_ncf.py:158,192).
 #include <math.h>
-#include <stdlib.h>
 
 #include <algorithm>
 
@@ -661,39 +660,15 @@ attention_merge_kernel(AttParams p, const int* __restrict__ row_ptr, const int* 
 // One CTA per row; pure streaming (four independent coalesced loads per thread and iteration, no dependent work), so
 // the dense scan costs a few microseconds instead of sitting on the critical path of the pooling kernel, and the
 // pooling kernel can split every row's non-zeros EVENLY over its warps.
-// STAGED: the row is first copied to shared memory with 40 independent loads per thread in flight (one memory latency per 10,240
-// columns instead of one per 128 — the two scans then run out of shared memory); rows wider than the shared memory take the
-// streaming form.
-template <bool STAGED>
+// This streaming form reads the row from global memory twice; it serves rows wider than the shared memory of um_compact_vec_kernel below.
 __global__ void __launch_bounds__(ATT_WARPS * 32)
 um_compact_kernel(const float* __restrict__ um, long long ld_um, int I, int* __restrict__ col, float* __restrict__ val,
                   int* __restrict__ row_nnz, AttWork w) {
-  extern __shared__ float um_row_smem[];
   __shared__ int s_cnt[ATT_WARPS];
   __shared__ int s_base;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int b = blockIdx.x;
-  const float* __restrict__ grow = um + (long long)b * ld_um;
-  if constexpr (STAGED) {
-    // loads are CLAMPED, not predicated: seven predicate registers cap a batch of predicated loads at ~7 in flight (SASS, round 2)
-    constexpr int NLD = 40;                                     // a 10,240-column row in ONE memory latency
-    for (int i0 = 0; i0 < I; i0 += ATT_WARPS * 32 * NLD) {
-      float v[NLD];
-#pragma unroll
-      for (int u = 0; u < NLD; ++u) {
-        const int i = i0 + u * (ATT_WARPS * 32) + (int)threadIdx.x;
-        v[u] = __ldcs(grow + min(i, I - 1));
-      }
-#pragma unroll
-      for (int u = 0; u < NLD; ++u) {
-        const int i = i0 + u * (ATT_WARPS * 32) + (int)threadIdx.x;
-        if (i < I) um_row_smem[i] = v[u];
-      }
-    }
-    __syncthreads();
-  }
-  const float* row = STAGED ? um_row_smem : grow;
-  auto ldv = [](const float* q) { if constexpr (STAGED) return *q; else return __ldg(q); };
+  const float* __restrict__ row = um + (long long)b * ld_um;
   const int chunks = (I + 31) >> 5;
   const int cpw = (chunks + ATT_WARPS - 1) / ATT_WARPS;
   const int i_begin = warp * cpw * 32, i_end = min(I, i_begin + cpw * 32);
@@ -703,7 +678,7 @@ um_compact_kernel(const float* __restrict__ um, long long ld_um, int I, int* __r
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
       const int i = i0 + u * 32 + lane;
-      v[u] = (i < i_end) ? ldv(row + i) : 0.f;
+      v[u] = (i < i_end) ? __ldg(row + i) : 0.f;
     }
 #pragma unroll
     for (int u = 0; u < 4; ++u) cnt += __popc(__ballot_sync(FULL, v[u] != 0.f));
@@ -724,7 +699,7 @@ um_compact_kernel(const float* __restrict__ um, long long ld_um, int I, int* __r
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
       const int i = i0 + u * 32 + lane;
-      v[u] = (i < i_end) ? ldv(row + i) : 0.f;
+      v[u] = (i < i_end) ? __ldg(row + i) : 0.f;
     }
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
@@ -740,7 +715,7 @@ um_compact_kernel(const float* __restrict__ um, long long ld_um, int I, int* __r
   }
 }
 
-// The staged form of the compaction with 128-bit accesses (round 2: the scalar form above issued ~1,700 instructions per warp and row —
+// The compaction staged through shared memory with 128-bit accesses (round 2: the scalar form above issued ~1,700 instructions per warp and row —
 // 60 % issue-slot utilisation, 14 us for the 19 MB matrix of config 2).  A row starts on a 4-byte boundary only, so it is staged into shared
 // memory SHIFTED by its phase (`shift` = words past a 16-byte boundary): padded element e = column e - shift, elements [0, shift) and the tail
 // pad are zeros and drop out of the compaction like any other zero.  Interior vectors move as LDG.128 -> STS.128 (all of a thread's loads in
@@ -884,8 +859,6 @@ struct AttInputs {
   void* ws; size_t ws_bytes;
   long long max_row_nnz;     // CSR form: upper bound of a row's length (0 = unknown -> I); sizes the work list and the partial slots
   long long nnz;             // CSR form: number of stored entries (0 = unknown); tightens the same bound
-  int prepare_light;         // prepare on a side stream: the compaction kernel without dynamic shared memory (co-resident with the GEMM CTAs)
-  int prepared;              // the work list (and the compaction of a dense matrix) is already in the workspace (b200rec_attention_pool_prepare)
 };
 
 static size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
@@ -914,9 +887,8 @@ static AttLayout att_layout(long long B, long long I, int U, bool dense, long lo
 struct AttLists { const int* col; const float* val; const int* row_nnz; const int* row_ptr; long long stride; };
 
 // First phase of the segment-parallel path: zero the counter, compact a dense matrix (or read the CSR's row lengths) and write
-// the work list.  It depends on `user_matrix` only — not on the projections — so the host may run it on a second stream next
-// to the GEMMs (b200rec_attention_pool_prepare; `launch` = false just recomputes the pointers into an already prepared workspace).
-static int att_prepare(int B, int I, int U, const AttInputs& in, cudaStream_t st, bool launch, AttWork& w, AttLists& lists) {
+// the work list.
+static int att_prepare(int B, int I, int U, const AttInputs& in, cudaStream_t st, AttWork& w, AttLists& lists) {
   const bool dense = in.um != nullptr;
   const AttLayout lay = att_layout(B, I, U, dense, in.max_row_nnz, in.nnz);
   unsigned char* ws = reinterpret_cast<unsigned char*>(in.ws);
@@ -928,26 +900,23 @@ static int att_prepare(int B, int I, int U, const AttInputs& in, cudaStream_t st
   const long long max_items = att_max_items(B, I, dense ? 0 : in.max_row_nnz, dense ? 0 : in.nnz);
   if (max_items > 0x7fffffffLL) return b200rec_fail(B200REC_ERR_UNSUPPORTED, "attention_pool: more than 2^31 segments");
   w.max_items = (int)max_items;
-  if (launch) B200REC_CUDA(cudaMemsetAsync(w.counter, 0, 2 * sizeof(int), st));
+  B200REC_CUDA(cudaMemsetAsync(w.counter, 0, 2 * sizeof(int), st));
   lists.col = in.col; lists.val = in.val; lists.row_nnz = nullptr; lists.row_ptr = in.row_ptr; lists.stride = 0;
   if (dense) {                         // streaming compaction of the dense matrix into row-padded lists (+ the work list)
     int* wcol = reinterpret_cast<int*>(ws + lay.compact);
     float* wval = reinterpret_cast<float*>(wcol + (size_t)B * I);
     int* wnnz = reinterpret_cast<int*>(wval + (size_t)B * I);
-    if (launch) {
-      const size_t row_bytes = (size_t)I * sizeof(float);
-      static const bool streaming = []() { const char* e = getenv("B200REC_ATT_COMPACT_STREAMING"); return e != nullptr && atoi(e) != 0; }();
-      if (row_bytes + 32 <= 96 * 1024 && !in.prepare_light && !streaming) {
-        static B200recSmemOptIn opted;
-        B200REC_CUDA(b200rec_opt_in_smem(opted, um_compact_vec_kernel, 96 * 1024));
-        um_compact_vec_kernel<<<B, ATT_WARPS * 32, row_bytes + 32, st>>>(in.um, in.ld_um, I, wcol, wval, wnnz, w);
-      } else {
-        um_compact_kernel<false><<<B, ATT_WARPS * 32, 0, st>>>(in.um, in.ld_um, I, wcol, wval, wnnz, w);
-      }
-      B200REC_CHECK_LAUNCH();
+    const size_t row_bytes = (size_t)I * sizeof(float);
+    if (row_bytes + 32 <= 96 * 1024) {
+      static B200recSmemOptIn opted;
+      B200REC_CUDA(b200rec_opt_in_smem(opted, um_compact_vec_kernel, 96 * 1024));
+      um_compact_vec_kernel<<<B, ATT_WARPS * 32, row_bytes + 32, st>>>(in.um, in.ld_um, I, wcol, wval, wnnz, w);
+    } else {
+      um_compact_kernel<<<B, ATT_WARPS * 32, 0, st>>>(in.um, in.ld_um, I, wcol, wval, wnnz, w);
     }
+    B200REC_CHECK_LAUNCH();
     lists.col = wcol; lists.val = wval; lists.row_nnz = wnnz; lists.row_ptr = nullptr; lists.stride = I;
-  } else if (launch) {
+  } else {
     att_worklist_kernel<<<ceil_div_i(B, 128), 128, 0, st>>>(in.row_ptr, B, w);
     B200REC_CHECK_LAUNCH();
   }
@@ -968,7 +937,7 @@ static int launch_att(const AttParams& p, const AttInputs& in, cudaStream_t st) 
   AttWork w;
   AttLists lists;
   {
-    const int rc = att_prepare(p.B, p.I, p.U, in, st, !in.prepared, w, lists);
+    const int rc = att_prepare(p.B, p.I, p.U, in, st, w, lists);
     if (rc) return rc;
   }
   const int* ccol = lists.col; const float* cval = lists.val; const int* cnnz = lists.row_nnz; const int* rp = lists.row_ptr;
@@ -1023,21 +992,6 @@ using namespace b200rec::attdrop;
 #define B200REC_ATT_ENTRY b200rec_attention_pool_dropout
 #else
 #define B200REC_ATT_ENTRY b200rec_attention_pool
-
-extern "C" int b200rec_attention_pool_prepare(const b200rec_attention_t* a, b200rec_stream_t stream) {
-  if (!a) return b200rec_fail(B200REC_ERR_BAD_ARG, "attention_pool_prepare: null descriptor");
-  if (a->B < 0 || a->I < 0 || a->U <= 0 || (a->U % 4)) return b200rec_fail(B200REC_ERR_BAD_ARG, "attention_pool_prepare: bad shape");
-  if (a->B == 0) return B200REC_OK;
-  if (!a->user_matrix && !(a->row_ptr && (a->col || a->I == 0))) return b200rec_fail(B200REC_ERR_BAD_ARG, "attention_pool_prepare: need user_matrix or CSR");
-  const bool dense = a->user_matrix != nullptr;
-  if (!a->workspace || a->workspace_bytes < att_layout(a->B, a->I, a->U, dense, a->max_row_nnz, a->nnz).total)
-    return b200rec_fail(B200REC_ERR_WORKSPACE, "attention_pool_prepare: workspace too small");
-  const long long ld_um = dense ? (a->ld_user_matrix ? a->ld_user_matrix : a->I) : 0;
-  AttInputs in{a->user_matrix, ld_um, a->row_ptr, a->col, a->val, a->workspace, a->workspace_bytes, a->max_row_nnz, a->nnz, 1, 0};
-  AttWork w;
-  AttLists lists;
-  return att_prepare((int)a->B, (int)a->I, a->U, in, (cudaStream_t)stream, true, w, lists);
-}
 
 extern "C" int b200rec_attention_pool_set_path(int path) {
   if (path < 0 || path > 2) return b200rec_fail(B200REC_ERR_BAD_ARG, "attention_pool_set_path: 0 auto, 1 registers, 2 TMA");
@@ -1101,7 +1055,7 @@ extern "C" int B200REC_ATT_ENTRY(const b200rec_attention_t* a, b200rec_stream_t 
   if (p.Ec && (!p.Er || p.E <= 0)) return b200rec_fail(B200REC_ERR_BAD_ARG, "attention_pool: training mask needs both embeddings");
   cudaStream_t st = (cudaStream_t)stream;
   const long long ld_um = a->user_matrix ? (a->ld_user_matrix ? a->ld_user_matrix : a->I) : 0;
-  AttInputs in{a->user_matrix, ld_um, a->row_ptr, a->col, a->val, a->workspace, a->workspace_bytes, a->max_row_nnz, a->nnz, 0, a->prepared};
+  AttInputs in{a->user_matrix, ld_um, a->row_ptr, a->col, a->val, a->workspace, a->workspace_bytes, a->max_row_nnz, a->nnz};
   if (a->table_dtype == B200REC_F32) {
     if (a->mode == MODE_NET) return dispatch_att<MODE_NET, float>(p, in, st);
     if (a->mode == MODE_DOT) return dispatch_att<MODE_DOT, float>(p, in, st);

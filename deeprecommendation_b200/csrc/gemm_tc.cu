@@ -1,12 +1,12 @@
 // K1a on the 5th-generation tensor cores:  Y = act((X · Wᵀ + bias) ∘ row_scale)  with tcgen05.mma + TMEM accumulators.
 //
-// Why the operands are NOT moved by TMA: the reference's profile width F = 2094 makes row pitches of 8376 bytes — not a
-// multiple of 16, which cuTensorMapEncodeTiled requires — and the inputs arrive as fp32 while the MMA wants bf16 or a
-// TF32 hi/lo split.  So eight producer warps read X and W with 64-bit loads, convert in registers and write the tiles
+// Why X is NOT moved by a TMA tensor map: the reference's profile width F = 2094 makes row pitches of 8376 bytes — not a
+// multiple of 16, which cuTensorMapEncodeTiled requires — and X arrives as fp32 while the MMA wants bf16 or a
+// TF32 hi/lo split.  So eight producer warps read X with 64-bit loads, convert in registers and write the tiles
 // straight into the canonical K-major SWIZZLE_128B shared-memory layout (16-byte chunk c of row r lives at chunk c^(r&7)
 // of its 128-byte row; 8-row groups are 1024 B apart), publish them to the async proxy with fence.proxy.async and an
-// mbarrier, and one elected thread of a ninth warp issues the MMAs.  HBM traffic is the compulsory one: every input
-// byte is read once as fp32, nothing is staged through a converted copy.
+// mbarrier, and one elected thread of a ninth warp issues the MMAs.  W is converted once into that layout
+// (b200rec_pack_weights_tc) and moved by TMA bulk copies.  Every X byte is read once as fp32.
 //
 // Two arithmetic modes on the same skeleton:
 //   TC_TF32X3 (fp32 parity, default): x = hi + lo with hi = round-to-TF32(x); D += A_hi·B_hi + A_hi·B_lo + A_lo·B_hi
@@ -20,8 +20,6 @@
 // CTA = 128 (M) x 128 (N) output tile, accumulator = 128 TMEM columns x 128 lanes (fp32), NSTAGE-deep smem ring.
 // Warp roles: warps 0-7 producers, then epilogue (tcgen05.ld 32x32b: warp w reads TMEM lanes 32*(w%4).., columns
 // 64*(w/4)..); warp 8 allocates TMEM and issues tcgen05.mma / tcgen05.commit.
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace b200rec {
@@ -119,13 +117,11 @@ __device__ __forceinline__ float tf32_round(float x) {
 
 struct TcParams {
   const float* X; long long ldx;
-  const float* W; long long ldw;
   int M, N, K;
   void* Y; long long ldy; int y_bf16;
   const float* bias; const float* row_scale; int relu;
-  const unsigned char* Wp;   // optional: W pre-packed by pack_weights_kernel (swizzled tiles), moved by TMA bulk copies
+  const unsigned char* Wp;   // W pre-packed by pack_weights_kernel (swizzled tiles), moved by TMA bulk copies
   const long long* row_index;   // optional: row m of the GEMM is row row_index[m] of X (resident profile table + ids)
-  int dbg;     // experiments only (B200REC_TC_DBG): 1 = no MMA, 2 = no prefetch loads, 4 = no proxy fence, 8 = no X loads at all, 16 = no W copies
   // split-K (b200rec_linear_tc_splitk): CTA z = blockIdx.z owns k-blocks [z*kb_per_split, ...) and writes its raw fp32 tile to
   // partial[z] (M x N, ld N); bias / scale / activation are applied by tc_splitk_reduce_kernel.  0 = the whole K in one CTA.
   int kb_per_split;
@@ -296,10 +292,9 @@ struct TileRegs {
 // these 193 KB CTAs takes the kernel from 30 us to 49 us.  A third form without clusters — tickets from a per-tile semaphore, the first split
 // to finish leaves its tile in one slab, the second adds it from L2 and completes the output — measured 46 us: only half of the CTAs take part in
 // that tail, eight warps each, whereas tc_splitk_reduce_kernel streams the two slabs with every SM (8 us).  The separate reduction stays.
-template <int MODE, int NSTAGE, int EPL, bool VEC, bool WPACK, int BN = TC_BN>
+template <int MODE, int NSTAGE, int EPL, bool VEC, int BN = TC_BN>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 gemm_tc_kernel(const __grid_constant__ TcBatch batch) {
-  static_assert(BN == 128 || (BN == 256 && WPACK), "the wide form needs packed weights");
   int q = 0;
 #pragma unroll
   for (int t = 1; t < TC_MAX_BATCH; ++t)
@@ -334,7 +329,7 @@ gemm_tc_kernel(const __grid_constant__ TcBatch batch) {
   if (tid == 0) {
 #pragma unroll
     for (int s = 0; s < NSTAGE; ++s) {
-      mbar_init(&full_bar[s], TC_PRODUCERS / 32 + (WPACK ? 1 : 0));   // one arrive per producer warp + the expect_tx arrive of the W bulk copy
+      mbar_init(&full_bar[s], TC_PRODUCERS / 32 + 1);   // one arrive per producer warp + the expect_tx arrive of the W bulk copy
       mbar_init(&empty_bar[s], 1);
     }
     mbar_init(&accum_bar, 1);
@@ -356,20 +351,18 @@ gemm_tc_kernel(const __grid_constant__ TcBatch batch) {
     // k-blocks of global loads in flight ahead of the store.  ncu (profiles/r01/ncu_full_gemm_tc_v3.txt, source page): 27 % of the
     // stall samples sat on the first use of the loaded registers (long scoreboard) with 2 k-blocks ahead.
     constexpr int PF = (MODE == TC_TF32X3) ? 2 : TC_PF16;    // (TF32: 3 and 4 were measured: register spills, 5-100 % slower)
-    TileAddr<MODE, EPL> aa, ab;
+    TileAddr<MODE, EPL> aa;
     aa.init(p.ldx, m0, p.M, warp, lane, p.row_index);
-    if constexpr (!WPACK) ab.init(p.ldw, n0, p.N, warp, lane);
     // packed W: tile (n-tile, k-block) = PLANES x 16 KB, already converted and swizzled (pack_weights_kernel)
-    const unsigned char* wp_tiles = WPACK ? p.Wp + ((size_t)blockIdx.x * NT * num_kb_total + kb_base) * (PLANES * TILE_BYTES) : nullptr;
+    const unsigned char* wp_tiles = p.Wp + ((size_t)blockIdx.x * NT * num_kb_total + kb_base) * (PLANES * TILE_BYTES);
     int kstore = kb_shift;                                    // k-block index of the stage being stored
-    TileRegs<MODE, EPL> xa[PF + 1], xb[PF + 1];
+    TileRegs<MODE, EPL> xa[PF + 1];
     int kload = kb_shift;                                     // k-block index of the next load
     int kcur = kb_shift;                                      // k-block index of the register buffer being stored
 #pragma unroll
     for (int d = 0; d < PF; ++d) {
-      if (d < num_kb && !(p.dbg & 8)) {
+      if (d < num_kb) {
         xa[d].template load<VEC>(p.X, aa, (kb_base + kload) * KB, p.K);
-        if constexpr (!WPACK) xb[d].template load<VEC>(p.W, ab, (kb_base + kload) * KB, p.K);
         kload = (kload + 1 == num_kb) ? 0 : kload + 1;
       }
     }
@@ -382,42 +375,33 @@ gemm_tc_kernel(const __grid_constant__ TcBatch batch) {
         if (kb < num_kb) {
           const int s = kb % NSTAGE;
           const uint32_t ph = (uint32_t)(kb / NSTAGE) & 1u;
-          if (kb + PF < num_kb && !(p.dbg & 10)) {             // loads of k-block kb+PF fly while kb is converted  (dbg 2 / 8: experiments)
+          if (kb + PF < num_kb) {                             // loads of k-block kb+PF fly while kb is converted
             xa[(j + PF) % (PF + 1)].template load<VEC>(p.X, aa, (kb_base + kload) * KB, p.K);
-            if constexpr (!WPACK) xb[(j + PF) % (PF + 1)].template load<VEC>(p.W, ab, (kb_base + kload) * KB, p.K);
             kload = (kload + 1 == num_kb) ? 0 : kload + 1;
           }
           mbar_wait(&empty_bar[s], ph ^ 1u);                  // first pass through the ring: returns immediately
           unsigned char* st = tiles + (size_t)s * STAGE_BYTES;
-          if constexpr (WPACK) {
-            if (tid == 0 && (p.dbg & 16)) mbar_arrive(&full_bar[s]);          // (experiment: no W copy)
-            if (tid == 0 && !(p.dbg & 16)) {                  // W tile(s): TMA bulk copies, no thread touches the data
-              mbar_arrive_expect_tx(&full_bar[s], NT * PLANES * TILE_BYTES);
-              if constexpr (NT == 1) {
-                tma_bulk_g2s(st + A_BYTES, wp_tiles + (size_t)kstore * (PLANES * TILE_BYTES), PLANES * TILE_BYTES, &full_bar[s]);
-              } else {
-                // two packed tiles [hi | lo] each -> stage layout [hi 0][hi 1][lo 0][lo 1]: the MMA sees one 256-row K-major operand per plane
+          if (tid == 0) {                                     // W tile(s): TMA bulk copies, no thread touches the data
+            mbar_arrive_expect_tx(&full_bar[s], NT * PLANES * TILE_BYTES);
+            if constexpr (NT == 1) {
+              tma_bulk_g2s(st + A_BYTES, wp_tiles + (size_t)kstore * (PLANES * TILE_BYTES), PLANES * TILE_BYTES, &full_bar[s]);
+            } else {
+              // two packed tiles [hi | lo] each -> stage layout [hi 0][hi 1][lo 0][lo 1]: the MMA sees one 256-row K-major operand per plane
 #pragma unroll
-                for (int nt = 0; nt < NT; ++nt)
+              for (int nt = 0; nt < NT; ++nt)
 #pragma unroll
-                  for (int pl = 0; pl < PLANES; ++pl)
-                    tma_bulk_g2s(st + A_BYTES + (pl * NT + nt) * TILE_BYTES,
-                                 wp_tiles + ((size_t)nt * num_kb_total + kstore) * (PLANES * TILE_BYTES) + (size_t)pl * TILE_BYTES, TILE_BYTES,
-                                 &full_bar[s]);
-              }
+                for (int pl = 0; pl < PLANES; ++pl)
+                  tma_bulk_g2s(st + A_BYTES + (pl * NT + nt) * TILE_BYTES,
+                               wp_tiles + ((size_t)nt * num_kb_total + kstore) * (PLANES * TILE_BYTES) + (size_t)pl * TILE_BYTES, TILE_BYTES,
+                               &full_bar[s]);
             }
-            kstore = (kstore + 1 == num_kb) ? 0 : kstore + 1;
           }
+          kstore = (kstore + 1 == num_kb) ? 0 : kstore + 1;
           const uint32_t st_u = smem_u32(st);
-          if ((kb_base + kcur + 1) * KB > p.K) {              // the one k-block that crosses K: masked stores (uniform branch)
-            xa[j].template store<true>(st_u, st_u + TILE_BYTES, aa);
-            if constexpr (!WPACK) xb[j].template store<true>(st_u + A_BYTES, st_u + A_BYTES + TILE_BYTES, ab);
-          } else {
-            xa[j].template store<false>(st_u, st_u + TILE_BYTES, aa);
-            if constexpr (!WPACK) xb[j].template store<false>(st_u + A_BYTES, st_u + A_BYTES + TILE_BYTES, ab);
-          }
+          if ((kb_base + kcur + 1) * KB > p.K) xa[j].template store<true>(st_u, st_u + TILE_BYTES, aa);   // the one k-block that crosses K: masked stores (uniform branch)
+          else xa[j].template store<false>(st_u, st_u + TILE_BYTES, aa);
           kcur = (kcur + 1 == num_kb) ? 0 : kcur + 1;
-          if (!(p.dbg & 4)) fence_proxy_async();              // generic-proxy smem writes -> visible to the tensor core
+          fence_proxy_async();                                // generic-proxy smem writes -> visible to the tensor core
           __syncwarp();                                       // one arrive per warp: 256 arrives on one mbarrier serialise in the shared-memory atomic unit
           if (lane == 0) mbar_arrive(&full_bar[s]);
         }
@@ -543,7 +527,6 @@ gemm_tc_kernel(const __grid_constant__ TcBatch batch) {
         const uint32_t b_hi = a_hi + A_BYTES;
 #pragma unroll
         for (int ks = 0; ks < 128 / UMMA_K_BYTES; ++ks) {
-          if (p.dbg & 1) break;
           const uint32_t off = (uint32_t)ks * UMMA_K_BYTES;
           if constexpr (MODE == TC_BF16) {
             umma<MODE>(tmem_base, make_desc(a_hi + off), make_desc(b_hi + off), idesc, (kb > 0 || ks > 0) ? 1u : 0u);
@@ -680,19 +663,19 @@ static int tc_splits(long long M, long long N, long long K, int mode, int* kb_pe
   return tc_splits_tiles(((M + 127) / 128) * ((N + 127) / 128), (N % 4) == 0, K, mode, kb_per_split);
 }
 
-template <int MODE, int EPL, bool VEC, bool WPACK, int BN = TC_BN>
+template <int MODE, int EPL, bool VEC, int BN = TC_BN>
 static int launch_tc_epl(const TcBatch& b, cudaStream_t st) {
   constexpr int PLANES = TcMode<MODE>::PLANES;
   constexpr int NSTAGE = BN == 256 ? ((MODE == TC_BF16) ? 4 : 2) : ((MODE == TC_BF16) ? 4 : 3);
   const size_t smem = (size_t)NSTAGE * (1 + BN / 128) * PLANES * TILE_BYTES + 1024;
   static B200recSmemOptIn opted;                     // per template instantiation, one bit per device
-  B200REC_CUDA(b200rec_opt_in_smem(opted, gemm_tc_kernel<MODE, NSTAGE, EPL, VEC, WPACK, BN>, (int)smem));
+  B200REC_CUDA(b200rec_opt_in_smem(opted, gemm_tc_kernel<MODE, NSTAGE, EPL, VEC, BN>, (int)smem));
   int nmax = 0;
   for (int q = 0; q < b.n; ++q) nmax = b.prob[q].N > nmax ? b.prob[q].N : nmax;
   const TcParams& p0 = b.prob[0];
   const int nsplit = p0.kb_per_split ? ceil_div_i(ceil_div_i(p0.K, TcMode<MODE>::KB), p0.kb_per_split) : 1;
   dim3 grid(ceil_div_i(nmax, BN), b.tile_start[b.n], nsplit);
-  gemm_tc_kernel<MODE, NSTAGE, EPL, VEC, WPACK, BN><<<grid, TC_THREADS, smem, st>>>(b);
+  gemm_tc_kernel<MODE, NSTAGE, EPL, VEC, BN><<<grid, TC_THREADS, smem, st>>>(b);
   B200REC_CHECK_LAUNCH();
   if (p0.kb_per_split) {
     for (int q = 0; q < b.n; ++q) {                  // (a batch shares K and kb_per_split: b200rec_linear_tc_splitk_batch)
@@ -711,28 +694,13 @@ static int launch_tc(const TcBatch& b, cudaStream_t st) {
   auto aligned = [&](int n) {
     for (int q = 0; q < b.n; ++q) {
       const TcParams& p = b.prob[q];
-      if (!((p.K % n) == 0 && (p.ldx % n) == 0 && ((uintptr_t)p.X % (4 * n)) == 0 &&
-            (p.Wp != nullptr || ((p.ldw % n) == 0 && ((uintptr_t)p.W % (4 * n)) == 0))))
-        return false;
+      if (!((p.K % n) == 0 && (p.ldx % n) == 0 && ((uintptr_t)p.X % (4 * n)) == 0)) return false;
     }
     return true;
   };
-  bool packed = true;
-  for (int q = 0; q < b.n; ++q) packed = packed && b.prob[q].Wp != nullptr;
-  if (packed) {
-    if (aligned(4)) return launch_tc_epl<MODE, 4, true, true, BN>(b, st);
-    if (aligned(2)) return launch_tc_epl<MODE, 2, true, true, BN>(b, st);
-    return launch_tc_epl<MODE, 2, false, true, BN>(b, st);
-  }
-  if constexpr (BN != TC_BN) return b200rec_fail(B200REC_ERR_BAD_ARG, "linear_tc_wide: needs packed weights");
-  for (int q = 0; q < b.n; ++q)
-    if (b.prob[q].Wp != nullptr && b.prob[q].W == nullptr) return b200rec_fail(B200REC_ERR_BAD_ARG, "linear_tc: a batch mixes packed-only and plain weights");
-  if constexpr (BN == TC_BN) {
-    if (aligned(4)) return launch_tc_epl<MODE, 4, true, false>(b, st);        // 128-bit loads (e.g. K = 128 transforms)
-    if (aligned(2)) return launch_tc_epl<MODE, 2, true, false>(b, st);        // 64-bit loads (F = 2094)
-    return launch_tc_epl<MODE, 2, false, false>(b, st);                       // odd K / pitch: scalar loads
-  }
-  return B200REC_ERR_BAD_ARG;
+  if (aligned(4)) return launch_tc_epl<MODE, 4, true, BN>(b, st);        // 128-bit loads (e.g. K = 128 transforms)
+  if (aligned(2)) return launch_tc_epl<MODE, 2, true, BN>(b, st);        // 64-bit loads (F = 2094)
+  return launch_tc_epl<MODE, 2, false, BN>(b, st);                       // odd K / pitch: scalar loads
 }
 
 }  // namespace b200rec
@@ -759,21 +727,21 @@ extern "C" int b200rec_pack_weights_tc(const float* W, int64_t N, int64_t K, int
   return B200REC_OK;
 }
 
-static int tc_fill(TcParams& p, const float* X, int64_t M, int64_t K, int64_t ldx, const float* W, int64_t N, int64_t ldw, const float* bias,
+// W and ldw of the entry points are not read: the GEMM takes the weights from `packed_w`
+static int tc_fill(TcParams& p, const float* X, int64_t M, int64_t K, int64_t ldx, int64_t N, const float* bias,
                    const float* row_scale, int relu, void* Y, int64_t ldy, int y_dtype, const void* packed_w,
                    const int64_t* row_index = nullptr, int64_t x_rows = 0) {
-  if (M < 0 || N <= 0 || K <= 0 || (!W && !packed_w) || (M > 0 && (!X || !Y))) return b200rec_fail(B200REC_ERR_BAD_ARG, "linear_tc: bad argument");
+  if (M < 0 || N <= 0 || K <= 0 || (M > 0 && (!X || !Y))) return b200rec_fail(B200REC_ERR_BAD_ARG, "linear_tc: bad argument");
+  if (!packed_w) return b200rec_fail(B200REC_ERR_BAD_ARG, "linear_tc: needs the packed weights (b200rec_pack_weights_tc, same mode)");
   if (M > INT32_MAX || N > INT32_MAX || K > INT32_MAX) return b200rec_fail(B200REC_ERR_UNSUPPORTED, "linear_tc: dim > int32");
-  if (ldx < K || ldw < K || ldy < N) return b200rec_fail(B200REC_ERR_BAD_ARG, "linear_tc: leading dimension too small");
-  if ((row_index ? x_rows : M) * ldx >= (1LL << 32) || (!packed_w && N * ldw >= (1LL << 32))) return b200rec_fail(B200REC_ERR_UNSUPPORTED, "linear_tc: operand larger than 2^32 elements");
+  if (ldx < K || ldy < N) return b200rec_fail(B200REC_ERR_BAD_ARG, "linear_tc: leading dimension too small");
+  if ((row_index ? x_rows : M) * ldx >= (1LL << 32)) return b200rec_fail(B200REC_ERR_UNSUPPORTED, "linear_tc: operand larger than 2^32 elements");
   if (row_index && x_rows <= 0) return b200rec_fail(B200REC_ERR_BAD_ARG, "linear_tc: row_index needs the row count of X");
   if (y_dtype != B200REC_F32 && y_dtype != B200REC_BF16) return b200rec_fail(B200REC_ERR_BAD_ARG, "linear_tc: bad y_dtype");
   p.row_index = reinterpret_cast<const long long*>(row_index);
-  p.X = X; p.ldx = ldx; p.W = W; p.ldw = ldw; p.M = (int)M; p.N = (int)N; p.K = (int)K;
+  p.X = X; p.ldx = ldx; p.M = (int)M; p.N = (int)N; p.K = (int)K;
   p.Wp = (const unsigned char*)packed_w;
   p.Y = Y; p.ldy = ldy; p.y_bf16 = y_dtype == B200REC_BF16; p.bias = bias; p.row_scale = row_scale; p.relu = relu;
-  const char* e = getenv("B200REC_TC_DBG");
-  p.dbg = e ? atoi(e) : 0;
   p.kb_per_split = 0;
   p.partial = nullptr;
   return B200REC_OK;
@@ -784,7 +752,7 @@ extern "C" int b200rec_linear_tc(const float* X, int64_t M, int64_t K, int64_t l
                                  const void* packed_w, const int64_t* row_index, int64_t x_rows, b200rec_stream_t stream) {
   TcBatch b;
   b.n = 1;
-  const int rc = tc_fill(b.prob[0], X, M, K, ldx, W, N, ldw, bias, row_scale, relu, Y, ldy, y_dtype, packed_w, row_index, x_rows);
+  const int rc = tc_fill(b.prob[0], X, M, K, ldx, N, bias, row_scale, relu, Y, ldy, y_dtype, packed_w, row_index, x_rows);
   if (rc) return rc;
   if (M == 0) return B200REC_OK;
   b.tile_start[0] = 0;
@@ -807,7 +775,7 @@ extern "C" int b200rec_linear_tc_splitk(const float* X, int64_t M, int64_t K, in
                                         const void* packed_w, void* workspace, size_t workspace_bytes, b200rec_stream_t stream) {
   TcBatch b;
   b.n = 1;
-  const int rc = tc_fill(b.prob[0], X, M, K, ldx, W, N, ldw, bias, row_scale, relu, Y, ldy, y_dtype, packed_w, nullptr, 0);
+  const int rc = tc_fill(b.prob[0], X, M, K, ldx, N, bias, row_scale, relu, Y, ldy, y_dtype, packed_w, nullptr, 0);
   if (rc) return rc;
   if (M == 0) return B200REC_OK;
   if (mode != B200REC_TC_TF32X3 && mode != B200REC_TC_BF16) return b200rec_fail(B200REC_ERR_BAD_ARG, "linear_tc_splitk: bad mode");
@@ -854,9 +822,8 @@ extern "C" int b200rec_linear_tc_wide(const float* X, int64_t M, int64_t K, int6
   TcBatch b;
   b.n = 1;
   if (mode != B200REC_TC_TF32X3 && mode != B200REC_TC_BF16X3) return b200rec_fail(B200REC_ERR_BAD_ARG, "linear_tc_wide: mode is TF32X3 or BF16X3");
-  if (!packed_w) return b200rec_fail(B200REC_ERR_BAD_ARG, "linear_tc_wide: needs the packed weights (b200rec_pack_weights_tc, same mode)");
   if (N <= 128 || ((N + 127) / 128) % 2) return b200rec_fail(B200REC_ERR_UNSUPPORTED, "linear_tc_wide: N must cover an even number of 128-column tiles");
-  const int rc = tc_fill(b.prob[0], X, M, K, ldx, nullptr, N, K, bias, row_scale, relu, Y, ldy, y_dtype, packed_w, row_index, x_rows);
+  const int rc = tc_fill(b.prob[0], X, M, K, ldx, N, bias, row_scale, relu, Y, ldy, y_dtype, packed_w, row_index, x_rows);
   if (rc) return rc;
   if (M == 0) return B200REC_OK;
   int kbps = 0;
@@ -880,7 +847,7 @@ extern "C" int b200rec_linear_tc_batch(const b200rec_linear_problem_t* problems,
   for (int q = 0; q < n_problems; ++q) {
     const b200rec_linear_problem_t& r = problems[q];
     if (r.M == 0) continue;
-    const int rc = tc_fill(b.prob[b.n], r.X, r.M, K, r.ldx, r.W, r.N, r.ldw, r.bias, r.row_scale, r.relu, r.Y, r.ldy, r.y_dtype, r.packed_w);
+    const int rc = tc_fill(b.prob[b.n], r.X, r.M, K, r.ldx, r.N, r.bias, r.row_scale, r.relu, r.Y, r.ldy, r.y_dtype, r.packed_w);
     if (rc) return rc;
     b.tile_start[b.n + 1] = b.tile_start[b.n] + ceil_div_i(r.M, TC_BM);
     ++b.n;
@@ -933,7 +900,7 @@ extern "C" int b200rec_linear_tc_splitk_batch(const b200rec_linear_problem_t* pr
   for (int q = 0; q < n_problems; ++q) {
     const b200rec_linear_problem_t& r = problems[q];
     if (r.M == 0) continue;
-    const int rc = tc_fill(b.prob[b.n], r.X, r.M, K, r.ldx, r.W, r.N, r.ldw, r.bias, r.row_scale, r.relu, r.Y, r.ldy, r.y_dtype, r.packed_w);
+    const int rc = tc_fill(b.prob[b.n], r.X, r.M, K, r.ldx, r.N, r.bias, r.row_scale, r.relu, r.Y, r.ldy, r.y_dtype, r.packed_w);
     if (rc) return rc;
     if (splits > 1) {
       b.prob[b.n].kb_per_split = kbps;

@@ -6,8 +6,6 @@
 // through a row gather, which is GraphNCF's `combined[itemIds]` / `combined[userIds]`) straight into the
 // first activation buffer in shared memory, and every intermediate activation ping-pongs between two
 // shared-memory buffers; only the final (B, out) scores are written to HBM.
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace b200rec {
@@ -212,9 +210,8 @@ extern "C" int b200rec_mlp_tower(const float* in0, int64_t ld0, const int64_t* i
   // small batches: fewer rows per CTA so that more SMs take part
   const bool small = B < (long long)16 * sms * 2;
   // a batch that 4-row CTAs still fit into one wave (512 pairs -> 128 CTAs): the tower is a latency chain per CTA, more and shorter
-  // chains finish sooner (B200REC_MLP_TM4=0 switches it off)
-  static const bool tm4_on = []() { const char* e = getenv("B200REC_MLP_TM4"); return e == nullptr || atoi(e) != 0; }();
-  const bool tiny = tm4_on && B <= (long long)4 * sms;
+  // chains finish sooner
+  const bool tiny = B <= (long long)4 * sms;
   const int TM = tiny ? 4 : (small ? 8 : 16);
   size_t smem = ((size_t)2 * TM * stride + (size_t)(small ? 4 : 2) * MLP_THREADS * MLP_WS) * sizeof(float);
   if (smem > 200 * 1024) return b200rec_fail(B200REC_ERR_UNSUPPORTED, "mlp_tower: layer too wide for shared memory");

@@ -8,8 +8,6 @@
 // through mbarriers: 8 producer warps (global fp32 -> TF32 hi/lo -> swizzled smem ring), one MMA warp (3xTF32: hi·hi into a
 // main accumulator, hi·lo + lo·hi into a second one), 4 epilogue warps draining the previous tile's accumulators from TMEM
 // (two accumulator pairs = all 512 columns) while the next tile is produced.  fp32 parity: the same split as gemm_tc.cu.
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace b200rec {
@@ -78,7 +76,6 @@ struct NodeGemmParams {
   // all-gather fused into the epilogue (partitioned propagation): every tile is also stored to Yx[q], q < n_extra — the same
   // place of the peer ranks' feature tables, mapped over NVLink (csrc/peer.cu)
   void* Yx[B200REC_PEER_MAX]; int n_extra;
-  int dbg;                             // experiments (B200REC_NT_DBG): 1 = no stores, 2 = no MMA, 4 = no TMEM loads
 };
 
 template <int NKB, bool PUSH>
@@ -220,34 +217,32 @@ node_gemm_kernel(const __grid_constant__ NodeGemmParams p) {
           *reinterpret_cast<float4*>(stg + lane * NT_STG_LD + j) = make_float4(o[0], o[1], o[2], o[3]);
         }
         __syncwarp();
-        if (!(p.dbg & 1)) {
 #pragma unroll
-          for (int i = 0; i < 8; ++i) {
-            const int r = i * 4 + (lane >> 3), cc = (lane & 7) * 4;
-            const int grow = tile * 128 + e * 32 + r, n = cg * 32 + cc;
-            if (grow < p.M && n < p.N) {
-              const float4 v = *reinterpret_cast<const float4*>(stg + r * NT_STG_LD + cc);
-              const int n_dst = PUSH ? p.n_extra + 1 : 1;           // PUSH: the peers' copies of the table (NVLink stores) after the local one
+        for (int i = 0; i < 8; ++i) {
+          const int r = i * 4 + (lane >> 3), cc = (lane & 7) * 4;
+          const int grow = tile * 128 + e * 32 + r, n = cg * 32 + cc;
+          if (grow < p.M && n < p.N) {
+            const float4 v = *reinterpret_cast<const float4*>(stg + r * NT_STG_LD + cc);
+            const int n_dst = PUSH ? p.n_extra + 1 : 1;           // PUSH: the peers' copies of the table (NVLink stores) after the local one
 #pragma unroll 1
-              for (int dq = 0; dq < n_dst; ++dq) {
-                void* const Yq = (!PUSH || dq == 0) ? p.Y : p.Yx[dq - 1];
-                if (p.y_bf16) {                                      // 4 rows x 64 bytes per warp instruction
-                  __nv_bfloat16* d = reinterpret_cast<__nv_bfloat16*>(Yq) + (long long)grow * p.ldy + n;
-                  if (n + 3 < p.N && (((uintptr_t)d & 7) == 0)) {
-                    const __nv_bfloat162 lo = __floats2bfloat162_rn(v.x, v.y), hi = __floats2bfloat162_rn(v.z, v.w);
-                    *reinterpret_cast<uint2*>(d) = make_uint2(*reinterpret_cast<const unsigned*>(&lo), *reinterpret_cast<const unsigned*>(&hi));
-                  } else {
-                    const float o[4] = {v.x, v.y, v.z, v.w};
-                    for (int q = 0; q < 4 && n + q < p.N; ++q) d[q] = __float2bfloat16_rn(o[q]);
-                  }
-                  continue;
-                }
-                float* d = reinterpret_cast<float*>(Yq) + (long long)grow * p.ldy + n;
-                if (n + 3 < p.N && (((uintptr_t)d & 15) == 0)) *reinterpret_cast<float4*>(d) = v;
-                else {
+            for (int dq = 0; dq < n_dst; ++dq) {
+              void* const Yq = (!PUSH || dq == 0) ? p.Y : p.Yx[dq - 1];
+              if (p.y_bf16) {                                      // 4 rows x 64 bytes per warp instruction
+                __nv_bfloat16* d = reinterpret_cast<__nv_bfloat16*>(Yq) + (long long)grow * p.ldy + n;
+                if (n + 3 < p.N && (((uintptr_t)d & 7) == 0)) {
+                  const __nv_bfloat162 lo = __floats2bfloat162_rn(v.x, v.y), hi = __floats2bfloat162_rn(v.z, v.w);
+                  *reinterpret_cast<uint2*>(d) = make_uint2(*reinterpret_cast<const unsigned*>(&lo), *reinterpret_cast<const unsigned*>(&hi));
+                } else {
                   const float o[4] = {v.x, v.y, v.z, v.w};
-                  for (int q = 0; q < 4 && n + q < p.N; ++q) d[q] = o[q];
+                  for (int q = 0; q < 4 && n + q < p.N; ++q) d[q] = __float2bfloat16_rn(o[q]);
                 }
+                continue;
+              }
+              float* d = reinterpret_cast<float*>(Yq) + (long long)grow * p.ldy + n;
+              if (n + 3 < p.N && (((uintptr_t)d & 15) == 0)) *reinterpret_cast<float4*>(d) = v;
+              else {
+                const float o[4] = {v.x, v.y, v.z, v.w};
+                for (int q = 0; q < 4 && n + q < p.N; ++q) d[q] = o[q];
               }
             }
           }
@@ -277,7 +272,6 @@ node_gemm_kernel(const __grid_constant__ NodeGemmParams p) {
           for (int ks = 0; ks < 4; ++ks) {                       // 8 TF32 (32 bytes) of K per MMA
             const uint32_t off = (uint32_t)ks * 32u;
             const uint32_t first = (kb > 0 || ks > 0) ? 1u : 0u;
-            if (p.dbg & 2) continue;
             nt_umma_tf32(d_main, nt_desc(a_hi + off), nt_desc(w_hi + off), idesc, first);     // hi · hi
             nt_umma_tf32(d_cross, nt_desc(a_hi + off), nt_desc(w_lo + off), idesc, first);    // hi · lo
             nt_umma_tf32(d_cross, nt_desc(a_lo + off), nt_desc(w_hi + off), idesc, 1u);       // lo · hi
@@ -332,10 +326,6 @@ static int shortk_run(const float* X, int64_t M, int64_t K, int64_t ldx, const v
   p.bias = bias; p.row_scale = row_scale; p.relu = relu; p.Y = Y; p.ldy = ldy; p.y_bf16 = y_dtype == B200REC_BF16;
   p.n_extra = n_extra;
   for (int q = 0; q < B200REC_PEER_MAX; ++q) p.Yx[q] = q < n_extra ? extra[q] : nullptr;
-  {
-    const char* e = getenv("B200REC_NT_DBG");
-    p.dbg = e ? atoi(e) : 0;
-  }
   cudaStream_t st = (cudaStream_t)stream;
   if (n_extra > 0) {
     switch (K / 32) {

@@ -17,7 +17,6 @@
 // flight per warp.  (A cp.async/LDGSTS shared-memory ring was tried and measured 1.5x SLOWER — 3.4 vs 2.25 ms per
 // layer on the MovieLens-25M shape — and was dropped; see DESIGN.md §6.)
 #include <math.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 
@@ -108,29 +107,17 @@ template <> struct Lane16<__nv_bfloat16> {
 };
 
 __device__ __forceinline__ uint4 ldg16(const unsigned char* p) { return __ldg(reinterpret_cast<const uint4*>(p)); }
-// Feature rows are the only data of a layer that is re-read (2E gathers over N rows); the CSR streams (`__ldcs`) and the
-// outputs pass through once.  KEEP = load the rows with an L2 evict_last policy so that the streams do not push them out
-// (profiles/r01: 2.2 GB of DRAM reads per layer against 0.63 GB compulsory with the default policy).
-__device__ __forceinline__ uint64_t l2_keep_policy() {
-  uint64_t pol;
-  asm("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
-  return pol;
-}
-__device__ __forceinline__ uint4 ldg16_keep(const unsigned char* p, uint64_t pol) {
-  uint4 r;
-  asm("ld.global.nc.L2::cache_hint.v4.u32 {%0, %1, %2, %3}, [%4], %5;" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p), "l"(pol));
-  return r;
-}
 
 // G lanes cooperate on one edge (each lane owns 16 bytes of the source row; G*16*NV >= row bytes), so 32/G edges
 // advance per warp step.  The inner loop is branch- and predicate-free: padding / masked edges carry (source 0,
 // weight 0) and lanes beyond the row width read column 0, so every load is valid and the per-edge cost is
 // 2 SHFL + 1 IMAD.WIDE.U32 + 1 LDG.128 + 4 FFMA (the first version spent ~26 instructions per edge on predicated
 // 64-bit address arithmetic and zero-fill moves — profiles/r01).
-template <int G, int NV, typename T, bool GAT, bool KEEP, int UN = 8, bool PUSH = false>
-__global__ void __launch_bounds__(SPMM_WARPS * 32, ((NV == 1 && UN == 8 && !GAT) || (NV * UN == 8 && NV > 1 && !GAT && sizeof(T) == 4)) ? SPMM_MIN_CTAS : 1)
+template <int G, int NV, typename T, bool GAT, bool PUSH = false>
+__global__ void __launch_bounds__(SPMM_WARPS * 32, (NV == 1 && !GAT) ? SPMM_MIN_CTAS : 1)
 spmm_chunk_kernel(const __grid_constant__ SpmmParams p) {
   constexpr int EPW = 32 / G;                       // edges per warp step
+  constexpr int UN = 8;                             // warp steps whose row loads are in flight together
   constexpr int VPL = Lane16<T>::VPL;
   constexpr int STEPS = 32 / EPW;                   // warp steps per 32-edge block (= G)
   const int lane = threadIdx.x & 31;
@@ -143,7 +130,6 @@ spmm_chunk_kernel(const __grid_constant__ SpmmParams p) {
   const float dinv_row = p.dinv ? __ldg(p.dinv + row) : 1.f;     //  ncu showed the final FMUL waiting on dinv[row])
   const int e = min(s + p.chunk_size, __ldg(p.row_ptr + row + 1));
   const unsigned stride_bytes = (unsigned)(p.ld_t * (long long)sizeof(T));
-  const uint64_t keep = KEEP ? l2_keep_policy() : 0ull;
   const unsigned char* base[NV];
   bool active[NV];
 #pragma unroll
@@ -217,7 +203,7 @@ spmm_chunk_kernel(const __grid_constant__ SpmmParams p) {
 #pragma unroll
           for (int nv = 0; nv < NV; ++nv) {
             const unsigned char* src = base[nv] + (unsigned long long)cc * stride_bytes;
-            x[u][nv] = KEEP ? ldg16_keep(src, keep) : ldg16(src);
+            x[u][nv] = ldg16(src);
           }
         }
 #pragma unroll
@@ -373,20 +359,9 @@ spmm_fixup_kernel(const __grid_constant__ SpmmParams p) {
 template <int G, int NV, typename T>
 static int launch_chunks(const SpmmParams& p, cudaStream_t st) {
   const int grid = ceil_div_i(p.n_chunks, SPMM_WARPS);
-  static const bool keep = []() { const char* e = getenv("B200REC_SPMM_L2_KEEP"); return e != nullptr && atoi(e) != 0; }();   // off by default: measured 3.21 vs 3.16 ms per config-3 step with the hint
-  static const bool unroll16 = []() { const char* e = getenv("B200REC_SPMM_UNROLL"); return e != nullptr && atoi(e) == 16; }();
-  if constexpr (NV > 1 && G < 32) {      // narrow-group layouts (several edges per warp step): plain and push epilogues only
-    constexpr int UNW = 8 / NV;
-    if (p.push_parts > 0) spmm_chunk_kernel<G, NV, T, false, false, UNW, true><<<grid, SPMM_WARPS * 32, 0, st>>>(p);
-    else spmm_chunk_kernel<G, NV, T, false, false, UNW, false><<<grid, SPMM_WARPS * 32, 0, st>>>(p);
-    B200REC_CHECK_LAUNCH();
-    return B200REC_OK;
-  }
-  if (p.push_parts > 0) spmm_chunk_kernel<G, NV, T, false, false, 8, true><<<grid, SPMM_WARPS * 32, 0, st>>>(p);
-  else if (p.att_src) spmm_chunk_kernel<G, NV, T, true, false><<<grid, SPMM_WARPS * 32, 0, st>>>(p);
-  else if (keep) spmm_chunk_kernel<G, NV, T, false, true><<<grid, SPMM_WARPS * 32, 0, st>>>(p);
-  else if (NV == 1 && G >= 16 && unroll16) spmm_chunk_kernel<G, NV, T, false, false, (NV == 1 && G >= 16) ? 16 : 8><<<grid, SPMM_WARPS * 32, 0, st>>>(p);
-  else spmm_chunk_kernel<G, NV, T, false, false><<<grid, SPMM_WARPS * 32, 0, st>>>(p);
+  if (p.push_parts > 0) spmm_chunk_kernel<G, NV, T, false, true><<<grid, SPMM_WARPS * 32, 0, st>>>(p);
+  else if (p.att_src) spmm_chunk_kernel<G, NV, T, true><<<grid, SPMM_WARPS * 32, 0, st>>>(p);
+  else spmm_chunk_kernel<G, NV, T, false><<<grid, SPMM_WARPS * 32, 0, st>>>(p);
   B200REC_CHECK_LAUNCH();
   return B200REC_OK;
 }
@@ -398,14 +373,7 @@ static int launch_spmm(const SpmmParams& p, cudaStream_t st) {
     int rc;
     if (row_bytes <= 128) rc = launch_chunks<8, 1, T>(p, st);
     else if (row_bytes <= 256) rc = launch_chunks<16, 1, T>(p, st);
-    else if (row_bytes <= 512) {
-      // 512-byte rows: G lanes per edge x NV 128-bit loads per lane.  Fewer lanes per edge = more edges per SHFL of the (source, weight)
-      // broadcast; the L1 data pipe (register write-back of LDG + SHFL) is this kernel's limiter (profiles/r02/ncu_full_shard_spmm_v1.txt)
-      static const int g512 = []() { const char* e = getenv("B200REC_SPMM_G512"); return e ? atoi(e) : 32; }();
-      if (g512 == 8 && !p.att_src && sizeof(T) == 4) rc = launch_chunks<8, 4, T>(p, st);
-      else if (g512 == 16 && !p.att_src && sizeof(T) == 4) rc = launch_chunks<16, 2, T>(p, st);
-      else rc = launch_chunks<32, 1, T>(p, st);
-    }
+    else if (row_bytes <= 512) rc = launch_chunks<32, 1, T>(p, st);
     else if (row_bytes <= 1024) rc = launch_chunks<32, 2, T>(p, st);
     else if (row_bytes <= 2048 && sizeof(T) == 4) rc = launch_chunks<32, 4, T>(p, st);
     else return b200rec_fail(B200REC_ERR_UNSUPPORTED, "spmm: node_emb wider than 512");

@@ -10,7 +10,6 @@ from the two edge lists once per graph and cached on the graph object.
 from __future__ import annotations
 
 import ctypes as C
-import os
 
 import torch
 
@@ -345,9 +344,6 @@ class StreamPlan:
 
 def default_stream_seg(nnz: int) -> int:
     """entries per warp: long segments amortise the set-up, but a launch should still be >= ~8 warps per resident warp slot of the GPU"""
-    env = os.environ.get('B200REC_SPMM_SEG')
-    if env:
-        return int(env)
     return 256 if nnz >= 24_000_000 else (128 if nnz >= 2_000_000 else 64)
 
 

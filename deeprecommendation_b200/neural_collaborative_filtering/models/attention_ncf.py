@@ -1,7 +1,6 @@
 """AttentionNCF on the B200 path (reference: neural_collaborative_filtering/models/attention_ncf.py:64-224)."""
 from __future__ import annotations
 
-import os
 import weakref
 
 import torch
@@ -13,17 +12,7 @@ from ..util import build_MLP_layers, mlp_parameters, run_mlp
 from .base import NCF, _named_like
 
 
-_SIDE_STREAMS = {}
 RECOMMEND_SLAB_BYTES = 1 << 30      # default budget of one chunk's h1 slab in `AttentionNCF.recommend` (users per chunk = budget / (nI·H1P·4))
-
-
-def _side_stream(device):
-    """one extra stream per device for work that is independent of the projection GEMMs (K2's first phase)"""
-    key = torch.device(device).index if torch.device(device).index is not None else torch.cuda.current_device()
-    s = _SIDE_STREAMS.get(key)
-    if s is None:
-        s = _SIDE_STREAMS[key] = torch.cuda.Stream(device=key)
-    return s
 
 
 def _pad_rows(w, b, mult=4):
@@ -51,10 +40,6 @@ class AttentionNCF(NCF):
       K1b  out = MLP([Ec, user_emb])                       item first (attention_ncf.py:219)
 
     Nothing of shape (B·I, E) or (B, I, ·) is ever materialised (the reference builds two of them, :154-155)."""
-
-    # K2's first phase on a side stream next to the projection GEMMs (inference).  Off by default: at config 2 the fork / join
-    # inside the captured graph and the shared-memory-free compaction cost more than the overlap hides (193 vs 177 us per step).
-    overlap_prepare = os.environ.get('B200REC_ATT_OVERLAP_PREPARE', '0') == '1'
 
     def __init__(self, item_dim, item_emb=128, user_emb=128, att_dense=None, mlp_dense_layers=None, use_cos_sim_instead=False,
                  dropout_rate=0.2, message_dropout=None):
@@ -179,29 +164,11 @@ class AttentionNCF(NCF):
             # The rated-item sweep fills the device exactly at config 2 (74 x 2 tiles on 148 SMs — adding the candidates' 4
             # row tiles to that launch costs a second wave, measured 132 vs 71 us), so the candidates keep their own GEMM.
             Wr, br, Wc, bc, bU, a2, a20, H = comp
-            # K2's first phase (compaction of the dense user_matrix + work list) needs only the matrix: with `overlap_prepare`
-            # it runs on a side stream underneath the projection GEMMs and is joined right before the pooling kernel
-            prepared = None
-            if self.overlap_prepare and user_matrix.is_cuda and user_matrix.shape[0] > 0 and user_matrix.shape[1] > 0:
-                cur = torch.cuda.current_stream(user_matrix.device)
-                side = _side_stream(user_matrix.device)
-                side.wait_stream(cur)
-                with torch.cuda.stream(side):
-                    prepared = ops.attention_prepare(user_matrix, (user.weight.shape[0] + 3) // 4 * 4)
             EcPc = ops.linear_raw(candidate_items, Wc, bc)                              # :150 (+ candidate half of :176)
             PrQ = ops.linear_raw(rated_items, Wr, br)                                   # :151 folded with :176, + Q = R·W_Uᵀ
             Ec, Pc = EcPc[:, :E], EcPc[:, E:]
             Pr, Q = PrQ[:, :H], PrQ[:, H:]
             mode = L.ATT_NET
-            if prepared is not None:
-                cur.wait_stream(side)
-                res = ops.attention_pool_raw(Pc, Pr, Q, mode=mode, a2=a2, a20=a20, bU=bU, return_attention_weights=return_attention_weights,
-                                             prepared=prepared)
-                user_emb, att = res if return_attention_weights else (res, None)
-                if user_emb.shape[1] != U:
-                    user_emb = user_emb[:, :U]
-                out = run_mlp(self.MLP, Ec, user_emb, training=False)
-                return (out, att.detach()) if return_attention_weights else out
         else:
             Wcat, bcat, bU = self._stacked_projection()
             Ec = ops.linear(candidate_items, item.weight, item.bias)                    # :150

@@ -143,12 +143,9 @@ _gemm_engine = os.environ.get('B200REC_GEMM_ENGINE', 'bf16x3')
 TC_MIN_ROWS = 2048
 TC_SPLITK_MIN_ROWS = 128      # below TC_MIN_ROWS the tensor-core GEMM runs split-K (if K is long enough to be dealt out)
 SHORTK_MIN_ROWS = 4096  # below this a handful of 64x64 FFMA tiles is as fast as the persistent kernel's set-up
-SPLITK_ANY_N = os.environ.get('B200REC_SPLITK_ANY_N', '1') == '1'   # split-K also when N % 4 != 0 (padded slabs)
-TC_WIDE = os.environ.get('B200REC_TC_WIDE', '1') == '1'      # 128 x 256 tiles + split-K for 128 < N (csrc/gemm_tc.cu, BN = 256)
 TC_MIN_K = 512          # short-K GEMMs (the d x d GraphNCF transforms) are epilogue/latency-bound: FFMA is as fast there
 
 
-_pack_weights = True          # move the W operand of the tensor-core GEMM by TMA from a pre-swizzled copy
 _pack_cache = {}              # (data_ptr, version, shape, ld, mode) -> packed buffer; a handful of weight matrices at most
 
 
@@ -235,7 +232,7 @@ def linear_raw(x, weight, bias=None, row_scale=None, relu=False, out=None, out_d
         raise ValueError('linear: shape not supported by the short-K kernel')
     if engine != 'simt' and ((M >= TC_MIN_ROWS and K >= TC_MIN_K) or engine.endswith('!')) and (x_rows if row_index is not None else M) * ldx < 2 ** 32:
         mode = _tc_mode(engine)
-        if TC_WIDE and mode == L.TC_TF32X3 and _pack_weights and N > 128 and ((N + 127) // 128) % 2 == 0 and K >= 256:
+        if mode == L.TC_TF32X3 and N > 128 and ((N + 127) // 128) % 2 == 0 and K >= 256:
             # 128 x 256 tiles: every X block converted and staged once for both halves of W, k range split over the CTAs
             if engine.startswith('bf16x3'):              # the same three products on a bf16 hi/lo split (2x MMA rate, ~4e-6)
                 mode = L.TC_BF16X3
@@ -246,18 +243,17 @@ def linear_raw(x, weight, bias=None, row_scale=None, relu=False, out=None, out_d
                 L.check(lib.b200rec_linear_tc_wide(_ptr(x), M, K, ldx, N, _ptr(bias), _ptr(row_scale), int(relu), _ptr(out), ldy, _dtype_code(out.dtype),
                                                    mode, _ptr(packed), _ptr(row_index), x_rows, _ptr(ws), wsb, _stream()), 'linear_tc_wide')
             return out
-        packed = _packed_weight(w, ldw, mode) if _pack_weights else None
+        packed = _packed_weight(w, ldw, mode)
         with _on(x.device), _timed('linear_tc', (M, K, N)):
             L.check(lib.b200rec_linear_tc(_ptr(x), M, K, ldx, _ptr(w), N, ldw, _ptr(bias), _ptr(row_scale), int(relu), _ptr(out), ldy,
                                           _dtype_code(out.dtype), mode, _ptr(packed), _ptr(row_index), x_rows, _stream()), 'linear_tc')
         return out
-    if (engine != 'simt' and row_index is None and TC_SPLITK_MIN_ROWS <= M < TC_MIN_ROWS and K >= TC_MIN_K and M * ldx < 2 ** 32
-            and (N % 4 == 0 or SPLITK_ANY_N)):
+    if engine != 'simt' and row_index is None and TC_SPLITK_MIN_ROWS <= M < TC_MIN_ROWS and K >= TC_MIN_K and M * ldx < 2 ** 32:
         # short-M, long-K (a batch of pairs against the F-wide profiles): split-K on the tensor cores
         mode = _tc_mode(engine)
         ws_bytes = lib.b200rec_linear_tc_splitk_workspace(M, N, K, mode)
         if ws_bytes:
-            packed = _packed_weight(w, ldw, mode) if _pack_weights else None
+            packed = _packed_weight(w, ldw, mode)
             ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
             with _on(x.device), _timed('linear_tc_splitk', (M, K, N)):
                 L.check(lib.b200rec_linear_tc_splitk(_ptr(x), M, K, ldx, _ptr(w), N, ldw, _ptr(bias), _ptr(row_scale), int(relu), _ptr(out), ldy,
@@ -301,11 +297,11 @@ def linear_tc_batch(problems, engine=None):
             out = torch.empty((M, N), dtype=torch.float32, device=dev)
         elif out.shape != (M, N) or out.stride(1) != 1:
             raise ValueError('linear_tc_batch: bad `out`')
-        packed = _packed_weight(weight if weight is w else w, ldw, mode) if _pack_weights else None
+        packed = _packed_weight(weight if weight is w else w, ldw, mode)
         p = arr[q]
         p.X, p.M, p.ldx = x.data_ptr(), M, ldx
         p.W, p.N, p.ldw = w.data_ptr(), N, ldw
-        p.packed_w = packed.data_ptr() if packed is not None else None
+        p.packed_w = packed.data_ptr()
         p.bias = bias.data_ptr() if bias is not None else None
         p.row_scale, p.relu = None, 0
         p.Y, p.ldy, p.y_dtype = out.data_ptr(), (out.stride(0) if M > 1 else max(N, out.stride(0))), _dtype_code(out.dtype)
@@ -342,11 +338,11 @@ def linear_pair(xa, wa, ba, xb, wb, bb):
         if bias is not None and (bias.dtype != torch.float32 or not bias.is_contiguous()):
             bias = bias.contiguous().float()
         out = torch.empty((M, N), dtype=torch.float32, device=x.device)
-        packed = _packed_weight(weight if weight is w else w, ldw, mode) if _pack_weights else None
+        packed = _packed_weight(weight if weight is w else w, ldw, mode)
         pr = arr[q]
         pr.X, pr.M, pr.ldx = x.data_ptr(), M, ldx
         pr.W, pr.N, pr.ldw = w.data_ptr(), N, ldw
-        pr.packed_w = packed.data_ptr() if packed is not None else None
+        pr.packed_w = packed.data_ptr()
         pr.bias = bias.data_ptr() if bias is not None else None
         pr.row_scale, pr.relu = None, 0
         pr.Y, pr.ldy, pr.y_dtype = out.data_ptr(), N, L.F32
@@ -646,33 +642,6 @@ def set_attention_path(path: str):
     L.check(L.lib().b200rec_attention_pool_set_path({'auto': 0, 'registers': 1, 'tma': 2}[path]), 'attention_pool_set_path')
 
 
-class AttentionPrepared:
-    """Workspace of `attention_pool_raw` with its first phase (compaction of the dense user_matrix + work list) already
-    launched — see `attention_prepare`."""
-
-    def __init__(self, ws, um, shape, U):
-        self.ws, self.um, self.shape, self.U = ws, um, shape, U
-
-
-def attention_prepare(user_matrix, U):
-    """Launches K2's first phase for a dense `(B, I)` user_matrix on the CURRENT stream (b200rec_attention_pool_prepare).  It reads
-    nothing but the matrix, so AttentionNCF runs it on a side stream next to the projection GEMMs and joins before
-    `attention_pool_raw(..., prepared=...)`."""
-    _require_cuda(user_matrix)
-    um, ld = _row_major(user_matrix)
-    B, I = um.shape
-    d = L.AttentionDesc()
-    d.user_matrix, d.ld_user_matrix = um.data_ptr(), ld
-    d.B, d.I, d.U = B, I, U
-    wsb = L.lib().b200rec_attention_pool_workspace(B, I, U, 1)
-    ws = torch.empty(max(wsb, 16), dtype=torch.uint8, device=um.device)
-    d.workspace, d.workspace_bytes = ws.data_ptr(), wsb
-    if B > 0 and I > 0:
-        with _on(um.device), _timed('attention_prepare', (B, I)):
-            L.check(L.lib().b200rec_attention_pool_prepare(C.byref(d), _stream()), 'attention_pool_prepare')
-    return AttentionPrepared(ws, um, (B, I), U)
-
-
 def _set_dropout_seed(d, seed, device):
     """`seed`: a Python int (baked into the launch), or a one-element int64 CUDA tensor the kernels read at run time — what a captured CUDA graph
     needs, since a replay must draw a new mask (the tensor is produced by torch's graph-safe generator inside the capture)."""
@@ -686,7 +655,7 @@ def _set_dropout_seed(d, seed, device):
 
 def attention_pool_raw(Pc, Pr, Q, *, mode=L.ATT_NET, a2=None, a20=None, bU=None, user_matrix=None, csr=None,
                        return_attention_weights=False, train_mask=None, drop_zero_scores=False, score_scale=1.0, use_workspace=True, max_row_nnz=0,
-                       prepared=None, inner_dropout=None):
+                       inner_dropout=None):
     """out (B,U) [, att (B,I)] — b200rec_attention_pool.  `csr` = (row_ptr int32, col int32, val fp32); `max_row_nnz` (CSR only,
     optional) = a host-known bound of the row lengths, so that the segment grid is not sized by I."""
     _require_cuda(Pc, Pr, Q, user_matrix)
@@ -712,10 +681,6 @@ def attention_pool_raw(Pc, Pr, Q, *, mode=L.ATT_NET, a2=None, a20=None, bU=None,
             t = t.detach().contiguous().float().view(-1)
             keep.append(t)
             setattr(d, name, t.data_ptr())
-    if prepared is not None and (prepared.shape != (B, I) or prepared.U != U or B == 0 or I == 0):
-        prepared = None
-    if prepared is not None:
-        user_matrix = prepared.um
     if user_matrix is not None:
         um, ld = _row_major(user_matrix)
         if um.shape != (B, I):
@@ -735,10 +700,7 @@ def attention_pool_raw(Pc, Pr, Q, *, mode=L.ATT_NET, a2=None, a20=None, bU=None,
         wsb = L.lib().b200rec_attention_pool_workspace_csr(B, I, U, d.max_row_nnz, d.nnz) if use_workspace else 0
     else:
         wsb = L.lib().b200rec_attention_pool_workspace(B, I, U, 1) if use_workspace else 0
-    if prepared is not None:
-        keep.append(prepared.ws)
-        d.workspace, d.workspace_bytes, d.prepared = prepared.ws.data_ptr(), prepared.ws.numel(), 1
-    elif wsb:
+    if wsb:
         ws = torch.empty(wsb, dtype=torch.uint8, device=Pc.device)
         keep.append(ws)
         d.workspace, d.workspace_bytes = ws.data_ptr(), wsb
@@ -826,17 +788,14 @@ def spmm_raw(index, t, *, w, dinv=None, x_next=None, acc_in=None, acc_out=None, 
         L.check(L.lib().b200rec_spmm(C.byref(d), _stream()), 'spmm')
 
 
-SPMM_STREAM = os.environ.get('B200REC_SPMM_STREAM', '1') == '1'      # inference SpMM: edge-balanced stream kernel where it applies
-
-
-STREAM_MAX_NNZ = int(os.environ.get('B200REC_SPMM_STREAM_MAX_NNZ', str(16_000_000)))
+STREAM_MAX_NNZ = 16_000_000
 
 
 def stream_applicable(t, nnz, *, skip_bits=None, att_src=None):
     """the stream kernel covers LightGCN inference with 64 < node_emb <= 128 (a lane owns 4 columns) on indices of up to STREAM_MAX_NNZ
     entries — the shards of a partitioned graph, where it is 5-15 % faster (profiles/r02); narrower rows and the whole 50 M-entry graph
     (1.43 vs 1.42 ms per layer) keep the row-owner kernel"""
-    return (SPMM_STREAM and skip_bits is None and att_src is None and 64 < t.shape[1] <= 128 and t.shape[1] % 4 == 0 and 0 < nnz <= STREAM_MAX_NNZ)
+    return (skip_bits is None and att_src is None and 64 < t.shape[1] <= 128 and t.shape[1] % 4 == 0 and 0 < nnz <= STREAM_MAX_NNZ)
 
 
 def spmm_stream_raw(plan, t, *, x_next=None, acc_in=None, acc_out=None, acc_scale=1.0, push=None):
@@ -986,7 +945,7 @@ def propagate_gat(t, ps, index, skip_bits=None):
 # ------------------------------------------------------------------------------------------------------------------
 # K2 autograd wrapper
 # ------------------------------------------------------------------------------------------------------------------
-ATT_BWD_SLICES = int(os.environ.get('B200REC_ATT_BWD_SLICES', '4'))   # CTAs per candidate row in K2's backward: 0.170 ms (1) / 0.116 (4) / 0.114 (8) at config 2
+ATT_BWD_SLICES = 4   # CTAs per candidate row in K2's backward: 0.170 ms (1) / 0.116 (4) / 0.114 (8) at config 2
 
 
 def _f32_rows(t):
@@ -1269,9 +1228,6 @@ def allpairs_topk_raw(A, B, packed, mode, k, *, return_scores=False, seen=None, 
     return val, idx, scores
 
 
-RELU_DOT_ALWAYS = os.environ.get('B200REC_RELU_DOT_ALWAYS', '1') == '1'
-
-
 def allpairs_relu_dot_raw(A, B, w2, b2, k, *, return_scores=False, seen=None, n_splits=0):
     """score(u, i) = b2 + w2·ReLU(A[u] + B[i]) for every pair + the k best columns per row — b200rec_allpairs_relu_dot_topk (exact fp32)."""
     _require_cuda(A, B, w2)
@@ -1330,16 +1286,10 @@ def mlp_allpairs_topk(row_emb, col_emb, weights, biases, k, *, rows_first=True, 
         W2, b2, w3, b3 = weights[1], biases[1], weights[2], biases[2]
         if W2.shape[0] > 128:
             raise NotImplementedError(f'all-pairs kernel: second hidden width {W2.shape[0]} > 128')
-    elif precision == 'fp32' or RELU_DOT_ALWAYS:
-        # one hidden layer: score = b2 + w2·ReLU(a_u + b_i) has no GEMM left — exact FP32 kernel (csrc/allpairs.cu, relu_dot).  It is also FASTER
-        # than the 2-row tensor-core trick below (0.47 s vs 0.83 s per 1.25e10 pairs), so the bf16 request takes it too (exact is within 1e-2).
-        return allpairs_relu_dot_raw(A, Bm, weights[1].detach(), biases[1], k, return_scores=return_scores, seen=seen, n_splits=n_splits)
     else:
-        # one hidden layer: score = w2·h1 + b2 = ReLU(w2·h1) - ReLU(-w2·h1) + b2 — two rows of the generic second layer
-        w2 = weights[1].detach().view(1, -1)
-        W2 = torch.cat((w2, -w2), 0)
-        b2 = torch.zeros(2, dtype=torch.float32, device=dev)
-        w3 = torch.tensor([1.0, -1.0], dtype=torch.float32, device=dev)
-        b3 = biases[1]
+        # one hidden layer: score = b2 + w2·ReLU(a_u + b_i) has no GEMM left — exact FP32 kernel (csrc/allpairs.cu, relu_dot).  It is also FASTER
+        # than running it as two rows of the tensor-core kernel's second layer (0.47 s vs 0.83 s per 1.25e10 pairs), so the bf16 request takes it
+        # too (exact is within 1e-2).
+        return allpairs_relu_dot_raw(A, Bm, weights[1].detach(), biases[1], k, return_scores=return_scores, seen=seen, n_splits=n_splits)
     packed = allpairs_pack(W2, b2, w3, b3, H1p, mode)
     return allpairs_topk_raw(A, Bm, packed, mode, k, return_scores=return_scores, seen=seen, n_splits=n_splits)

@@ -43,8 +43,6 @@ _CTRL_BYTES = 4096                 # flags uint32[16][16] (1 KB) | counters uint
 _OFF_COUNTERS = L.PEER_CHANNELS * L.PEER_MAX * 4
 _OFF_ERR = _OFF_COUNTERS + 2 * L.PEER_CHANNELS * 4
 WAIT_TIMEOUT_NS = 10_000_000_000
-# the item side of a layer (wait for the partials, slot reduction, transform + broadcast) runs on a second stream under the user-row SpMM
-OVERLAP = os.environ.get('B200REC_PEER_OVERLAP', '1') == '1'
 TRACE = os.environ.get('B200REC_PEER_TRACE', '0') == '1'
 
 
@@ -361,8 +359,7 @@ def _steps(model, sh: PeerShard, userIds, itemIds, keep=None):
         spare_u = empty(nu) if L_ > 1 else None
         xi_next = empty(ni) if L_ > 1 else None
         main = torch.cuda.current_stream(dev)
-        side = sh.side_stream() if OVERLAP else None
-        joined = None
+        side = sh.side_stream()
         # Layer 0's messages straight from the node features: t0 = dinv ∘ (W_t (W_e f + b_e) + b_t) = dinv ∘ ((W_t W_e) f + (W_t b_e + b_t)) — composite
         # weights formed once per weight version in float64.  So the first SpMM waits for ONE transform only; the embeddings x0 (needed from the
         # first running-mean update on) and the broadcast of the item messages run on the side stream underneath it.
@@ -375,17 +372,13 @@ def _steps(model, sh: PeerShard, userIds, itemIds, keep=None):
             sh.signal(CH_T0)
             embed()
 
-        x0_ready = None
-        if side is not None:
-            start = torch.cuda.Event()
-            start.record(main)
-            side.wait_event(start)
-            with torch.cuda.stream(side):
-                layer0_side()
-                x0_ready = torch.cuda.Event()
-                x0_ready.record(side)
-        else:
+        start = torch.cuda.Event()
+        start.record(main)
+        side.wait_event(start)
+        with torch.cuda.stream(side):
             layer0_side()
+            x0_ready = torch.cuda.Event()
+            x0_ready.record(side)
 
         def item_side(l, par, last, scale):                                          # C_l: needs every rank's A_l, nothing of B_l
             sh.stamp(f'C{l} begin')
@@ -405,31 +398,25 @@ def _steps(model, sh: PeerShard, userIds, itemIds, keep=None):
                 ops.propagate_step(sh.index_items, t_users, dinv=sh.dinv_items_all, push=sh.push_spec(par, d))
             sh.signal(CH_A0 + par)
             sh.stamp(f'A{l} end')
-            if side is not None:
-                forked = torch.cuda.Event()
-                forked.record(main)
+            forked = torch.cuda.Event()
+            forked.record(main)
             yield
-            if side is not None:                                                     # C_l on the side stream, under B_l
-                side.wait_event(forked)
-                with torch.cuda.stream(side):
-                    item_side(l, par, last, scale)
-                    joined = torch.cuda.Event()
-                    joined.record(side)
+            side.wait_event(forked)                                                  # C_l on the side stream, under B_l
+            with torch.cuda.stream(side):
+                item_side(l, par, last, scale)
+                joined = torch.cuda.Event()
+                joined.record(side)
             sh.wait(CH_T0 + par)
-            if l == 0 and x0_ready is not None:
+            if l == 0:
                 main.wait_event(x0_ready)                                            # x0_users is B_0's running-mean input
             sh.stamp(f'B{l} table arrived')
             if nu:                                                                   # B_l: own user rows from the gathered table
                 ops.propagate_step(sh.index_users, sh.table(par, d, t_dtype), dinv=sh.dinv_users, x_next=None if last else spare_u,
                                    acc_in=x0_users if l == 0 else acc_users, acc_out=acc_users, acc_scale=scale)
-            if side is None:
-                yield
-                item_side(l, par, last, scale)
             sh.stamp(f'B{l} end')
             if not last and nu:
                 ops.linear_raw(spare_u, lin_u.weight, lin_u.bias, row_scale=sh.dinv_users, out=t_users[:nu])
-        if joined is not None:
-            main.wait_event(joined)
+        main.wait_event(joined)
         sh.stamp('layers joined')
     if keep is not None:                        # tests: the owned rows of the combined embedding
         keep['items'], keep['users'] = acc_items, acc_users

@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define B200REC_VERSION 203
+#define B200REC_VERSION 204
 
 typedef void* b200rec_stream_t; /* cudaStream_t */
 
@@ -51,7 +51,8 @@ int b200rec_linear(const float* X, int64_t M, int64_t K, int64_t ldx, const floa
                    b200rec_stream_t stream);
 
 /* Same contract on the tensor cores (tcgen05.mma, TMEM accumulators; csrc/gemm_tc.cu).  mode B200REC_TC_TF32X3: fp32-parity
- * 3xTF32 split (rel <= 1e-5); B200REC_TC_BF16: bf16 operands (rel <= 1e-2).  Needs no workspace; meant for M >= ~1024.
+ * 3xTF32 split (rel <= 1e-5); B200REC_TC_BF16: bf16 operands (rel <= 1e-2).  Meant for M >= ~1024.  The weights come from `packed_w`
+ * (b200rec_pack_weights_tc of W, same mode), which is required: NULL returns B200REC_ERR_BAD_ARG.  W and ldw are not read.
  * `row_index` (M int64, or NULL): GEMM row m reads row row_index[m] of an X table of `x_rows` rows — the gather of
  * `item_profiles[rated_items_ids]` (src/content_providers/dynamic_profiles_provider.py:70) fused into the projection. */
 int b200rec_linear_tc(const float* X, int64_t M, int64_t K, int64_t ldx, const float* W, int64_t N, int64_t ldw, const float* bias,
@@ -60,7 +61,7 @@ int b200rec_linear_tc(const float* X, int64_t M, int64_t K, int64_t ldx, const f
 /* Split-K form for SHORT-M, long-K GEMMs (a 512-pair batch against the F = 2094 profiles: 4 x 2 output tiles would occupy 8 of 148
  * SMs): the k-blocks are dealt out over ~SMs / tiles CTAs per output tile, every CTA leaves a raw fp32 tile in `workspace`
  * (b200rec_linear_tc_splitk_workspace bytes; 0 = the shape is not split and none is needed) and a second kernel adds the slabs in
- * split order (deterministic) and applies bias / row_scale / ReLU.  N % 4 == 0 to be split. */
+ * split order (deterministic) and applies bias / row_scale / ReLU. */
 size_t b200rec_linear_tc_splitk_workspace(int64_t M, int64_t N, int64_t K, int mode);
 int b200rec_linear_tc_splitk(const float* X, int64_t M, int64_t K, int64_t ldx, const float* W, int64_t N, int64_t ldw, const float* bias,
                              const float* row_scale, int relu, void* Y, int64_t ldy, int y_dtype, int mode, const void* packed_w,
@@ -106,7 +107,7 @@ int b200rec_dense_nnz_count(const float* X, int64_t M, int64_t ldx, int64_t c0, 
 int b200rec_dense_nnz_fill(const float* X, int64_t M, int64_t ldx, int64_t c0, int64_t c1, const int* row_ptr, int* col, float* val,
                            b200rec_stream_t stream);
 /* Up to four such GEMMs sharing K and mode in ONE launch (candidate + rated-item projections, the two halves of
- * AttentionNet.0 — attention_ncf.py:150-151,176): problem q covers its own rows; fields as in b200rec_linear_tc. */
+ * AttentionNet.0 — attention_ncf.py:150-151,176): problem q covers its own rows; fields as in b200rec_linear_tc (`packed_w` required). */
 typedef struct {
   const float* X; int64_t M; int64_t ldx;
   const float* W; int64_t N; int64_t ldw; const void* packed_w;
@@ -119,8 +120,8 @@ int b200rec_linear_tc_batch(const b200rec_linear_problem_t* problems, int n_prob
 size_t b200rec_linear_tc_splitk_batch_workspace(const b200rec_linear_problem_t* problems, int n_problems, int64_t K, int mode);
 int b200rec_linear_tc_splitk_batch(const b200rec_linear_problem_t* problems, int n_problems, int64_t K, int mode, void* workspace,
                                    size_t workspace_bytes, b200rec_stream_t stream);
-/* Optional: W converted once into MMA-ready swizzled tiles (bf16, TF32 hi/lo or bf16 hi/lo, zero-padded).  With `packed_w` the GEMM moves
- * the W operand by TMA bulk copies (cp.async.bulk) and only X is converted by the producer warps.  128-byte aligned buffer. */
+/* W converted once into MMA-ready swizzled tiles (bf16, TF32 hi/lo or bf16 hi/lo, zero-padded): the `packed_w` of the tensor-core GEMMs,
+ * which move it by TMA bulk copies (cp.async.bulk) while the producer warps convert X.  128-byte aligned buffer. */
 size_t b200rec_packed_weight_bytes(int64_t N, int64_t K, int mode);
 int b200rec_pack_weights_tc(const float* W, int64_t N, int64_t K, int64_t ldw, int mode, void* packed, size_t packed_bytes,
                             b200rec_stream_t stream);
@@ -217,7 +218,6 @@ typedef struct {
   size_t workspace_bytes; /* of a dense matrix, work list of <=64-non-zero segments, one warp each, merge kernel); NULL = one fused kernel */
   int64_t max_row_nnz;    /* CSR form, optional: upper bound of a row's length (0 = unknown, I is used) and the number of stored entries */
   int64_t nnz;            /* (0 = unknown).  They only size the work list / partial slots: b200rec_attention_pool_workspace_csr(). */
-  int prepared;           /* 1 = b200rec_attention_pool_prepare already ran on this workspace for this user_matrix / CSR */
   int64_t ld_pc;          /* leading dimension of Pc in elements (a column slice of the [Ec | Pc] projection is used in place); 0 = H */
   float dropout_p;        /* training only, b200rec_attention_pool_dropout: p of the Dropout between AttentionNet's ReLU and its head Linear */
   uint64_t dropout_seed;  /* (attention_ncf.py:112-117); mask = Philox2x32-10 keyed by the seed, regenerated by the backward kernel */
@@ -247,10 +247,6 @@ int b200rec_attention_recommend(const float* Pc, int64_t ld_pc, const float* Pr,
  * round((1 - dropout_p)·65536) / 65536, one Philox2x32-10 call (counter = (i, b·64 + hidden group), key = seed) per 4 hidden units
  * (csrc/common.cuh).  A separately compiled copy of the kernels (csrc/attention_pool_drop.cu): the scoring build above is untouched. */
 int b200rec_attention_pool_dropout(const b200rec_attention_t* a, b200rec_stream_t stream);
-/* First phase of the segment-parallel path on its own: compaction of the dense matrix / work list into `workspace`.  It reads only
- * user_matrix (or the CSR) — B, I, U, the matrix fields and the workspace of `a` must be set, the tables may be NULL — so a host can
- * launch it on a second stream while the projection GEMMs run, then call b200rec_attention_pool with the same workspace and prepared = 1. */
-int b200rec_attention_pool_prepare(const b200rec_attention_t* a, b200rec_stream_t stream);
 /* How the segment-parallel path gathers table rows: 0 = auto (TMA bulk copies into shared memory when the tables exceed half of L2,
  * register-staged 128-bit loads otherwise), 1 = always registers, 2 = TMA whenever the layout allows (H, U <= 128, 16-byte rows). */
 int b200rec_attention_pool_set_path(int path);

@@ -52,6 +52,16 @@ def test_workspace_queries_run_without_gpu():
     assert lib.b200rec_scan_workspace(10_000_000) > 0
     assert lib.b200rec_sort_pairs_workspace(1 << 20) >= 2 * 4 * (1 << 20)
     assert lib.b200rec_csr_workspace(1000, 100) > 0
+    # argument checks run on the host too: the tensor-core GEMMs refuse a NULL packed_w before any launch
+    X, W, Y = 256, 512, 768                                   # never dereferenced
+    with pytest.raises(ValueError, match='packed'):
+        _lib.check(lib.b200rec_linear_tc(X, 128, 64, 64, W, 64, 64, None, None, 0, Y, 64, _lib.F32, _lib.TC_TF32X3, None, None, 0, None), 'linear_tc')
+    with pytest.raises(ValueError, match='packed'):
+        _lib.check(lib.b200rec_linear_tc_splitk(X, 128, 64, 64, W, 64, 64, None, None, 0, Y, 64, _lib.F32, _lib.TC_TF32X3, None, None, 0, None),
+                   'linear_tc_splitk')
+    prob = _lib.LinearProblem(X=X, M=128, ldx=64, W=W, N=64, ldw=64, packed_w=None, Y=Y, ldy=64, y_dtype=_lib.F32)
+    with pytest.raises(ValueError, match='packed'):
+        _lib.check(lib.b200rec_linear_tc_batch(ctypes.byref(prob), 1, 64, _lib.TC_TF32X3, None), 'linear_tc_batch')
 
 
 @pytest.mark.skipif(torch.cuda.is_available(), reason='checks the no-GPU behaviour')

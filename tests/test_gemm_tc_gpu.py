@@ -140,22 +140,17 @@ def test_linear_pair_batched_splitk(Ma, Mb, K, Na, Nb):
 
 
 @pytest.mark.parametrize('M,K,N', [(9461, 2094, 256), (2500, 2094, 256), (4096, 512, 384 + 128), (3000, 1000, 130), (2049, 2094, 200)])
-def test_linear_tc_wide_tiles_fp32_parity(M, K, N):
+def test_linear_tc_wide_tiles_fp32_parity_vs_128_tiles(M, K, N):
     """128 x 256 tiles + split-K (b200rec_linear_tc_wide): the default route of large-M GEMMs with 128 < N.  Same fp32 tolerance as the
     128 x 128 form, deterministic, agrees with it to fp32 rounding; row_index gather, bias / row scale / ReLU after the slab reduction."""
     from deeprecommendation_b200 import ops
     x, w, b, s = _case(M, K, N, M + N)
     ref = torch.nn.functional.linear(x.double(), w.double(), b.double())
     xd, wd, bd, sd = x.cuda(), w.cuda(), b.cuda(), s.cuda()
-    assert ops.TC_WIDE
     y = ops.linear_raw(xd, wd, bd, engine='tf32x3!')
     assert maxnorm_rel(y, ref) < 1e-5
     assert torch.equal(y, ops.linear_raw(xd, wd, bd, engine='tf32x3!'))
-    ops.TC_WIDE = False
-    try:
-        y128 = ops.linear_raw(xd, wd, bd, engine='tf32x3!')
-    finally:
-        ops.TC_WIDE = True
+    y128 = ops.linear_tc_batch([(xd, wd, bd, None)], engine='tf32x3')[0]          # the 128 x 128 tiles
     assert maxnorm_rel(y, y128) < 2e-6
     out = torch.full((M, N + 8), 3.0, device='cuda')
     ops.linear_raw(xd, wd, bd, sd, True, out=out[:, 4:4 + N], engine='tf32x3!')

@@ -582,28 +582,6 @@ def test_attention_forward_resident_equals_dense_forward():
         assert torch.equal(att_d, att_r), engine
 
 
-def test_attention_overlap_prepare_equals_default():
-    """AttentionNCF.overlap_prepare (K2's first phase through b200rec_attention_pool_prepare on a side stream, `prepared = 1`)
-    gives the same bits as the single-stream path, eagerly and replayed from a captured CUDA graph."""
-    d, _, kw = load('attention_full')
-    wkw = {k: v for k, v in kw.items() if k not in ('use_cos_sim_instead', 'message_dropout')}
-    m = _models().AttentionNCF(**kw).to(DEV).eval()
-    m.load_state_dict(synth.to_torch(synth.attention_ncf_weights(seed=int(d['weight_seed']), **wkw)))
-    cand, rated, um = (torch.from_numpy(a).to(DEV) for a in attention_full_inputs(d))
-    with torch.no_grad():
-        ref_out, ref_att = m(cand, rated, um, return_attention_weights=True)
-        m.overlap_prepare = True
-        out, att = m(cand, rated, um, return_attention_weights=True)
-        assert torch.equal(out, ref_out) and torch.equal(att, ref_att)
-        torch.cuda.synchronize()
-        g = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(g):
-            gout = m(cand, rated, um)
-        g.replay()
-        torch.cuda.synchronize()
-        assert torch.equal(gout, ref_out)
-
-
 @pytest.mark.parametrize('masked', [False, True])
 def test_lightgat_gradients_vs_oracle_autograd(masked):
     """LightGATConv training step (gnn_ncf.py:97-177 under train.py:99-105): forward on K3's edge-softmax kernel, closed-form backward

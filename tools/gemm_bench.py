@@ -12,13 +12,15 @@ for M, K, N in SHAPES:
     for eng in ('simt', 'tf32x3', 'tf32x3!', 'tf32x3!narrow', 'bf16x3!', 'bf16!') + (('shortk!',) if K <= 128 else ()):
         if eng == 'tf32x3!narrow' and N <= 128:
             continue
-        ops.TC_WIDE = eng != 'tf32x3!narrow'
-        eng_call = 'tf32x3!' if eng == 'tf32x3!narrow' else eng
+        if eng == 'tf32x3!narrow':                      # the 128 x 128 tiles that the wide form replaces for 128 < N
+            run = lambda: ops.linear_tc_batch([(x, w, b, None)], engine='tf32x3')
+        else:
+            run = lambda: ops.linear_raw(x, w, b, engine=eng)
         ts = []
         for r in range(7):
             flush.zero_()
             a, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            a.record(); ops.linear_raw(x, w, b, engine=eng_call); e.record(); torch.cuda.synchronize()
+            a.record(); run(); e.record(); torch.cuda.synchronize()
             ts.append(a.elapsed_time(e))
         ms = sorted(ts)[len(ts) // 2]
         gb = 4.0 * (M * K + N * K + M * N) / 1e9
