@@ -12,7 +12,7 @@ OK, ERR_CUDA, ERR_BAD_ARG, ERR_UNSUPPORTED, ERR_WORKSPACE = 0, 1, 2, 3, 4
 F32, BF16 = 0, 1
 ATT_NET, ATT_DOT = 0, 1
 TC_TF32X3, TC_BF16, TC_BF16X3 = 0, 1, 2
-ABI_VERSION = 204          # B200REC_VERSION of include/b200rec.h these bindings were written against (checked when the library is loaded)
+ABI_VERSION = 205          # B200REC_VERSION of include/b200rec.h these bindings were written against (checked when the library is loaded)
 AP_BF16, AP_BF16X2 = 0, 1
 MLP_MAX_LAYERS = 8
 PEER_MAX, PEER_CHANNELS, PEER_HANDLE_BYTES = 16, 16, 64
@@ -106,6 +106,11 @@ SIGNATURES = {
     'b200rec_attention_recommend_workspace': (c_sz, [c_i64, c_i64, c_int]),
     'b200rec_attention_recommend': (c_int, [c_vp, c_i64, c_vp, c_i64, c_int, c_int, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_int, c_i64, c_vp, c_vp, c_vp,
                                             c_vp, c_i64, c_vp, c_i64, c_vp]),
+    'b200rec_attention_explain_workspace': (c_sz, [c_i64, c_int]),
+    'b200rec_attention_explain_count': (c_int, [c_vp, c_i64, c_vp, c_i64, c_int, c_int, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_int,
+                                                C.c_double, C.c_double, c_vp, c_vp, c_sz, c_vp]),
+    'b200rec_attention_explain_fill': (c_int, [c_vp, c_i64, c_vp, c_i64, c_int, c_int, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_int,
+                                               c_vp, c_vp, c_sz, c_vp, c_vp, c_vp]),
     'b200rec_spmm': (c_int, [C.POINTER(SpmmDesc), c_vp]),
     'b200rec_spmm_stream': (c_int, [C.POINTER(SpmmStreamDesc), c_vp]),
     'b200rec_scan_workspace': (c_sz, [c_i64]),

@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 LIB = os.path.join(os.path.dirname(HERE), 'libb200rec.so')
 NVCC = os.environ.get('NVCC', '/usr/local/cuda/bin/nvcc')
-SOURCES = ['api.cu', 'gemm_f32.cu', 'gemm_tc.cu', 'mlp_tower.cu', 'attention_pool.cu', 'attention_pool_bwd.cu', 'spmm.cu', 'graph_build.cu', 'topk.cu', 'allpairs.cu', 'node_gemm.cu', 'peer.cu', 'gather_sum.cu', 'spmm_stream.cu', 'attention_pool_drop.cu', 'collate.cu', 'neg_sample.cu', 'attention_recommend.cu']
+SOURCES = ['api.cu', 'gemm_f32.cu', 'gemm_tc.cu', 'mlp_tower.cu', 'attention_pool.cu', 'attention_pool_bwd.cu', 'spmm.cu', 'graph_build.cu', 'topk.cu', 'allpairs.cu', 'node_gemm.cu', 'peer.cu', 'gather_sum.cu', 'spmm_stream.cu', 'attention_pool_drop.cu', 'collate.cu', 'neg_sample.cu', 'attention_recommend.cu', 'attention_explain.cu']
 FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17', '-Xcompiler', '-fPIC',
          '--expt-relaxed-constexpr', '-I', os.path.join(ROOT, 'include')]
 

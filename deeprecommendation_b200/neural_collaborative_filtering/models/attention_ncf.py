@@ -392,24 +392,59 @@ class AttentionNCF(NCF):
                 val[s:s + n], idx[s:s + n] = ops.topk_rows(sc, k)
         return (val, idx, scores) if return_scores else (val, idx)
 
+    def explain(self, item_profiles, list_ptr, list_item, list_val, items, users=None, explain_factor=1.5, explain_constant=0.025):
+        """Explanations of many users' recommendations: the reference's "because you liked ..." (src/webapp/backend.py:102-110) for the output
+        of `recommend`, in one call.  `val, idx = m.recommend(...)` followed by `m.explain(..., idx, users=...)` covers the whole serving call.
+
+        item_profiles, list_ptr, list_item, list_val and `users` as for `recommend`.  `items` (len(users), k) int64 catalogue rows, 1 <= k <= 64,
+        -1 = padding (exactly `recommend`'s top_items; any catalogue row is accepted, also a user's own list items).  Entry i of user u's list
+        explains candidate b when α_bi > explain_factor / max(R_u, 1) + explain_constant — `recommend_for_user`'s rule: R_u = length of u's list,
+        zero-centred entries included; α_bi = the eval-mode attention weight `forward(..., return_attention_weights=True)` reports.
+        Zero-centred entries have α = 0 and never explain; an empty list explains nothing.
+
+        K9 (csrc/attention_explain.cu) on `recommend`'s cached catalogue tables: after a `recommend` call on the same profiles and weights no
+        projection GEMM runs.  Returns (ptr (nU·k + 1,) int64, because (n,) int64 catalogue rows, attention (n,) fp32): row u·k + j explains
+        items[u, j] with because[ptr[r]:ptr[r+1]], in list order (ascending catalogue row); padding rows are empty."""
+        if self.training:
+            raise RuntimeError('explain() is an inference call: model.eval() first')
+        ops._require_cuda(item_profiles, list_ptr, list_item, list_val, users, items)
+        if list_ptr.dtype != torch.int64 or list_item.dtype != torch.int32 or list_val.dtype != torch.float32:
+            raise ValueError('explain(): list_ptr must be int64, list_item int32 and list_val float32')
+        if items.dtype != torch.int64 or items.dim() != 2:
+            raise ValueError('explain(): items must be a (len(users), k) int64 tensor')
+        if not 1 <= items.shape[1] <= 64:
+            raise ValueError('explain(): need 1 <= k <= 64')
+        dev = item_profiles.device
+        nI = item_profiles.shape[0]
+        users = torch.arange(max(list_ptr.numel() - 1, 0), device=dev) if users is None else users.to(dev).long().contiguous()
+        if items.shape[0] != users.numel():
+            raise ValueError(f'explain(): items has {items.shape[0]} rows for {users.numel()} users')
+        self._check_lists(list_ptr, list_item, list_val, users, nI, 'explain')
+        if items.numel() and bool(((items < -1) | (items >= nI)).any()):
+            raise ValueError(f'explain(): items must hold catalogue rows in [0, {nI}) or -1')
+        with torch.no_grad():
+            Pc, Pr, mode, a2, a20 = self._recommend_tables(item_profiles)[:5]
+            return ops.attention_explain_raw(Pc, Pr, mode=mode, a2=a2, a20=a20, list_ptr=list_ptr, list_item=list_item, list_val=list_val,
+                                             users=users, items=items, explain_factor=explain_factor, explain_constant=explain_constant)
+
     @staticmethod
-    def _check_lists(list_ptr, list_item, list_val, users, nI):
-        """Host-side range checks of the rating lists and user rows (one device read-back): K8 reads `list_ptr[users]` and the table rows
+    def _check_lists(list_ptr, list_item, list_val, users, nI, what='recommend'):
+        """Host-side range checks of the rating lists and user rows (one device read-back): K8 and K9 read `list_ptr[users]` and the table rows
         `list_item[...]` without bounds checks."""
         n_rows = list_ptr.numel() - 1
         if n_rows < 0:
-            raise ValueError('recommend(): list_ptr needs at least one element')
+            raise ValueError(f'{what}(): list_ptr needs at least one element')
         z = torch.zeros((), dtype=torch.bool, device=list_ptr.device)
         flags = torch.stack((
             ((users < 0) | (users >= n_rows)).any() if users.numel() else z,
             (list_ptr[0] != 0) | (list_ptr[-1] > min(list_item.numel(), list_val.numel())) | ((list_ptr[1:] < list_ptr[:-1]).any() if n_rows else z),
             ((list_item < 0) | (list_item >= nI)).any() if list_item.numel() else z)).tolist()
         if flags[0]:
-            raise ValueError(f'recommend(): `users` must be list rows in [0, {n_rows})')
+            raise ValueError(f'{what}(): `users` must be list rows in [0, {n_rows})')
         if flags[1]:
-            raise ValueError('recommend(): list_ptr must start at 0, be non-decreasing and end within list_item / list_val')
+            raise ValueError(f'{what}(): list_ptr must start at 0, be non-decreasing and end within list_item / list_val')
         if flags[2]:
-            raise ValueError(f'recommend(): list_item must hold catalogue rows in [0, {nI})')
+            raise ValueError(f'{what}(): list_item must hold catalogue rows in [0, {nI})')
 
     @staticmethod
     def _mask_seen(scores, users, list_ptr, list_item):

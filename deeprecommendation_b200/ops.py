@@ -1086,6 +1086,52 @@ def attention_recommend_raw(Pc, Pr, Ai, Qp, *, mode, a2, a20, list_ptr, list_ite
     return out
 
 
+def attention_explain_raw(Pc, Pr, *, mode, a2, a20, list_ptr, list_item, list_val, users, items, explain_factor=1.5, explain_constant=0.025):
+    """The list entries i of user `users[u]` with α_bi > explain_factor · (1 / max(R_u, 1)) + explain_constant for every candidate b = items[u, j]
+    (src/webapp/backend.py:102-110) — b200rec_attention_explain_count, one read-back of the total, b200rec_attention_explain_fill.
+    Pc / Pr / mode / a2 / a20 and the rating lists as for `attention_recommend_raw`; `items` (nU, k) int64 catalogue rows, 1 <= k <= 64, rows
+    outside [0, nI) are padding.  Returns (ptr (nU·k + 1,) int64, because (n,) int64 catalogue rows, attention (n,) fp32): row u·k + j explains
+    items[u, j], its entries in list order."""
+    _require_cuda(Pc, Pr, a2, a20, list_ptr, list_item, list_val, users, items)
+    if list_ptr.dtype != torch.int64 or users.dtype != torch.int64 or items.dtype != torch.int64:
+        raise ValueError('attention_explain: list_ptr, users and items must be int64')
+    if list_item.dtype != torch.int32:
+        raise ValueError('attention_explain: list_item must be int32')
+    if list_val.dtype != torch.float32:
+        raise ValueError('attention_explain: list_val must be float32')
+    nI, H = Pc.shape
+    if Pr.shape != (nI, H):
+        raise ValueError('attention_explain: table shapes disagree')
+    if items.dim() != 2 or items.shape[0] != users.numel():
+        raise ValueError('attention_explain: items must be (len(users), k)')
+    ld_pc, ld_pr = _check_rows(Pc, 'Pc'), _check_rows(Pr, 'Pr')
+    list_ptr, list_item, list_val, users, items = (t.contiguous() for t in (list_ptr, list_item, list_val, users, items))
+    if a2 is not None:
+        a2 = a2.detach().contiguous().float()
+    if a20 is not None:
+        a20 = a20.detach().contiguous().float()
+    nU, k = items.shape
+    dev = Pc.device
+    lib = L.lib()
+    ptr = torch.empty(nU * k + 1, dtype=torch.int64, device=dev)
+    wsb = int(lib.b200rec_attention_explain_workspace(nU, k))
+    ws = torch.empty(max(wsb, 16), dtype=torch.uint8, device=dev)
+    args = (_ptr(Pc), ld_pc, _ptr(Pr), ld_pr, H, int(mode), _ptr(a2), _ptr(a20), nI, _ptr(list_ptr), _ptr(list_item), _ptr(list_val), _ptr(users),
+            nU, _ptr(items), k)
+    with _on(dev):
+        with _timed('attention_explain_count', (nU, k, H)):
+            L.check(lib.b200rec_attention_explain_count(*args, float(explain_factor), float(explain_constant), _ptr(ptr), _ptr(ws), ws.numel(),
+                                                        _stream()), 'attention_explain_count')
+        n = int(ptr[-1].item())
+        because = torch.empty(n, dtype=torch.int64, device=dev)
+        attention = torch.empty(n, dtype=torch.float32, device=dev)
+        if n:
+            with _timed('attention_explain_fill', (nU, k, H)):
+                L.check(lib.b200rec_attention_explain_fill(*args, _ptr(ptr), _ptr(ws), ws.numel(), _ptr(because), _ptr(attention), _stream()),
+                        'attention_explain_fill')
+    return ptr, because, attention
+
+
 # ------------------------------------------------------------------------------------------------------------------
 # top-k
 # ------------------------------------------------------------------------------------------------------------------

@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define B200REC_VERSION 204
+#define B200REC_VERSION 205
 
 typedef void* b200rec_stream_t; /* cudaStream_t */
 
@@ -243,6 +243,26 @@ int b200rec_attention_recommend(const float* Pc, int64_t ld_pc, const float* Pr,
                                 const float* Ai, int64_t ld_ai, const float* Qp, int64_t ld_q, int H1P, int64_t n_items, const int64_t* list_ptr,
                                 const int32_t* list_item, const float* list_val, const int64_t* users, int64_t n_users, float* h1, int64_t ld_h1,
                                 b200rec_stream_t stream);
+/* ---- K9  AttentionNCF explanations of many users' recommendations (csrc/attention_explain.cu) -----------------------------------------
+ * Replaces the explanation step of src/webapp/backend.py:102-110 for k recommended items of each of many users: the entries i of user u's list
+ * with α_bi > explain_factor · (1 / max(R_u, 1)) + explain_constant (computed in double, compared in fp32), R_u = length of u's list, zero-centred
+ * entries included.  α_bi is K8's attention weight (same tables, same mode, same score arithmetic); zero-centred entries have α = 0 and never
+ * explain, an empty list explains nothing.
+ * items (n_users, k) int64 catalogue rows, 1 <= k <= 64; a row outside [0, n_items) (e.g. -1, K8's top-k padding) is padding and explains nothing.
+ * Row r = u·k + j of the output explains items[u, j]; its entries are in list order.  The other operands are those of b200rec_attention_recommend.
+ * Two calls on one stream, with the same operands and workspace (b200rec_attention_explain_workspace bytes):
+ *   _count  writes ptr (n_users·k + 1) int64: ptr[0] = 0, ptr[r+1] - ptr[r] = entries of row r;  the caller reads n = ptr[n_users·k]
+ *   _fill   writes because (n) int64 list items (catalogue rows) and attention (n) fp32 α at [ptr[r], ptr[r+1]).
+ * No atomics: bit-identical results run to run. */
+size_t b200rec_attention_explain_workspace(int64_t n_users, int k);
+int b200rec_attention_explain_count(const float* Pc, int64_t ld_pc, const float* Pr, int64_t ld_pr, int H, int mode, const float* a2, const float* a20,
+                                    int64_t n_items, const int64_t* list_ptr, const int32_t* list_item, const float* list_val, const int64_t* users,
+                                    int64_t n_users, const int64_t* items, int k, double explain_factor, double explain_constant, int64_t* ptr,
+                                    void* workspace, size_t workspace_bytes, b200rec_stream_t stream);
+int b200rec_attention_explain_fill(const float* Pc, int64_t ld_pc, const float* Pr, int64_t ld_pr, int H, int mode, const float* a2, const float* a20,
+                                   int64_t n_items, const int64_t* list_ptr, const int32_t* list_item, const float* list_val, const int64_t* users,
+                                   int64_t n_users, const int64_t* items, int k, const int64_t* ptr, const void* workspace, size_t workspace_bytes,
+                                   int64_t* because, float* attention, b200rec_stream_t stream);
 /* The same op with AttentionNet's inner Dropout applied in training mode: hidden = ReLU(Pc[b] + Pr[i]) ∘ m / keep, m ~ Bernoulli(keep), keep =
  * round((1 - dropout_p)·65536) / 65536, one Philox2x32-10 call (counter = (i, b·64 + hidden group), key = seed) per 4 hidden units
  * (csrc/common.cuh).  A separately compiled copy of the kernels (csrc/attention_pool_drop.cu): the scoring build above is untouched. */

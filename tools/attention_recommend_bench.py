@@ -1,4 +1,5 @@
-"""AttentionNCF.recommend (K8) at config 2 and on a catalogue larger than L2, against the per-user `recommend_for_user` loop in the same run.
+"""AttentionNCF.recommend (K8) and AttentionNCF.explain (K9) at config 2 and on a catalogue larger than L2, against the per-user
+`recommend_for_user` loop (which ranks and explains) in the same run.
 
     python tools/attention_recommend_bench.py [--out FILE.json] [--large-users N] [--large-items N]
 
@@ -102,6 +103,18 @@ def main():
         per_op[name] += sum(v)
     val, items, scores = model.recommend(*lists, k=10, return_scores=True)
 
+    # explanations of the same top-10 (K9), on the tables recommend() cached
+    for _ in range(2):
+        model.explain(*lists, items)
+    explain_warm = [timed(lambda: model.explain(*lists, items))[0] for _ in range(a.reps)]
+    timer = ops.OpTimer()
+    prev = ops.set_timer(timer)
+    for _ in range(a.reps):
+        expl = model.explain(*lists, items)
+    torch.cuda.synchronize()
+    ops.set_timer(prev)
+    explain_ops = {name: statistics.median(v) for (name, _), v in timer.summary().items()}
+
     # the per-user loop of the existing serving call, same users, end to end
     pos = [torch.from_numpy(idx[row_ptr[u]:row_ptr[u + 1]].astype(np.int64)).to(dev) for u in range(nU)]
     rat = [torch.from_numpy(rr[row_ptr[u]:row_ptr[u + 1]].astype(np.float64)).to(dev) for u in range(nU)]
@@ -110,6 +123,10 @@ def main():
     loop_ms, recs = timed(lambda: [model.recommend_for_user(prov.table, pos[u], rat[u], k=10) for u in range(nU)])
     same_items = sum(int(torch.equal(items[u], recs[u]['items'])) for u in range(nU))
     top_rel = max(float((val[u] - recs[u]['scores']).abs().max() / recs[u]['scores'].abs().max()) for u in range(nU))
+    e_ptr, e_because = expl[0].tolist(), expl[1]
+    same_because = sum(int(torch.equal(e_because[e_ptr[u * 10 + j]:e_ptr[u * 10 + j + 1]], recs[u]['because'][j]))
+                       for u in range(nU) for j in range(10) if torch.equal(items[u], recs[u]['items']))
+    loop_entries = sum(int(b.numel()) for r in recs for b in r['because'])
 
     # parity on sampled users against forward (K2 path) over the same (user, unseen item) pairs
     sample = np.random.default_rng(0).choice(nU, 16, replace=False)
@@ -139,6 +156,17 @@ def main():
         'top10_items_identical_to_loop_users': same_items, 'top10_scores_max_rel_vs_loop': top_rel,
         'parity_vs_forward_sampled_users': len(sample), 'parity_max_rel': max(par),
         'op_model': op_model(lens, nI, H, H1, clock_ghz),
+        'explain': {
+            'explain_ms_median': statistics.median(explain_warm), 'explain_ms_all': explain_warm,
+            'explain_over_recommend': statistics.median(explain_warm) / med,
+            'kernel_ms_median (CUDA events)': explain_ops,
+            'explanations': int(e_ptr[-1]), 'explanations_in_loop': loop_entries,
+            'rows_with_because_identical_to_loop': same_because, 'rows': nU * 10,
+            'op_model': {'what': 'ESTIMATE from shapes, not a measurement: 3 passes over each user list for each of its k candidates, ~3·H '
+                                 'lane-instructions per (candidate, entry) score',
+                         'lane_instructions': 3.0 * 10 * float(lens.sum()) * 3 * H,
+                         'longest_list_chunks_per_pass': int((lens.max() + 31) // 32)},
+        },
     }
     del model, prov, scores
     torch.cuda.empty_cache()
@@ -148,14 +176,17 @@ def main():
     model, prov, row_ptr, _, _ = setup(nUl, nIl, int(round(100_836 / 610 * nUl)), 7, 44, dev, whole_catalogue=True)
     lists = (prov.table, prov.d_list_ptr, prov.d_list_item, prov.d_list_val)
     nIl = prov.table.shape[0]
-    model.recommend(*lists, k=10)
+    _, top = model.recommend(*lists, k=10)
     times = [timed(lambda: model.recommend(*lists, k=10))[0] for _ in range(3)]
+    model.explain(*lists, top)
+    explain_times = [timed(lambda: model.explain(*lists, top))[0] for _ in range(3)]
     tables = model._recommend_tables(prov.table)
     table_bytes = tables[0].shape[0] * tables[0].stride(0) * 4          # the four tables are views of one (nI, N) GEMM output
     lens = np.diff(row_ptr)
     res['large_catalogue'] = {'users': nUl, 'items': nIl, 'list_entries': int(lens.sum()), 'tables_bytes': table_bytes,
                               'recommend_ms_median': statistics.median(times), 'recommend_ms_all': times,
-                              'pairs_per_s': nUl * nIl / (statistics.median(times) * 1e-3), 'op_model': op_model(lens, nIl, H, H1, clock_ghz)}
+                              'pairs_per_s': nUl * nIl / (statistics.median(times) * 1e-3), 'op_model': op_model(lens, nIl, H, H1, clock_ghz),
+                              'explain_top10_ms_median': statistics.median(explain_times), 'explain_top10_ms_all': explain_times}
     txt = json.dumps(res, indent=1)
     print(txt)
     if a.out:
