@@ -339,7 +339,8 @@ class AttentionNCF(NCF):
         self._rec_cache = (key, weakref.ref(item_profiles), out)
         return out
 
-    def recommend(self, item_profiles, list_ptr, list_item, list_val, k=10, users=None, ignore_seen=True, return_scores=False, chunk_users=None):
+    def recommend(self, item_profiles, list_ptr, list_item, list_val, k=10, users=None, ignore_seen=True, return_scores=False, chunk_users=None,
+                  precision='fp32'):
         """Top-k catalogue items for many users at once: the reference's serving call (src/webapp/backend.py:78-121, one user x every
         catalogue item, attention_ncf.py:136-224) batched over users.
 
@@ -352,9 +353,15 @@ class AttentionNCF(NCF):
 
         Pipeline per chunk: K8 (csrc/attention_recommend.cu: attention pooling over the shared list, h1 slab) on the cached catalogue tables
         (`_recommend_tables`), the remaining MLP layers on the slab (K1a), seen pairs set to NaN, `ops.topk_rows`.
+        precision 'fp32' (default, max-norm relative error <= 1e-5) or 'bf16' (<= 1e-2): the attention scores, the softmax and α are the fp32 ones,
+        bit for bit (so `explain` of a bf16 call's items is that of an fp32 call), the pooling runs on bf16 tensor cores (K8b: Q' and the
+        weights α·um rounded to bf16, fp32 accumulation) and the hidden layers after the first on K1a's bf16 engine; the output layer is the
+        fp32 path's.  The bf16 copy of Q' is made on the first bf16 call and cached with the catalogue tables.
         Returns (top_scores (nU, k) fp32, top_items (nU, k) int64 catalogue rows, padded with (-inf, -1)[, scores (nU, nI)])."""
         if self.training:
             raise RuntimeError('recommend() is an inference call: model.eval() first')
+        if precision not in ('fp32', 'bf16'):
+            raise ValueError(f"recommend(): precision must be 'fp32' or 'bf16', not {precision!r}")
         ops._require_cuda(item_profiles, list_ptr, list_item, list_val, users)
         if list_ptr.dtype != torch.int64 or list_item.dtype != torch.int32 or list_val.dtype != torch.float32:
             raise ValueError('recommend(): list_ptr must be int64, list_item int32 and list_val float32')
@@ -369,6 +376,12 @@ class AttentionNCF(NCF):
         weights, biases, _ = mlp_parameters(self.MLP)
         with torch.no_grad():
             Pc, Pr, mode, a2, a20, Ai, Qp, H1 = self._recommend_tables(item_profiles)
+            hidden = None
+            if precision == 'bf16':
+                if len(self._rec_cache) == 3:                          # the bf16 copy of Q' lives and dies with the cached tables
+                    self._rec_cache += (Qp.to(torch.bfloat16, memory_format=torch.contiguous_format),)
+                # K = H1 <= 256 is below ops.TC_MIN_K, where the default routing picks the FFMA GEMM: force the bf16 tensor cores
+                Qp, hidden = self._rec_cache[3], 'bf16!'
             H1P = Ai.shape[1]
             if chunk_users is None:
                 chunk_users = max(1, RECOMMEND_SLAB_BYTES // max(1, nI * H1P * 4))
@@ -384,7 +397,7 @@ class AttentionNCF(NCF):
                 x = ops.attention_recommend_raw(Pc, Pr, Ai, Qp, mode=mode, a2=a2, a20=a20, list_ptr=list_ptr, list_item=list_item,
                                                 list_val=list_val, users=uc)[:, :H1]
                 for li in range(1, last):
-                    x = ops.linear_raw(x, weights[li], biases[li], relu=True)
+                    x = ops.linear_raw(x, weights[li], biases[li], relu=True, engine=hidden)
                 ops.linear_raw(x, weights[last], biases[last], out=sc.view(n * nI, 1))
                 del x
                 if ignore_seen:                                        # item_features.drop(...) (backend.py:85): never selected by the top-k

@@ -1055,7 +1055,9 @@ def attention_recommend_raw(Pc, Pr, Ai, Qp, *, mode, a2, a20, list_ptr, list_ite
     """h1 = ReLU(Ai[b] + Σ_i softmax_i(s_bi)·val_i·Qp[i]) for every (user of `users`, catalogue row b) — b200rec_attention_recommend.
     Pc / Pr (nI, H) score tables (mode ATT_NET: s = a2·ReLU(Pc[b] + Pr[i]) + a20; ATT_DOT: s = <Pc[b], Pr[i]>); Ai / Qp (nI, H1P) with
     H1P in {32, 64, 128, 256}; the rating lists in K6's resident format (list_ptr int64, list_item int32, list_val fp32 centred); `users`
-    int64 list rows.  Returns (len(users)·nI, H1P) fp32, row u·nI + b (or fills `out` of that shape)."""
+    int64 list rows.  Returns (len(users)·nI, H1P) fp32, row u·nI + b (or fills `out` of that shape).
+    The dtype of Qp picks the kernel: fp32 runs K8; bf16 runs K8b (b200rec_attention_recommend_bf16: the same scores and α, the pooling
+    on bf16 tensor cores with the weights α·val rounded to bf16, fp32 accumulation)."""
     _require_cuda(Pc, Pr, Ai, Qp, a2, a20, list_ptr, list_item, list_val, users, out)
     if list_ptr.dtype != torch.int64 or users.dtype != torch.int64:
         raise ValueError('attention_recommend: list_ptr and users must be int64')
@@ -1067,7 +1069,17 @@ def attention_recommend_raw(Pc, Pr, Ai, Qp, *, mode, a2, a20, list_ptr, list_ite
     H1P = Ai.shape[1]
     if Pr.shape != (nI, H) or Ai.shape[0] != nI or Qp.shape != (nI, H1P):
         raise ValueError('attention_recommend: table shapes disagree')
-    ld_pc, ld_pr, ld_ai, ld_q = _check_rows(Pc, 'Pc'), _check_rows(Pr, 'Pr'), _check_rows(Ai, 'Ai'), _check_rows(Qp, 'Qp')
+    ld_pc, ld_pr, ld_ai = _check_rows(Pc, 'Pc'), _check_rows(Pr, 'Pr'), _check_rows(Ai, 'Ai')
+    lib = L.lib()
+    if Qp.dtype == torch.float32:
+        ld_q, entry, name = _check_rows(Qp, 'Qp'), lib.b200rec_attention_recommend, 'attention_recommend'
+    elif Qp.dtype == torch.bfloat16:
+        if Qp.dim() != 2 or Qp.stride(1) != 1 or Qp.stride(0) % 8 or Qp.data_ptr() % 16:
+            raise ValueError('attention_recommend: a bf16 Qp must be a 2-D table with unit column stride, 16-byte aligned rows')
+        ld_q = Qp.stride(0) if Qp.shape[0] > 1 else max(Qp.stride(0), (H1P + 7) // 8 * 8)
+        entry, name = lib.b200rec_attention_recommend_bf16, 'attention_recommend_bf16'
+    else:
+        raise ValueError(f'attention_recommend: Qp must be float32 (K8) or bfloat16 (K8b), not {Qp.dtype}')
     list_ptr, list_item, list_val, users = list_ptr.contiguous(), list_item.contiguous(), list_val.contiguous(), users.contiguous()
     if a2 is not None:
         a2 = a2.detach().contiguous().float()
@@ -1079,10 +1091,9 @@ def attention_recommend_raw(Pc, Pr, Ai, Qp, *, mode, a2, a20, list_ptr, list_ite
     elif out.shape != (nU * nI, H1P) or out.dtype != torch.float32 or out.stride(1) != 1:
         raise ValueError('attention_recommend: bad `out`')
     ldo = out.stride(0) if out.shape[0] > 1 else H1P
-    with _on(Pc.device), _timed('attention_recommend', (nU, nI, H, H1P)):
-        L.check(L.lib().b200rec_attention_recommend(_ptr(Pc), ld_pc, _ptr(Pr), ld_pr, H, int(mode), _ptr(a2), _ptr(a20), _ptr(Ai), ld_ai, _ptr(Qp), ld_q,
-                                                    H1P, nI, _ptr(list_ptr), _ptr(list_item), _ptr(list_val), _ptr(users), nU, _ptr(out), ldo,
-                                                    _stream()), 'attention_recommend')
+    with _on(Pc.device), _timed(name, (nU, nI, H, H1P)):
+        L.check(entry(_ptr(Pc), ld_pc, _ptr(Pr), ld_pr, H, int(mode), _ptr(a2), _ptr(a20), _ptr(Ai), ld_ai, _ptr(Qp), ld_q, H1P, nI, _ptr(list_ptr),
+                      _ptr(list_item), _ptr(list_val), _ptr(users), nU, _ptr(out), ldo, _stream()), name)
     return out
 
 

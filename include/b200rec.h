@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define B200REC_VERSION 205
+#define B200REC_VERSION 206
 
 typedef void* b200rec_stream_t; /* cudaStream_t */
 
@@ -243,6 +243,14 @@ int b200rec_attention_recommend(const float* Pc, int64_t ld_pc, const float* Pr,
                                 const float* Ai, int64_t ld_ai, const float* Qp, int64_t ld_q, int H1P, int64_t n_items, const int64_t* list_ptr,
                                 const int32_t* list_item, const float* list_val, const int64_t* users, int64_t n_users, float* h1, int64_t ld_h1,
                                 b200rec_stream_t stream);
+/* K8b: the same op for AttentionNCF.recommend(precision='bf16') — src/webapp/backend.py:78-121 / attention_ncf.py:136-224 as above, with the
+ * pooling on bf16 tensor cores.  Qp is a bf16 table (n_items, H1P), ld_q in elements (% 8 == 0), rows 16-byte aligned; the pooling weights
+ * α·val are rounded to bf16, accumulation is fp32.  The scores and α are computed exactly as in b200rec_attention_recommend (bit-identical).
+ * Every other operand, the output and the error codes are those of b200rec_attention_recommend. */
+int b200rec_attention_recommend_bf16(const float* Pc, int64_t ld_pc, const float* Pr, int64_t ld_pr, int H, int mode, const float* a2,
+                                     const float* a20, const float* Ai, int64_t ld_ai, const uint16_t* Qp, int64_t ld_q, int H1P, int64_t n_items,
+                                     const int64_t* list_ptr, const int32_t* list_item, const float* list_val, const int64_t* users,
+                                     int64_t n_users, float* h1, int64_t ld_h1, b200rec_stream_t stream);
 /* ---- K9  AttentionNCF explanations of many users' recommendations (csrc/attention_explain.cu) -----------------------------------------
  * Replaces the explanation step of src/webapp/backend.py:102-110 for k recommended items of each of many users: the entries i of user u's list
  * with α_bi > explain_factor · (1 / max(R_u, 1)) + explain_constant (computed in double, compared in fp32), R_u = length of u's list, zero-centred

@@ -1,11 +1,12 @@
 """AttentionNCF.recommend (K8) and AttentionNCF.explain (K9) at config 2 and on a catalogue larger than L2, against the per-user
-`recommend_for_user` loop (which ranks and explains) in the same run.
+`recommend_for_user` loop (which ranks and explains) in the same run; and recommend(precision='bf16') (K8b) against fp32 on both workloads.
 
     python tools/attention_recommend_bench.py [--out FILE.json] [--large-users N] [--large-items N]
 
 Config 2 = the inputs of bench.py's build_attention (synth.interactions_small(610, 9724, 100_836, seed=42), item profiles seed 43, weights
 seed 1, item_emb = user_emb = att_dense = 128, MLP [256, 128]): all 610 users x the catalogue, top-10.  Call times are host clocks around
-calls bracketed by a device synchronise; per-op times come from CUDA events of one extra call (ops.OpTimer).  The operation-count model
+calls bracketed by a device synchronise; per-op times come from CUDA events of one extra call (ops.OpTimer).  The two precisions
+are timed alternating, median of --reps calls each.  The operation-count model
 is computed from the shapes and printed as an estimate, never as a measurement."""
 import argparse
 import json
@@ -67,6 +68,42 @@ def op_model(list_lens, nI, H, H1, clock_ghz, sms=148):
                     'lane-instructions ~ 3·H per interaction for the scores (FADD, FMNMX, FFMA) + H1 for the pooling (FFMA)',
             'interactions': inter, 'lane_instructions': lane, 'clock_ghz': clock_ghz,
             'fp32_bound_ms': lane / (sms * 128 * clock_ghz * 1e9) * 1e3}
+
+
+def per_op_ms(fn):
+    """CUDA-event time per op name of one call"""
+    timer = ops.OpTimer()
+    prev = ops.set_timer(timer)
+    fn()
+    torch.cuda.synchronize()
+    ops.set_timer(prev)
+    out = {}
+    for (name, _), v in timer.summary().items():
+        out[name] = out.get(name, 0.0) + sum(v)
+    return out
+
+
+def precisions(model, lists, reps):
+    """fp32 against bf16 on the same users, top-10: call times alternating, per-op times, max-norm error of the bf16 scores against the fp32
+    ones (per user, over the unseen items) and how many users get the same top-10 set"""
+    for prec in ('fp32', 'bf16', 'fp32', 'bf16'):
+        model.recommend(*lists, k=10, precision=prec)
+    t = {'fp32': [], 'bf16': []}
+    for _ in range(reps):
+        for prec in ('fp32', 'bf16'):
+            t[prec].append(timed(lambda: model.recommend(*lists, k=10, precision=prec))[0])
+    _, i32, s32 = model.recommend(*lists, k=10, return_scores=True)
+    _, i16, s16 = model.recommend(*lists, k=10, return_scores=True, precision='bf16')
+    seen = torch.isnan(s32)
+    a, b = s16.masked_fill(seen, 0.0).double(), s32.masked_fill(seen, 0.0).double()
+    rel = ((a - b).abs().amax(1) / b.abs().amax(1).clamp_min(1e-30)).max().item()
+    same = int((i16.sort(1).values == i32.sort(1).values).all(1).sum().item())
+    med = {k: statistics.median(v) for k, v in t.items()}
+    return {'recommend_ms_median': med, 'recommend_ms_all': t, 'bf16_speedup': med['fp32'] / med['bf16'],
+            'per_op_ms_one_warm_call (CUDA events)': {prec: per_op_ms(lambda: model.recommend(*lists, k=10, precision=prec))
+                                                      for prec in ('fp32', 'bf16')},
+            'bf16_vs_fp32_maxnorm_rel_worst_user': rel, 'bf16_nan_pattern_equal': bool(torch.equal(torch.isnan(s16), seen)),
+            'top10_sets_identical_users': same, 'users': int(i32.shape[0])}
 
 
 def main():
@@ -168,6 +205,7 @@ def main():
                          'longest_list_chunks_per_pass': int((lens.max() + 31) // 32)},
         },
     }
+    res['config2']['precision'] = precisions(model, lists, a.reps)
     del model, prov, scores
     torch.cuda.empty_cache()
 
@@ -186,7 +224,8 @@ def main():
     res['large_catalogue'] = {'users': nUl, 'items': nIl, 'list_entries': int(lens.sum()), 'tables_bytes': table_bytes,
                               'recommend_ms_median': statistics.median(times), 'recommend_ms_all': times,
                               'pairs_per_s': nUl * nIl / (statistics.median(times) * 1e-3), 'op_model': op_model(lens, nIl, H, H1, clock_ghz),
-                              'explain_top10_ms_median': statistics.median(explain_times), 'explain_top10_ms_all': explain_times}
+                              'explain_top10_ms_median': statistics.median(explain_times), 'explain_top10_ms_all': explain_times,
+                              'precision': precisions(model, lists, a.reps)}
     txt = json.dumps(res, indent=1)
     print(txt)
     if a.out:
