@@ -14,6 +14,7 @@ import ctypes as C
 import torch
 
 from . import _lib as L
+from .derived import Derived
 from .ops import _ptr, _stream, _require_cuda
 
 SPMM_CHUNK = 256
@@ -351,32 +352,19 @@ def stream_plan(index, dinv=None, seg=None) -> StreamPlan:
     """cached StreamPlan of a GraphIndex / local index for its own (or the given) deg^-1/2"""
     dinv = index.dinv if dinv is None else dinv
     seg = default_stream_seg(int(index.col.numel())) if seg is None else seg
-    cache = index.__dict__.setdefault('_stream_plans', {})
-    key = (seg, None if dinv is None else (dinv.data_ptr(), dinv._version), None if index.w is None else (index.w.data_ptr(), index.w._version))
-    plan = cache.get(key)
-    if plan is None:
-        if len(cache) > 4:
-            cache.clear()
-        plan = cache[key] = StreamPlan(index.row_ptr, index.col, index.w, dinv, seg)
-    return plan
+    plans = index.__dict__.setdefault('_stream_plans', Derived(5))
+    return plans.get((dinv, index.w), lambda: StreamPlan(index.row_ptr, index.col, index.w, dinv, seg), seg)
 
 
 def get_index(graph) -> GraphIndex:
-    """GraphIndex of a graph object (ours or the reference's PyG `Data`), built once and cached on it."""
-    idx = getattr(graph, '_b200rec_index', None)
+    """GraphIndex of a graph object (ours or the reference's PyG `Data`), built once and cached on it.  Replacing or editing an edge
+    list or an attr tensor, or changing the node counts, rebuilds it (and drops a partition of the old graph)."""
+    store = graph.__dict__.setdefault('_b200rec_index', Derived(1))
     u2i, i2u = graph.user2item_edge_index, graph.item2user_edge_index
     au, ai = getattr(graph, 'user2item_edge_attr', None), getattr(graph, 'item2user_edge_attr', None)
     n_nodes = int(graph.item_features.shape[0] + graph.user_features.shape[0])
-    # identity of everything the index was derived from (addresses, in-place versions, sizes): replacing or editing an edge list or
-    # an attr tensor, or changing the node counts, rebuilds it
-    key = tuple((t.data_ptr(), t._version, tuple(t.shape), str(t.device)) if torch.is_tensor(t) else None for t in (u2i, i2u, au, ai)) + (n_nodes,)
-    if idx is not None and getattr(idx, '_key', None) == key:
-        return idx
-    idx = GraphIndex(u2i, i2u, au, ai, n_nodes)
-    idx._key = key
-    try:
-        object.__setattr__(graph, '_b200rec_partition', None)
-        object.__setattr__(graph, '_b200rec_index', idx)
-    except Exception:
-        pass
-    return idx
+
+    def build():
+        graph.__dict__['_b200rec_partition'] = None
+        return GraphIndex(u2i, i2u, au, ai, n_nodes)
+    return store.get((u2i, i2u, au, ai), build, n_nodes)

@@ -1,13 +1,12 @@
 """AttentionNCF on the B200 path (reference: neural_collaborative_filtering/models/attention_ncf.py:64-224)."""
 from __future__ import annotations
 
-import weakref
-
 import torch
 from torch import nn
 
 from ... import _lib as L
 from ... import ops
+from ...derived import Derived
 from ..util import build_MLP_layers, mlp_parameters, run_mlp
 from .base import NCF, _named_like
 
@@ -59,6 +58,11 @@ class AttentionNCF(NCF):
             else:
                 self.AttentionNet = nn.Sequential(nn.Linear(2 * item_emb, 1))
         self.MLP = build_MLP_layers(item_emb + user_emb, mlp_dense_layers, dropout_rate=dropout_rate)
+        self._proj_cache = Derived(1)        # _stacked_projection
+        self._comp_cache = Derived(1)        # _composite_projection
+        self._att_cache = Derived(1)         # _attention_halves
+        self._rec_cache = Derived(1)         # _recommend_tables
+        self._rec_bf16 = Derived(1)          # bf16 copy of the cached Q' table (recommend(precision='bf16'))
 
     def important_hypeparams(self) -> str:
         return '_cosine' if self.use_cos_sim_instead else f'_attNet{self.att_dense}'
@@ -98,15 +102,11 @@ class AttentionNCF(NCF):
         """[W_I ; W_U] and [b_I ; 0] for the single sweep over rated_items.  Under no_grad the stacked copies are cached
         until a parameter changes (its `_version` moves with every optimizer step / load_state_dict)."""
         item, user = self.ItemEmbeddings[0], self.UserEmbeddings[0]
-        grad = torch.is_grad_enabled() and any(p.requires_grad for p in (item.weight, user.weight))
-        key = None if grad else tuple((p.data_ptr(), p._version) for p in (item.weight, item.bias, user.weight, user.bias))
-        cached = getattr(self, '_proj_cache', None)
-        if key is not None and cached is not None and cached[0] == key:
-            return cached[1]
-        WU, bU = _pad_rows(user.weight, user.bias)
-        out = (torch.cat((item.weight, WU), 0), torch.cat((item.bias, torch.zeros_like(bU)), 0), bU)
-        self._proj_cache = (key, tuple(t.detach() for t in out)) if key is not None else None
-        return out
+
+        def stack():
+            WU, bU = _pad_rows(user.weight, user.bias)
+            return torch.cat((item.weight, WU), 0), torch.cat((item.bias, torch.zeros_like(bU)), 0), bU
+        return self._proj_cache.get((item.weight, item.bias, user.weight, user.bias), stack)
 
     def _composite_projection(self):
         """Inference-only algebra: AttentionNet.0's halves are folded into the profile projections, so that the attention
@@ -123,21 +123,18 @@ class AttentionNCF(NCF):
             return None
         item, user, first = self.ItemEmbeddings[0], self.UserEmbeddings[0], self.AttentionNet[0]
         params = (item.weight, item.bias, user.weight, user.bias, first.weight, first.bias, self.AttentionNet[3].weight)
-        key = tuple((p.data_ptr(), p._version) for p in params)
-        cached = getattr(self, '_comp_cache', None)
-        if cached is not None and cached[0] == key:
-            return cached[1]
-        with torch.no_grad():
-            A1c, A1r, a1, a2, a20 = halves
-            WI, bI = item.weight.double(), item.bias.double()
-            WU, bU = _pad_rows(user.weight.detach(), user.bias.detach())
-            Wr = torch.cat(((A1r.double() @ WI).float(), WU), 0).contiguous()
-            br = torch.cat(((A1r.double() @ bI).float(), torch.zeros_like(bU)), 0).contiguous()
-            Wc = torch.cat((item.weight.detach(), (A1c.double() @ WI).float()), 0).contiguous()
-            bc = torch.cat((item.bias.detach(), (A1c.double() @ bI + a1.double()).float()), 0).contiguous()
-        out = (Wr, br, Wc, bc, bU, a2, a20, A1r.shape[0])
-        self._comp_cache = (key, out)
-        return out
+
+        def compose():
+            with torch.no_grad():
+                A1c, A1r, a1, a2, a20 = halves
+                WI, bI = item.weight.double(), item.bias.double()
+                WU, bU = _pad_rows(user.weight.detach(), user.bias.detach())
+                Wr = torch.cat(((A1r.double() @ WI).float(), WU), 0).contiguous()
+                br = torch.cat(((A1r.double() @ bI).float(), torch.zeros_like(bU)), 0).contiguous()
+                Wc = torch.cat((item.weight.detach(), (A1c.double() @ WI).float()), 0).contiguous()
+                bc = torch.cat((item.bias.detach(), (A1c.double() @ bI + a1.double()).float()), 0).contiguous()
+            return Wr, br, Wc, bc, bU, a2, a20, A1r.shape[0]
+        return self._comp_cache.get(params, compose)
 
     def _attention_halves(self):
         """(A1c, A1r, a1, a2, head bias) of AttentionNet as STABLE view objects (so their MMA-ready packed copies stay cached)
@@ -145,14 +142,9 @@ class AttentionNCF(NCF):
         if self.use_cos_sim_instead or len(self.AttentionNet) == 1 or self.AttentionNet[0].weight.shape[0] % 4:
             return None
         first, head = self.AttentionNet[0], self.AttentionNet[3]
-        key = (first.weight.data_ptr(), first.weight._version, head.weight.data_ptr(), head.weight._version)
-        cached = getattr(self, '_att_cache', None)
-        if cached is None or cached[0] != key:
-            E = first.weight.shape[1] // 2
-            w = first.weight.detach()
-            cached = (key, (w[:, :E], w[:, E:], first.bias.detach(), head.weight.detach().view(-1), head.bias.detach()))
-            self._att_cache = cached
-        return cached[1]
+        w, E = first.weight, first.weight.shape[1] // 2
+        return self._att_cache.get((w, first.bias, head.weight, head.bias), lambda: (
+            w.detach()[:, :E], w.detach()[:, E:], first.bias.detach(), head.weight.detach().view(-1), head.bias.detach()))
 
     def forward(self, candidate_items, rated_items, user_matrix, return_attention_weights=False):
         item, user = self.ItemEmbeddings[0], self.UserEmbeddings[0]
@@ -301,14 +293,11 @@ class AttentionNCF(NCF):
             H = (self.AttentionNet[0].weight.shape[0] + 3) // 4 * 4 if len(self.AttentionNet) > 1 else 4
         if H > 256:
             raise NotImplementedError(f'recommend(): attention width {H} > 256 is not supported')
-        params = tuple(self.parameters())
-        key = (tuple(item_profiles.shape), item_profiles._version, item_profiles.device) + tuple((p.data_ptr(), p._version) for p in params)
-        cached = getattr(self, '_rec_cache', None)
-        if cached is not None and cached[0] == key and cached[1]() is item_profiles:
-            return cached[2]
         item, user = self.ItemEmbeddings[0], self.UserEmbeddings[0]
-        R = item_profiles if item_profiles.dtype == torch.float32 else item_profiles.float()
-        with torch.no_grad():
+
+        def build():
+            self._rec_bf16.clear()                                                         # the bf16 copy of Q' goes with the old tables
+            R = item_profiles if item_profiles.dtype == torch.float32 else item_profiles.float()
             WI, bI, WU, bU = (t.detach().double() for t in (item.weight, item.bias, user.weight, user.bias))
             W1, b1 = weights[0].detach().double(), biases[0].detach().double()
             W1e, W1u = W1[:, :E], W1[:, E:]
@@ -335,9 +324,9 @@ class AttentionNCF(NCF):
                 Ec, Ai, Qp = T[:, :E], T[:, Ep:Ep + H1P], T[:, Ep + H1P:]
                 Pc, Pr, mode, a2, a20 = self._score_tables(Ec, Ec)
                 Pc, Pr = Pc.detach().contiguous(), Pr.detach().contiguous()
-        out = (Pc, Pr, mode, a2, a20, Ai, Qp, H1)
-        self._rec_cache = (key, weakref.ref(item_profiles), out)
-        return out
+            return Pc, Pr, mode, a2, a20, Ai, Qp, H1
+        with torch.no_grad():                          # constants of the catalogue and the weights: cached in any grad mode, like the forward's
+            return self._rec_cache.get((item_profiles, *self.parameters()), build)
 
     def recommend(self, item_profiles, list_ptr, list_item, list_val, k=10, users=None, ignore_seen=True, return_scores=False, chunk_users=None,
                   precision='fp32'):
@@ -378,10 +367,9 @@ class AttentionNCF(NCF):
             Pc, Pr, mode, a2, a20, Ai, Qp, H1 = self._recommend_tables(item_profiles)
             hidden = None
             if precision == 'bf16':
-                if len(self._rec_cache) == 3:                          # the bf16 copy of Q' lives and dies with the cached tables
-                    self._rec_cache += (Qp.to(torch.bfloat16, memory_format=torch.contiguous_format),)
+                Qp = self._rec_bf16.get((Qp,), lambda: Qp.to(torch.bfloat16, memory_format=torch.contiguous_format))
                 # K = H1 <= 256 is below ops.TC_MIN_K, where the default routing picks the FFMA GEMM: force the bf16 tensor cores
-                Qp, hidden = self._rec_cache[3], 'bf16!'
+                hidden = 'bf16!'
             H1P = Ai.shape[1]
             if chunk_users is None:
                 chunk_users = max(1, RECOMMEND_SLAB_BYTES // max(1, nI * H1P * 4))

@@ -4,6 +4,8 @@ from __future__ import annotations
 import torch
 from torch import nn
 
+from ...derived import Derived
+
 
 def _named_like(dataset_class, *names) -> bool:
     """True if the class (ours or the reference's own) derives from a dataset class with one of these names, so the
@@ -33,16 +35,15 @@ class NCF(nn.Module):
         return ''
 
     # ---- derived copies of the weights (packed MMA tiles, composite / transposed matrices, cached embeddings) -----------------------
-    # They are keyed on (address, tensor `_version`).  Loading a state dict, moving / casting the module, or editing parameters through
+    # They are kept in `derived.Derived` stores (the model's own are attributes of it) and reused only while every source is the same live
+    # tensor at the same address with the same `_version`.  Loading a state dict, moving / casting the module, or editing parameters through
     # `.data` (which does NOT bump `_version`) must drop them: the first two are hooked here, the third is what `invalidate_caches()` is for.
-    _DERIVED = ('_proj_cache', '_comp_cache', '_att_cache', '_cache', '_peer_layer0', '_emb_cache', '_rec_cache')
-
     def invalidate_caches(self):
         from ... import ops
         ops.invalidate_caches()
-        for name in self._DERIVED:
-            if name in self.__dict__:
-                object.__setattr__(self, name, None)
+        for v in self.__dict__.values():
+            if isinstance(v, Derived):
+                v.clear()
 
     def load_state_dict(self, *args, **kwargs):
         out = super().load_state_dict(*args, **kwargs)

@@ -5,6 +5,7 @@ import torch
 from torch import nn
 
 from ... import ops
+from ...derived import Derived
 from ..util import build_MLP_layers, mlp_parameters, run_mlp
 from .base import NCF, _named_like
 
@@ -22,6 +23,7 @@ class BasicNCF(NCF):
         self.item_embeddings = nn.Sequential(nn.Linear(item_dim, item_emb))
         self.user_embeddings = nn.Sequential(nn.Linear(user_dim, user_emb))
         self.MLP = build_MLP_layers(item_emb + user_emb, mlp_dense_layers, dropout_rate=dropout_rate)
+        self._emb_cache = Derived(1)         # (user table, item table) embeddings of forward_resident
 
     cache_eval_embeddings = False        # forward_resident: project every row of the resident tables once per weight version (inference)
 
@@ -38,14 +40,10 @@ class BasicNCF(NCF):
         if not self.cache_eval_embeddings:
             return self.forward(X_user.table.index_select(0, pu), X_item.table.index_select(0, pi))
         ue, ie = self.user_embeddings[0], self.item_embeddings[0]
-        key = (X_user.table.data_ptr(), X_user.table._version, X_item.table.data_ptr(), X_item.table._version,
-               tuple((p.data_ptr(), p._version) for p in (ue.weight, ue.bias, ie.weight, ie.bias)))
-        cached = getattr(self, '_emb_cache', None)
-        if cached is None or cached[0] != key:
-            with torch.no_grad():
-                cached = (key, ops.linear_raw(X_user.table, ue.weight, ue.bias), ops.linear_raw(X_item.table, ie.weight, ie.bias))
-            self._emb_cache = cached
-        return run_mlp(self.MLP, cached[1], cached[2], idx0=pu, idx1=pi, training=False)
+        user_emb, item_emb = self._emb_cache.get(
+            (X_user.table, X_item.table, ue.weight, ue.bias, ie.weight, ie.bias),
+            lambda: (ops.linear_raw(X_user.table, ue.weight, ue.bias), ops.linear_raw(X_item.table, ie.weight, ie.bias)))
+        return run_mlp(self.MLP, user_emb, item_emb, idx0=pu, idx1=pi, training=False)
 
     def forward(self, X_user, X_item):
         if hasattr(X_user, 'table') and hasattr(X_item, 'table'):

@@ -8,6 +8,7 @@ import torch
 from torch import nn
 
 from ... import ops
+from ...derived import Derived
 from ...graph import get_index
 from ..util import build_MLP_layers, mlp_parameters, run_mlp
 from .base import GNN_NCF, _named_like
@@ -99,7 +100,8 @@ class GraphNCF(GNN_NCF):
                            convType=convType)
         self.concat, self.message_dropout, self.node_dropout, self.convType = concat, message_dropout, node_dropout, convType
         self.cache_eval_embeddings = cache_eval_embeddings
-        self._cache = None
+        self._cache = Derived(1)                  # propagated embeddings (cache_eval_embeddings)
+        self._peer_layer0 = Derived(1)            # layer-0 composite weights of the peer-partitioned forward (peer.py)
         self.item_embeddings = nn.Sequential(nn.Linear(item_dim, node_emb))
         self.user_embeddings = nn.Sequential(nn.Linear(user_dim, node_emb))
         if convType == 'LightGCN':
@@ -255,13 +257,11 @@ class GraphNCF(GNN_NCF):
             removed = self._training_mask(index, userIds, itemIds, mask_targets)
             if removed is not None:
                 skip, dinv = index.masked(removed)
-        use_cache = self.cache_eval_embeddings and not self.training and not torch.is_grad_enabled()
-        key = (id(index), self.message_dtype, tuple(p._version for p in self.parameters())) if use_cache else None
-        if use_cache and self._cache is not None and self._cache[0] == key:
-            comb = self._cache[1]
+        if self.cache_eval_embeddings and not self.training and not torch.is_grad_enabled():
+            comb = self._cache.get((index, *self.parameters()), lambda: self._encode(graph, index, skip, dinv, False), self.message_dtype)
         else:
+            self._cache.clear()
             comb = self._encode(graph, index, skip, dinv, self.training)
-            self._cache = (key, comb) if use_cache else None
         if self.MLP is None:
             return ops.rowdot(comb, comb, userIds, itemIds)                               # :365
         return run_mlp(self.MLP, comb, comb, idx0=itemIds, idx1=userIds, training=self.training)   # item first (:361)

@@ -12,11 +12,11 @@ from __future__ import annotations
 
 import ctypes as C
 import os
-import weakref
 
 import torch
 
 from . import _lib as L
+from .derived import Derived
 
 
 class OpTimer:
@@ -146,35 +146,32 @@ SHORTK_MIN_ROWS = 4096  # below this a handful of 64x64 FFMA tiles is as fast as
 TC_MIN_K = 512          # short-K GEMMs (the d x d GraphNCF transforms) are epilogue/latency-bound: FFMA is as fast there
 
 
-_pack_cache = {}              # (data_ptr, version, shape, ld, mode) -> packed buffer; a handful of weight matrices at most
+_pack_cache = Derived(64)     # MMA-ready packed weights: a handful of weight matrices at most
+_wt_cache = Derived(64)       # transposed K1s tables
+_ap_cache = Derived(32)       # all-pairs second-layer packs
 
 
 def _packed_weight(w, ldw, mode):
     """MMA-ready copy of a weight matrix (b200rec_pack_weights_tc), cached until the tensor changes (`_version`)."""
-    key = (w.data_ptr(), w._version, tuple(w.shape), ldw, mode, w.device.index)
-    hit = _pack_cache.get(key)
-    if hit is not None and hit[0]() is w:          # same live tensor object, unchanged since it was packed
-        return hit[1]
-    lib = L.lib()
-    N, K = w.shape
-    nbytes = lib.b200rec_packed_weight_bytes(N, K, mode)
-    buf = torch.empty(nbytes, dtype=torch.uint8, device=w.device)
-    with _on(w.device):
-        L.check(lib.b200rec_pack_weights_tc(_ptr(w), N, K, ldw, mode, _ptr(buf), nbytes, _stream()), 'pack_weights_tc')
-    if len(_pack_cache) > 64:
-        _pack_cache.clear()
-    if not (torch.is_grad_enabled() and w.requires_grad):
-        _pack_cache[key] = (weakref.ref(w), buf)
-    return buf
+    def pack():
+        lib = L.lib()
+        N, K = w.shape
+        nbytes = lib.b200rec_packed_weight_bytes(N, K, mode)
+        buf = torch.empty(nbytes, dtype=torch.uint8, device=w.device)
+        with _on(w.device):
+            L.check(lib.b200rec_pack_weights_tc(_ptr(w), N, K, ldw, mode, _ptr(buf), nbytes, _stream()), 'pack_weights_tc')
+        return buf
+    return _pack_cache.get((w,), pack, ldw, mode)
 
 
 def invalidate_caches():
-    """Drops every derived copy of a weight kept by this module (MMA-ready packed weights, transposed tables, all-pairs packs).  The caches are
-    keyed on (address, `_version`): an in-place edit THROUGH `.data` (`p.data.copy_()`, some EMA / weight-averaging utilities) does not bump
-    `_version`, so such code must call this (the model classes do it from `load_state_dict` / `_apply` / `invalidate_caches()`)."""
+    """Drops every derived copy of a weight kept by this module (MMA-ready packed weights, transposed tables, all-pairs packs).  An entry
+    is reused only while its source is the same live tensor at the same address with the same `_version` (`derived.Derived`): an in-place
+    edit THROUGH `.data` (`p.data.copy_()`, some EMA / weight-averaging utilities) does not bump `_version`, so such code must call this
+    (the model classes do it from `load_state_dict` / `_apply` / `invalidate_caches()`)."""
     _pack_cache.clear()
-    globals().get('_wt_cache', {}).clear()
-    globals().get('_ap_cache', {}).clear()
+    _wt_cache.clear()
+    _ap_cache.clear()
 
 
 def _tc_mode(engine):
@@ -359,21 +356,9 @@ def linear_pair(xa, wa, ba, xb, wb, bb):
 # ------------------------------------------------------------------------------------------------------------------
 # K1s sparse projection (one-hot / multi-hot profile rows)
 # ------------------------------------------------------------------------------------------------------------------
-_wt_cache = {}
-
-
 def _transposed_weight(weight, c0, c1, dtype=torch.float32):
     """W[:, c0:c1]^T as a contiguous (c1 - c0, N) table (the "embedding table" K1s gathers from), cached per weight version."""
-    key = (weight.data_ptr(), weight._version, tuple(weight.shape), c0, c1, dtype, weight.device.index)
-    hit = _wt_cache.get(key)
-    if hit is not None and hit[0]() is weight:
-        return hit[1]
-    wt = weight.detach()[:, c0:c1].t().to(dtype).contiguous()
-    if len(_wt_cache) > 64:
-        _wt_cache.clear()
-    if not (torch.is_grad_enabled() and weight.requires_grad):
-        _wt_cache[key] = (weakref.ref(weight), wt)
-    return wt
+    return _wt_cache.get((weight,), lambda: weight.detach()[:, c0:c1].t().to(dtype).contiguous(), c0, c1, dtype)
 
 
 def linear_sparse_raw(weight, bias, *, csr=None, ids=None, cols=None, out=None, accumulate=False, table_dtype=torch.float32):
@@ -1213,9 +1198,6 @@ def sample_negatives_raw(sample_rows, neg_ptr, neg_item, neg_rating, *, w, seed,
 # ------------------------------------------------------------------------------------------------------------------
 # K5 all-pairs scoring + top-k (tcgen05)
 # ------------------------------------------------------------------------------------------------------------------
-_ap_cache = {}
-
-
 class AllPairsWeights:
     """second MLP layer in MMA-ready form (device) + the epilogue constants b2 | w3 | b3 as a HOST array (they travel in
     the kernel's parameter block)"""
@@ -1228,12 +1210,10 @@ def allpairs_pack(W2, b2, w3, b3, H1p, mode):
     """`AllPairsWeights` for `allpairs_topk_raw`; cached until a tensor changes (one device->host read of 2*H2+1 floats
     per weight version)."""
     _require_cuda(W2, b2, w3, b3)
-    # keyed on the tensor OBJECTS (weak references), not on addresses: a freed temporary's address is reused by the allocator
-    ts = tuple(t for t in (W2, b2, w3, b3) if t is not None)
-    key = tuple((id(t), t._version) for t in ts) + (H1p, mode)
-    hit = _ap_cache.get(key)
-    if hit is not None and all(r() is t for r, t in zip(hit[0], ts)):
-        return hit[1]
+    return _ap_cache.get((W2, b2, w3, b3), lambda: _allpairs_pack(W2, b2, w3, b3, H1p, mode), H1p, mode)
+
+
+def _allpairs_pack(W2, b2, w3, b3, H1p, mode):
     lib = L.lib()
     H2, H1 = W2.shape
     w2p = W2.detach().float()
@@ -1247,12 +1227,7 @@ def allpairs_pack(W2, b2, w3, b3, H1p, mode):
     buf = torch.empty(nbytes, dtype=torch.uint8, device=W2.device)
     with _on(W2.device):
         L.check(lib.b200rec_allpairs_pack(_ptr(w2p), H1p, H2, H1p, mode, _ptr(buf), nbytes, _stream()), 'allpairs_pack')
-    buf = AllPairsWeights(buf, epi, H2)
-    if len(_ap_cache) > 32:
-        _ap_cache.clear()
-    if not torch.is_grad_enabled() or not any(t.requires_grad for t in ts):
-        _ap_cache[key] = (tuple(weakref.ref(t) for t in ts), buf)
-    return buf
+    return AllPairsWeights(buf, epi, H2)
 
 
 def allpairs_topk_raw(A, B, packed, mode, k, *, return_scores=False, seen=None, n_splits=0):

@@ -240,7 +240,7 @@ def test_config2_all_users():
 
 
 # ---- 5. determinism -------------------------------------------------------------------------------------------------------------------
-def test_deterministic_and_chunking():
+def test_deterministic_and_chunking_on_the_cached_bf16_copy():
     from deeprecommendation_b200 import ops
     rng = np.random.default_rng(4)
     nI, F = 4200, 32
@@ -253,9 +253,10 @@ def test_deterministic_and_chunking():
     m.invalidate_caches()
     _equal(a, m.recommend(prof, *lists, k=10, return_scores=True, precision='bf16'))
     # K8b's h1 rows of a user do not depend on which users share the launch: bit for bit
-    Pc, Pr, mode, a2, a20, Ai = m._recommend_tables(prof)[:6]
+    Pc, Pr, mode, a2, a20, Ai, Qp = m._recommend_tables(prof)[:7]
     kw = dict(mode=mode, a2=a2, a20=a20, list_ptr=lists[0], list_item=lists[1], list_val=lists[2])
-    Qb = m._rec_cache[3]
+    (Qb,) = m._rec_bf16.values()                                         # the cached bf16 copy of the cached Q'
+    assert Qb.is_contiguous() and torch.equal(Qb, Qp.to(torch.bfloat16))
     h_all = ops.attention_recommend_raw(Pc, Pr, Ai, Qb, users=torch.arange(nU, device=DEV), **kw)
     h_one = torch.cat([ops.attention_recommend_raw(Pc, Pr, Ai, Qb, users=torch.tensor([u], device=DEV), **kw) for u in range(nU)])
     assert torch.equal(h_all, h_one)
@@ -280,16 +281,16 @@ def _fresh(m, prof, lists, precision):
     return f.recommend(prof, *lists, k=10, return_scores=True, precision=precision)
 
 
-def test_caches_follow_changes():
+def test_caches_and_the_bf16_store_follow_changes():
     rng = np.random.default_rng(8)
     nI, F = 200, 32
     m, _ = _model(F)
     prof = _profiles(rng, nI, F).to(DEV)
     lists = _dev(*_lists(rng, 8, nI, 80))
     fp32 = m.recommend(prof, *lists, k=10, return_scores=True)
-    assert len(m._rec_cache) == 3                                       # an fp32 call makes no bf16 copy
+    assert len(m._rec_cache) == 1 and len(m._rec_bf16) == 0             # an fp32 call makes no bf16 copy
     base = m.recommend(prof, *lists, k=10, return_scores=True, precision='bf16')
-    assert len(m._rec_cache) == 4
+    assert len(m._rec_bf16) == 1
     _equal(fp32, m.recommend(prof, *lists, k=10, return_scores=True))   # fp32 after bf16: untouched
     _equal(fp32, _fresh(m, prof, lists, 'fp32'))
     # an optimizer step (in place, bumps _version)
@@ -303,7 +304,7 @@ def test_caches_follow_changes():
     # load_state_dict
     _, sd2 = _model(F, seed=9)
     m.load_state_dict(sd2)
-    assert m._rec_cache is None
+    assert len(m._rec_cache) == 0 and len(m._rec_bf16) == 0
     _equal(m.recommend(prof, *lists, k=10, return_scores=True, precision='bf16'), _fresh(m, prof, lists, 'bf16'))
     _equal(m.recommend(prof, *lists, k=10, return_scores=True), _fresh(m, prof, lists, 'fp32'))
 

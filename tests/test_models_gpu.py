@@ -66,7 +66,7 @@ def test_basic_cfg1_batches_vs_oracle():
         assert maxnorm_rel(out, ref) < TOL
 
 
-def test_basic_resident_profiles_through_the_dataset_contract():
+def test_basic_resident_profiles_through_the_dataset_contract_and_embedding_store():
     """ResidentProfilesProvider (both profile tables in HBM, batches = row numbers) through FixedPointwiseDataset / FixedRankingDataset:
     identical bits to the dense contract; with cached per-row embeddings within 1e-5 of the oracle; training falls back to dense rows."""
     import pandas as pd
@@ -100,12 +100,12 @@ def test_basic_resident_profiles_through_the_dataset_contract():
     with torch.no_grad():
         cached, _ = FixedPointwiseDataset.do_forward(m, batch, DEV)
         assert maxnorm_rel(cached, ref) < TOL
-        assert m._emb_cache is not None and m._emb_cache[1].shape == (nU, 128) and m._emb_cache[2].shape == (nI, 128)
-        first = m._emb_cache[1]
+        (first,) = m._emb_cache.values()
+        assert first[0].shape == (nU, 128) and first[1].shape == (nI, 128)
         FixedPointwiseDataset.do_forward(m, batch, DEV)
-        assert m._emb_cache[1] is first                                # reused while the weights are unchanged
+        assert m._emb_cache.values()[0] is first                       # reused while the weights are unchanged
         m.load_state_dict(sd)
-        assert m._emb_cache is None                                    # dropped with the weights
+        assert len(m._emb_cache) == 0                                  # dropped with the weights
         # ranking form: (user, positive, negative) rows, two scores per sample
         trip = (res_p.get_user_profile(user_ids[pu]), res_p.get_item_profile(item_ids[pi]), res_p.get_item_profile(item_ids[pj]))
         pos, neg = FixedRankingDataset.do_forward(m, trip, DEV)
@@ -115,6 +115,68 @@ def test_basic_resident_profiles_through_the_dataset_contract():
     out = FixedPointwiseDataset.do_forward(m, batch, DEV)[0]
     out.sum().backward()
     assert torch.isfinite(m.user_embeddings[0].weight.grad).all()
+
+
+def test_basic_cached_embeddings_of_a_new_provider_at_the_old_addresses():
+    """cache_eval_embeddings: a provider dropped and rebuilt with other tables of the same size, which the caching allocator places at the
+    freed addresses (with `_version` 0 again), gets its own embeddings and not the old tables' cached ones"""
+    from deeprecommendation_b200.content_providers import ResidentProfilesProvider
+    kw = dict(item_dim=2094, user_dim=2094, item_emb=128, user_emb=128, mlp_dense_layers=[256, 128], dropout_rate=0.2)
+    m = _models().BasicNCF(**kw).to(DEV).eval()
+    m.load_state_dict(synth.to_torch(synth.basic_ncf_weights(seed=3, **kw)))
+    nI, nU, B = 700, 90, 300
+    rng = np.random.default_rng(1)
+    pu, pi = rng.integers(0, nU, B), rng.integers(0, nI, B)
+
+    def provider(seed):
+        users = ((synth.item_profiles(nU, seed=seed) - 0.3) * 0.1).astype(np.float32)
+        return ResidentProfilesProvider(np.arange(nI), synth.item_profiles(nI, seed=seed + 1), np.arange(nU), users, device=DEV)
+
+    def run(prov, cached):
+        m.cache_eval_embeddings = cached
+        with torch.no_grad():
+            return m(prov.get_user_profile(pu), prov.get_item_profile(pi))
+    prov = provider(11)
+    addresses = (prov.user_table.data_ptr(), prov.item_table.data_ptr())
+    run(prov, True)
+    del prov
+    prov = provider(21)
+    if (prov.user_table.data_ptr(), prov.item_table.data_ptr()) != addresses:
+        pytest.skip('the caching allocator placed the new tables elsewhere')
+    assert prov.user_table._version == prov.item_table._version == 0
+    cached = run(prov, True)
+    assert maxnorm_rel(cached, run(prov, False)) < TOL
+
+
+def test_graph_cached_embeddings_of_a_new_graph():
+    """cache_eval_embeddings=True: graph A freed, then a graph object of other edges with the same sizes built (CPython tends to give it and its
+    index the freed objects' `id`s) gets its own propagated embeddings"""
+    from deeprecommendation_b200.graph import GraphData, IdTable, create_graph, get_index
+    n_users, n_items, n, F = 400, 300, 8000, 32
+    kw = dict(item_dim=F, user_dim=F, num_gnn_layers=2, hetero=True, node_emb=64, mlp_dense_layers=[128], dropout_rate=0.2)
+    m = _models().GraphNCF(**kw, cache_eval_embeddings=True).to(DEV).eval()
+    m.load_state_dict(synth.to_torch(synth.graph_ncf_weights(seed=8, **kw)))
+    rng = np.random.default_rng(3)
+    fi, fu = (torch.from_numpy(rng.standard_normal((k, F)).astype(np.float32)).to(DEV) for k in (n_items, n_users))
+    ut, it = IdTable(torch.arange(n_users, device=DEV)), IdTable(torch.arange(n_items, device=DEV))
+    iid = torch.from_numpy(rng.integers(0, n_items, 128)).to(DEV)
+    uid = torch.from_numpy(rng.integers(0, n_users, 128) + n_items).to(DEV)
+
+    def graph(seed):
+        users, items, ratings = synth.interactions_zipf(n_users, n_items, n, seed=seed)
+        return create_graph(*(torch.from_numpy(a).to(DEV) for a in (users, items, ratings)), fi, fu, ut, it)
+    g = graph(7)
+    with torch.no_grad():
+        m(g, uid, iid, DEV)
+    index_id = id(get_index(g))
+    edges_b = vars(graph(17))
+    del g
+    g = GraphData(**edges_b)
+    with torch.no_grad():
+        cached = m(g, uid, iid, DEV)
+        print(f'the new graph index took the freed one\'s id: {id(get_index(g)) == index_id}')
+        m.cache_eval_embeddings = False
+        assert torch.equal(cached, m(g, uid, iid, DEV))
 
 
 # ---- AttentionNCF ----------------------------------------------------------------------------------------------------------
@@ -300,10 +362,11 @@ def test_graph_ncf_gat_medium_vs_oracle():
 
 
 @pytest.mark.parametrize('conv', ['LightGCN', 'LightGAT'])
-def test_graph_ncf_long_rows_cta_fixup_vs_oracle(conv):
+def test_graph_ncf_long_rows_cta_fixup_on_a_16_edge_chunk_index_vs_oracle(conv):
     """rows cut into MORE than 64 chunks (the CTA-cooperative branch of spmm_fixup_kernel): index built with 16-edge chunks, so
     that the hot items of a small Zipf graph own hundreds of partial slots"""
-    from deeprecommendation_b200.graph import GraphIndex, IdTable, create_graph
+    from deeprecommendation_b200.derived import Derived
+    from deeprecommendation_b200.graph import GraphIndex, IdTable, create_graph, get_index
     n_users, n_items, n, F, d_emb = 2500, 120, 60_000, 24, 64
     users, items, ratings = synth.interactions_zipf(n_users, n_items, n, seed=15)
     rng = np.random.default_rng(8)
@@ -321,7 +384,10 @@ def test_graph_ncf_long_rows_cta_fixup_vs_oracle(conv):
                      IdTable(torch.arange(n_users, device=DEV)), IdTable(torch.arange(n_items, device=DEV)))
     idx = GraphIndex(g.user2item_edge_index, g.item2user_edge_index, g.user2item_edge_attr, g.item2user_edge_attr, n_users + n_items, chunk=16)
     assert int(idx.row_ptr.diff().max()) > 64 * 16                      # some row really takes the long-row branch
-    object.__setattr__(g, '_b200rec_index', idx)
+    store = Derived(1)                                                  # what get_index caches on the graph
+    store.get((g.user2item_edge_index, g.item2user_edge_index, g.user2item_edge_attr, g.item2user_edge_attr), lambda: idx, n_users + n_items)
+    object.__setattr__(g, '_b200rec_index', store)
+    assert get_index(g) is idx
     m = _models().GraphNCF(**kw).to(DEV).eval()
     m.load_state_dict(sd)
     with torch.no_grad():

@@ -141,20 +141,31 @@ def test_sparse_row_containers_round_trip_and_take():
     assert np.array_equal(cp.get_item_profile(np.array([9, 0])).dense_rows().numpy(), rows[[3, 0]])
 
 
-def test_model_hooks_drop_derived_weight_copies():
+def test_model_hooks_empty_the_derived_stores():
     """load_state_dict / .to() / invalidate_caches() drop the derived copies of the weights (packed tiles, composites, cached embeddings) that are
-    keyed on (address, _version) — an edit through `.data` bumps neither (round-1 advisor finding)"""
+    reused while the source tensor keeps its address and _version — an edit through `.data` changes neither"""
     from deeprecommendation_b200 import ops
     from deeprecommendation_b200.neural_collaborative_filtering.models import AttentionNCF, GraphNCF
-    a = AttentionNCF(8, 4, 4, att_dense=4, mlp_dense_layers=[8])
-    a._comp_cache = ('stale', 1)
-    ops._pack_cache['stale'] = 1
+    ops_stores = (ops._pack_cache, ops._wt_cache, ops._ap_cache)
+
+    def fill_ops_stores(w):
+        ops._transposed_weight(w, 0, 4)
+        ops._pack_cache.get((w,), lambda: torch.zeros(1), w.shape[1], 0)
+        ops._ap_cache.get((w, None, None, None), lambda: torch.zeros(1), 64, 0)
+        assert all(len(s) == 1 for s in ops_stores)
+
+    a = AttentionNCF(8, 4, 4, att_dense=4, mlp_dense_layers=[8]).eval()
+    with torch.no_grad():
+        comp = a._composite_projection()
+        assert a._composite_projection() is comp and len(a._comp_cache) == 1 and len(a._att_cache) == 1
+        fill_ops_stores(a.ItemEmbeddings[0].weight)
     a.load_state_dict(a.state_dict())
-    assert a._comp_cache is None and 'stale' not in ops._pack_cache
+    assert len(a._comp_cache) == 0 and len(a._att_cache) == 0 and all(len(s) == 0 for s in ops_stores)
     g = GraphNCF(8, 8, 2, True, node_emb=4, mlp_dense_layers=[8], cache_eval_embeddings=True)
-    g._cache = ('stale', 1)
-    g.double()
-    assert g._cache is None
-    g._cache = ('stale', 1)
-    g.invalidate_caches()
-    assert g._cache is None
+    for drop in (g.double, g.invalidate_caches):
+        with torch.no_grad():
+            g._cache.get(tuple(g.parameters()), lambda: torch.zeros(1), g.message_dtype)
+            fill_ops_stores(g.item_embeddings[0].weight)
+        assert len(g._cache) == 1
+        drop()
+        assert len(g._cache) == 0 and all(len(s) == 0 for s in ops_stores)
