@@ -12,7 +12,7 @@ OK, ERR_CUDA, ERR_BAD_ARG, ERR_UNSUPPORTED, ERR_WORKSPACE = 0, 1, 2, 3, 4
 F32, BF16 = 0, 1
 ATT_NET, ATT_DOT = 0, 1
 TC_TF32X3, TC_BF16, TC_BF16X3 = 0, 1, 2
-ABI_VERSION = 206          # B200REC_VERSION of include/b200rec.h these bindings were written against (checked when the library is loaded)
+ABI_VERSION = 207          # B200REC_VERSION of include/b200rec.h these bindings were written against (checked when the library is loaded)
 AP_BF16, AP_BF16X2 = 0, 1
 MLP_MAX_LAYERS = 8
 PEER_MAX, PEER_CHANNELS, PEER_HANDLE_BYTES = 16, 16, 64
@@ -53,7 +53,8 @@ class SpmmDesc(C.Structure):
                 ('ld_t', c_i64), ('d', c_int), ('dinv', c_vp), ('partials', c_vp), ('x_next', c_vp), ('ld_x', c_i64),
                 ('acc_in', c_vp), ('acc_out', c_vp), ('ld_acc', c_i64), ('acc_scale', c_f), ('multi_row', c_vp),
                 ('multi_first_slot', c_vp), ('multi_n_slots', c_vp), ('n_multi', c_int), ('att_src', c_vp), ('partials_ml', c_vp),
-                ('push_dst', c_vp * PEER_MAX), ('push_parts', c_int), ('push_rows_per_part', c_int), ('push_offset', c_i64), ('push_ld', c_i64)]
+                ('push_dst', c_vp * PEER_MAX), ('push_parts', c_int), ('push_rows_per_part', c_int), ('push_offset', c_i64), ('push_ld', c_i64),
+                ('push_stats_offset', c_i64)]
 
 
 class SpmmStreamDesc(C.Structure):
@@ -143,6 +144,8 @@ SIGNATURES = {
     'b200rec_peer_signal': (c_int, [C.POINTER(c_vp), c_int, c_int, c_int, c_vp, c_vp]),
     'b200rec_peer_wait': (c_int, [c_vp, c_int, c_int, c_vp, c_i64, c_vp, c_vp]),
     'b200rec_peer_reduce': (c_int, [c_vp, c_int, c_i64, c_i64, c_i64, c_int, c_vp, c_i64, c_vp, c_vp, c_i64, c_f, c_vp]),
+    'b200rec_peer_reduce_softmax': (c_int, [c_vp, c_vp, c_int, c_i64, c_i64, c_i64, c_i64, c_int, c_vp, c_i64, c_vp, c_vp, c_i64, c_f, c_vp]),
+    'b200rec_peer_push_floats': (c_int, [c_vp, c_i64, C.POINTER(c_vp), c_int, c_i64, c_vp]),
     'b200rec_peer_push_rows': (c_int, [c_vp, c_i64, c_i64, c_int, C.POINTER(c_vp), c_int, c_i64, c_i64, c_vp]),
     'b200rec_device_timestamp': (c_int, [c_vp, c_vp]),
     'b200rec_peer_gather_rows': (c_int, [c_vp, c_i64, c_i64, c_i64, c_vp, c_i64, c_int, c_f, C.POINTER(c_vp), c_int, c_i64, c_i64, c_vp]),

@@ -8,12 +8,15 @@
 //   * K3's epilogue (csrc/spmm.cu, `push_*` fields) stores the partial item rows of a rank straight into the OWNER's receive
 //     slot over NVLink (reduce-scatter fused into the SpMM);
 //   * peer_reduce_kernel adds the P slots of the owned rows in rank order (deterministic) and folds the running mean in;
+//     for LightGAT, peer_reduce_softmax_kernel merges the slots' unnormalised rows by their softmax state (m, l) instead;
+//   * peer_push_floats_kernel copies the owners' LightGAT source scores (one float per item) into every rank's score table;
 //   * K1c's epilogue (csrc/node_gemm.cu, b200rec_linear_shortk_push) writes the transformed rows into the feature table of
 //     EVERY rank (all-gather fused into the transform GEMM);
 //   * peer_signal_kernel / peer_wait_kernel are the cross-GPU ordering: a release store of an epoch number into every peer's
 //     flag word after the producing kernel, an acquire spin (bounded by a timeout that raises an error flag instead of hanging
 //     the GPU) before the consuming kernel.  Epochs are counted on the device, so a captured CUDA graph can be replayed.
 //   * peer_gather_rows_kernel pushes the batch rows a rank owns into every rank's (2B, d) buffer (replaces an all-reduce).
+#include <math.h>
 #include <stdio.h>
 #include <string.h>
 
@@ -104,6 +107,52 @@ __global__ void __launch_bounds__(256) peer_reduce_kernel(const float* __restric
       *reinterpret_cast<float4*>(acc_out + (long long)r * ld_acc + c) =
           make_float4((a.x + v.x) * acc_scale, (a.y + v.y) * acc_scale, (a.z + v.z) * acc_scale, (a.w + v.w) * acc_scale);
     }
+  }
+}
+
+// LightGAT: the P slots are unnormalised rows relative to their own softmax max; merged with PyG's rule as K3's fix-up merges chunks.
+// A slot with l == 0 (nobody wrote it: the zero-initialised arena, or no edges from that rank) takes part neither in the max nor in the sums.
+__global__ void __launch_bounds__(256) peer_reduce_softmax_kernel(const float* __restrict__ recv, const float* __restrict__ stats, int n_slots,
+                                                                  long long slot_stride, long long ld_recv, long long stats_stride, int rows, int d4,
+                                                                  float* __restrict__ x_next, long long ld_x, const float* __restrict__ acc_in,
+                                                                  float* __restrict__ acc_out, long long ld_acc, float acc_scale) {
+  const long long total = (long long)rows * d4;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const int r = (int)(i / d4), c = (int)(i - (long long)r * d4) * 4;
+    const float* src = recv + (long long)r * ld_recv + c;
+    const float* ml = stats + 2ll * r;
+    float M = -INFINITY;
+    for (int s = 0; s < n_slots; ++s) {
+      const float2 v = __ldg(reinterpret_cast<const float2*>(ml + s * stats_stride));
+      if (v.y > 0.f) M = fmaxf(M, v.x);
+    }
+    float L = 0.f;
+    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+    for (int s = 0; s < n_slots; ++s) {
+      const float2 st = __ldg(reinterpret_cast<const float2*>(ml + s * stats_stride));
+      if (!(st.y > 0.f)) continue;
+      const float e = __expf(st.x - M);
+      L = fmaf(st.y, e, L);
+      const float4 t = __ldcs(reinterpret_cast<const float4*>(src + (long long)s * slot_stride));
+      v = make_float4(fmaf(t.x, e, v.x), fmaf(t.y, e, v.y), fmaf(t.z, e, v.z), fmaf(t.w, e, v.w));
+    }
+    const float inv = 1.f / (L + 1e-16f);
+    v = make_float4(v.x * inv, v.y * inv, v.z * inv, v.w * inv);
+    if (x_next) *reinterpret_cast<float4*>(x_next + (long long)r * ld_x + c) = v;
+    if (acc_out) {
+      float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (acc_in) a = *reinterpret_cast<const float4*>(acc_in + (long long)r * ld_acc + c);
+      *reinterpret_cast<float4*>(acc_out + (long long)r * ld_acc + c) =
+          make_float4((a.x + v.x) * acc_scale, (a.y + v.y) * acc_scale, (a.z + v.z) * acc_scale, (a.w + v.w) * acc_scale);
+    }
+  }
+}
+
+// n floats into the same place of n_dst buffers
+__global__ void __launch_bounds__(256) peer_push_floats_kernel(const float* __restrict__ src, long long n, PeerPtrs dst, int n_dst, long long dst_offset) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    const float v = src[i];
+    for (int q = 0; q < n_dst; ++q) reinterpret_cast<float*>(dst.p[q])[dst_offset + i] = v;
   }
 }
 
@@ -220,6 +269,33 @@ extern "C" int b200rec_peer_reduce(const float* recv, int n_slots, int64_t slot_
   const int grid = (int)std::min<long long>((total + 255) / 256, (long long)b200rec_num_sms() * 8);
   peer_reduce_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(recv, n_slots, slot_stride, ld_recv, (int)rows, d / 4, x_next, ld_x, acc_in, acc_out,
                                                              ld_acc, acc_scale);
+  B200REC_CHECK_LAUNCH();
+  return B200REC_OK;
+}
+
+extern "C" int b200rec_peer_reduce_softmax(const float* recv, const float* stats, int n_slots, int64_t slot_stride, int64_t ld_recv,
+                                           int64_t stats_stride, int64_t rows, int d, float* x_next, int64_t ld_x, const float* acc_in, float* acc_out,
+                                           int64_t ld_acc, float acc_scale, b200rec_stream_t stream) {
+  if (rows == 0) return B200REC_OK;
+  if (!recv || !stats || n_slots <= 0 || rows < 0 || d <= 0 || (d % 4) || (ld_recv % 4) || (slot_stride % 4) || ((uintptr_t)recv % 16) ||
+      (stats_stride % 2) || ((uintptr_t)stats % 8) || (x_next && (((uintptr_t)x_next % 16) || (ld_x % 4))) ||
+      (acc_out && (((uintptr_t)acc_out % 16) || (ld_acc % 4))) || (acc_in && ((uintptr_t)acc_in % 16)) || rows > INT32_MAX)
+    return b200rec_fail(B200REC_ERR_BAD_ARG, "peer_reduce_softmax: operands must allow 128-bit access (d, leading dims multiples of 4; stats 8-byte pairs)");
+  const long long total = rows * (long long)(d / 4);
+  const int grid = (int)std::min<long long>((total + 255) / 256, (long long)b200rec_num_sms() * 8);
+  peer_reduce_softmax_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(recv, stats, n_slots, slot_stride, ld_recv, stats_stride, (int)rows, d / 4, x_next,
+                                                                     ld_x, acc_in, acc_out, ld_acc, acc_scale);
+  B200REC_CHECK_LAUNCH();
+  return B200REC_OK;
+}
+
+extern "C" int b200rec_peer_push_floats(const float* src, int64_t n, void* const* dst, int n_dst, int64_t dst_offset, b200rec_stream_t stream) {
+  if (n == 0) return B200REC_OK;
+  PeerPtrs pp;
+  if (int rc = fill_ptrs(pp, dst, n_dst, "peer_push_floats: bad destination pointers")) return rc;
+  if (!src || n < 0 || dst_offset < 0) return b200rec_fail(B200REC_ERR_BAD_ARG, "peer_push_floats: bad source / size / offset");
+  const int grid = (int)std::min<long long>((n + 255) / 256, (long long)b200rec_num_sms() * 8);
+  peer_push_floats_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(src, n, pp, n_dst, dst_offset);
   B200REC_CHECK_LAUNCH();
   return B200REC_OK;
 }

@@ -65,6 +65,7 @@ struct SpmmParams {
   int push_rpp;              // rows per owner
   long long push_off;        // element offset of this rank's slot inside an arena
   long long push_ld;
+  long long push_ml_off;     // LightGAT + push: element offset of this rank's (m, l) statistics slot inside an arena
 };
 
 // writes 4 consecutive columns [c, c+4) of one finished row
@@ -84,6 +85,13 @@ __device__ __forceinline__ void row_epilogue4(const SpmmParams& p, int row, int 
     st4(p.acc_out + (long long)row * p.ld_acc + c,
         make_float4((a.x + v.x) * p.acc_scale, (a.y + v.y) * p.acc_scale, (a.z + v.z) * p.acc_scale, (a.w + v.w) * p.acc_scale));
   }
+}
+
+// LightGAT + push: a finished row travels unnormalised (relative to its own max m) with its softmax state (m, l); the owner merges the
+// P slots (b200rec_peer_reduce_softmax) and divides by the merged denominator
+__device__ __forceinline__ void push_softmax_state(const SpmmParams& p, int row, float m, float l) {
+  const int o = row / p.push_rpp;
+  *reinterpret_cast<float2*>(reinterpret_cast<float*>(p.push_dst[o]) + p.push_ml_off + 2ll * (row - o * p.push_rpp)) = make_float2(m, l);
 }
 
 template <typename T> struct Lane16;
@@ -223,7 +231,12 @@ spmm_chunk_kernel(const __grid_constant__ SpmmParams p) {
 
   if (g == 0) {
     float sc = (slot < 0 && p.dinv) ? dinv_row : 1.f;
-    if constexpr (GAT) {
+    if constexpr (GAT && PUSH) {
+      if (slot < 0) {
+        sc = 1.f;
+        if (sl == 0) push_softmax_state(p, row, gat_m, gat_l);
+      } else if (sl == 0) { p.partials_ml[2 * slot] = gat_m; p.partials_ml[2 * slot + 1] = gat_l; }
+    } else if constexpr (GAT) {
       if (slot < 0) sc = 1.f / (gat_l + 1e-16f);               // PyG softmax: exp(s - max) / (sum + 1e-16)
       else if (sl == 0) { p.partials_ml[2 * slot] = gat_m; p.partials_ml[2 * slot + 1] = gat_l; }
     }
@@ -302,7 +315,13 @@ spmm_fixup_kernel(const __grid_constant__ SpmmParams p) {
         for (int sidx = 0; sidx < n; ++sidx) M = fmaxf(M, p.partials_ml[2 * (first + sidx)]);
       }
       fixup_accumulate<NV, GAT>(p, first, 0, 1, n, lane, M, acc, Lsum);
-      const float sc = GAT ? 1.f / (Lsum + 1e-16f) : (p.dinv ? __ldg(p.dinv + row) : 1.f);
+      float sc;
+      if constexpr (GAT && PUSH) {
+        sc = 1.f;
+        if (lane == 0) push_softmax_state(p, row, M, Lsum);
+      } else {
+        sc = GAT ? 1.f / (Lsum + 1e-16f) : (p.dinv ? __ldg(p.dinv + row) : 1.f);
+      }
 #pragma unroll
       for (int nv = 0; nv < NV; ++nv)
         row_epilogue4<PUSH>(p, row, lane * 4 + nv * 128, sc, make_float4(acc[nv][0], acc[nv][1], acc[nv][2], acc[nv][3]));
@@ -348,7 +367,13 @@ spmm_fixup_kernel(const __grid_constant__ SpmmParams p) {
           t[nv].x += x.x; t[nv].y += x.y; t[nv].z += x.z; t[nv].w += x.w;
         }
       }
-      const float sc = GAT ? 1.f / (L + 1e-16f) : (p.dinv ? __ldg(p.dinv + row) : 1.f);
+      float sc;
+      if constexpr (GAT && PUSH) {
+        sc = 1.f;
+        if (lane == 0) push_softmax_state(p, row, M, L);
+      } else {
+        sc = GAT ? 1.f / (L + 1e-16f) : (p.dinv ? __ldg(p.dinv + row) : 1.f);
+      }
 #pragma unroll
       for (int nv = 0; nv < NV; ++nv) row_epilogue4<PUSH>(p, row, lane * 4 + nv * 128, sc, t[nv]);
     }
@@ -359,7 +384,8 @@ spmm_fixup_kernel(const __grid_constant__ SpmmParams p) {
 template <int G, int NV, typename T>
 static int launch_chunks(const SpmmParams& p, cudaStream_t st) {
   const int grid = ceil_div_i(p.n_chunks, SPMM_WARPS);
-  if (p.push_parts > 0) spmm_chunk_kernel<G, NV, T, false, true><<<grid, SPMM_WARPS * 32, 0, st>>>(p);
+  if (p.push_parts > 0 && p.att_src) spmm_chunk_kernel<G, NV, T, true, true><<<grid, SPMM_WARPS * 32, 0, st>>>(p);
+  else if (p.push_parts > 0) spmm_chunk_kernel<G, NV, T, false, true><<<grid, SPMM_WARPS * 32, 0, st>>>(p);
   else if (p.att_src) spmm_chunk_kernel<G, NV, T, true><<<grid, SPMM_WARPS * 32, 0, st>>>(p);
   else spmm_chunk_kernel<G, NV, T, false><<<grid, SPMM_WARPS * 32, 0, st>>>(p);
   B200REC_CHECK_LAUNCH();
@@ -381,7 +407,11 @@ static int launch_spmm(const SpmmParams& p, cudaStream_t st) {
   }
   if (p.n_multi > 0) {
     const int g2 = ceil_div_i(p.n_multi, FIX_WARPS);
-    if (p.push_parts > 0) {
+    if (p.push_parts > 0 && p.att_src) {
+      if (p.d <= 128) spmm_fixup_kernel<1, true, true><<<g2, FIX_WARPS * 32, 0, st>>>(p);
+      else if (p.d <= 256) spmm_fixup_kernel<2, true, true><<<g2, FIX_WARPS * 32, 0, st>>>(p);
+      else spmm_fixup_kernel<4, true, true><<<g2, FIX_WARPS * 32, 0, st>>>(p);
+    } else if (p.push_parts > 0) {
       if (p.d <= 128) spmm_fixup_kernel<1, false, true><<<g2, FIX_WARPS * 32, 0, st>>>(p);
       else if (p.d <= 256) spmm_fixup_kernel<2, false, true><<<g2, FIX_WARPS * 32, 0, st>>>(p);
       else spmm_fixup_kernel<4, false, true><<<g2, FIX_WARPS * 32, 0, st>>>(p);
@@ -447,11 +477,14 @@ extern "C" int b200rec_spmm(const b200rec_spmm_t* a, b200rec_stream_t stream) {
   p.n_multi = a->n_multi;
   p.att_src = a->att_src; p.partials_ml = a->partials_ml;
   p.push_parts = a->push_parts; p.push_rpp = a->push_rows_per_part; p.push_off = a->push_offset; p.push_ld = a->push_ld;
+  p.push_ml_off = a->push_stats_offset;
   for (int q = 0; q < B200REC_PEER_MAX; ++q) p.push_dst[q] = a->push_dst[q];
   if (p.push_parts < 0 || p.push_parts > B200REC_PEER_MAX) return b200rec_fail(B200REC_ERR_BAD_ARG, "spmm: push_parts out of range");
   if (p.push_parts > 0) {
-    if (p.att_src || p.push_rpp <= 0 || (p.push_ld % 4) || (p.push_off % 4) || p.push_ld < p.d)
-      return b200rec_fail(B200REC_ERR_BAD_ARG, "spmm: bad push arguments (LightGCN only; offsets / leading dimension multiples of 4)");
+    if (p.push_rpp <= 0 || (p.push_ld % 4) || (p.push_off % 4) || p.push_ld < p.d)
+      return b200rec_fail(B200REC_ERR_BAD_ARG, "spmm: bad push arguments (offsets / leading dimension multiples of 4)");
+    if (p.att_src && (p.push_ml_off <= 0 || (p.push_ml_off % 2)))
+      return b200rec_fail(B200REC_ERR_BAD_ARG, "spmm: LightGAT with push needs push_stats_offset (a positive multiple of 2)");
     for (int q = 0; q < p.push_parts; ++q)
       if (!p.push_dst[q] || ((uintptr_t)p.push_dst[q] % 16)) return b200rec_fail(B200REC_ERR_BAD_ARG, "spmm: null / misaligned push destination");
   }

@@ -722,10 +722,12 @@ def attention_pool_raw(Pc, Pr, Q, *, mode=L.ATT_NET, a2=None, a20=None, bU=None,
 # ------------------------------------------------------------------------------------------------------------------
 # K3 SpMM
 # ------------------------------------------------------------------------------------------------------------------
-def spmm_raw(index, t, *, w, dinv=None, x_next=None, acc_in=None, acc_out=None, acc_scale=1.0, skip_bits=None, att_src=None, push=None):
+def spmm_raw(index, t, *, w, dinv=None, x_next=None, acc_in=None, acc_out=None, acc_scale=1.0, skip_bits=None, att_src=None, push=None,
+             push_stats=None):
     """One propagation step over a `GraphIndex` (graph.py): b200rec_spmm.  Returns nothing; writes x_next / acc_out.
     `push` = (host array of arena addresses, parts, rows per part, element offset, leading dimension): finished rows go to the
-    receive slot of their owner rank instead (peer.py: reduce-scatter fused into the epilogue)."""
+    receive slot of their owner rank instead (peer.py: reduce-scatter fused into the epilogue).  With `att_src` (LightGAT) the
+    pushed rows are unnormalised and `push_stats` = element offset of this rank's (m, l) slot in the arenas is required."""
     _require_cuda(t)
     if t.stride(1) != 1:
         t = t.contiguous()
@@ -757,11 +759,14 @@ def spmm_raw(index, t, *, w, dinv=None, x_next=None, acc_in=None, acc_out=None, 
     d.n_multi = index.n_multi
     if push is not None:
         dst, parts, rpp, off, ld = push
-        if x_next is not None or acc_out is not None or att_src is not None:
-            raise ValueError('spmm: `push` replaces x_next / acc_out (LightGCN only)')
+        if x_next is not None or acc_out is not None:
+            raise ValueError('spmm: `push` replaces x_next / acc_out')
+        if att_src is not None and push_stats is None:
+            raise ValueError('spmm: LightGAT with `push` needs `push_stats` (the softmax state travels with the rows)')
         for q in range(parts):
             d.push_dst[q] = dst[q]
         d.push_parts, d.push_rows_per_part, d.push_offset, d.push_ld = parts, rpp, off, ld
+        d.push_stats_offset = push_stats or 0
     ml = None
     if att_src is not None:
         att_src = att_src.contiguous().float().view(-1)
@@ -820,14 +825,15 @@ def spmm_stream_raw(plan, t, *, x_next=None, acc_in=None, acc_out=None, acc_scal
         L.check(L.lib().b200rec_spmm_stream(C.byref(d), _stream()), 'spmm_stream')
 
 
-def propagate_step(index, t, *, dinv, x_next=None, acc_in=None, acc_out=None, acc_scale=1.0, skip_bits=None, att_src=None, push=None):
+def propagate_step(index, t, *, dinv, x_next=None, acc_in=None, acc_out=None, acc_scale=1.0, skip_bits=None, att_src=None, push=None,
+                   push_stats=None):
     """x' = dinv ∘ (A_w · t) (+ the fused running mean / the push epilogue) on whichever K3 form applies: the edge-balanced stream kernel for
     LightGCN inference at 64 < d <= 128, else the row-owner chunk kernel."""
     if stream_applicable(t, int(index.col.numel()), skip_bits=skip_bits, att_src=att_src):
         from .graph import stream_plan
         return spmm_stream_raw(stream_plan(index, dinv), t, x_next=x_next, acc_in=acc_in, acc_out=acc_out, acc_scale=acc_scale, push=push)
     return spmm_raw(index, t, w=index.w, dinv=dinv, x_next=x_next, acc_in=acc_in, acc_out=acc_out, acc_scale=acc_scale, skip_bits=skip_bits,
-                    att_src=att_src, push=push)
+                    att_src=att_src, push=push, push_stats=push_stats)
 
 
 class _PropagateFn(torch.autograd.Function):

@@ -18,7 +18,16 @@ Per layer l on rank r (one stream, `par = l & 1` selects one of two copies of ev
           signal(T);  t_users for the next layer (local)
 
 After the last layer the owners push the 2B batch rows into every rank's `rows` buffer (peer_gather_rows) and every rank runs the
-MLP on the batch.  signal / wait are epoch flags inside the arenas (release / acquire at system scope; waits time out into an
+MLP on the batch.
+
+LightGAT (convType='LightGAT'): the transforms carry no degree scaling and K3 runs the edge softmax over the source scores
+ps[s] = a_src·x[s].  In A_l a rank sees only its own users' edges of an item row, so K3 pushes that partial row UNNORMALISED (relative
+to its own max m) together with its softmax state (m, l) into the owner's statistics slot; C_l merges the P slots with PyG's rule
+(peer_reduce_softmax: M = max m_s, x = Σ acc_s e^(m_s - M) / (Σ l_s e^(m_s - M) + 1e-16)).  B_l needs the score of every item: the owners
+publish theirs into the score table S[par] of every rank next to T[par], under the same flag.  User scores stay local.
+
+concat=True: every rank keeps its owned rows of comb = [x0 | x1 | ... | xL]; each layer writes its column block (x_next with a leading
+dimension) and the batch rows travel (L+1)·d wide.  signal / wait are epoch flags inside the arenas (release / acquire at system scope; waits time out into an
 error flag instead of hanging the GPU), counted on the device so that a captured CUDA graph can be replayed.
 
 The arenas are cudaMalloc'd by libb200rec and exchanged as CUDA IPC handles through torch.distributed (plumbing).
@@ -162,6 +171,10 @@ class PeerShard:
             cur += slab
         off['rows'] = cur
         cur += _align(2 * batch_max * d_max * 4)
+        # LightGAT: item score tables (P * rpp fp32) and the (m, l) softmax state of every receive slot (P * rpp, 2) fp32
+        for name, nbytes in (('S0', world * rpp * 4), ('S1', world * rpp * 4), ('stats0', world * rpp * 8), ('stats1', world * rpp * 8)):
+            off[name] = cur
+            cur += _align(nbytes)
         off['total'] = cur
         return off
 
@@ -185,27 +198,59 @@ class PeerShard:
         """local copy of the transformed item features of ALL items: (P * rpp, d)"""
         return self.arena.view(self.off[f'T{par}'], (self.table_rows, d), dtype)
 
+    def scores(self, par):
+        """local copy of the LightGAT source scores of ALL items: (P * rpp,) fp32"""
+        return self.arena.view(self.off[f'S{par}'], (self.table_rows,))
+
     def push_spec(self, par, d):
         """(destination arenas, parts, rows per part, element offset of MY receive slot, leading dimension) for K3's epilogue"""
         return (self.arena.ptrs(self.off[f'recv{par}']), self.world, self.rpp, self.rank * self.rpp * d, d)
 
-    def reduce(self, par, d, *, x_next, acc_in, acc_out, acc_scale):
+    def stats_offset(self, par):
+        """element offset of MY (m, l) statistics slot from the push destinations of `push_spec(par, ...)`, which point at the receive
+        sections `recv{par}` of the arenas (LightGAT pushes)"""
+        return (self.off[f'stats{par}'] - self.off[f'recv{par}']) // 4 + self.rank * self.rpp * 2
+
+    def reduce(self, par, d, *, x_next, acc_in, acc_out, acc_scale, softmax=False):
+        """owned item rows from the P receive slots: a sum (LightGCN) or the softmax merge by the slots' (m, l) (LightGAT)"""
         if self.it_rows == 0:
             return
         recv = self.arena.view(self.off[f'recv{par}'], (self.world * self.rpp, d))
+        ld_x = x_next.stride(0) if x_next is not None else 0
+        ld_acc = acc_out.stride(0) if acc_out is not None else d
+        lib = L.lib()
         with torch.cuda.device(self.device), ops._timed('peer_reduce', (self.it_rows, d, self.world)):
-            L.check(L.lib().b200rec_peer_reduce(_ptr(recv), self.world, self.rpp * d, d, self.it_rows, d, _ptr(x_next), d if x_next is not None else 0,
-                                               _ptr(acc_in), _ptr(acc_out), d, float(acc_scale), _stream()), 'peer_reduce')
+            if softmax:
+                stats = self.arena.view(self.off[f'stats{par}'], (self.world * self.rpp, 2))
+                L.check(lib.b200rec_peer_reduce_softmax(_ptr(recv), _ptr(stats), self.world, self.rpp * d, d, 2 * self.rpp, self.it_rows, d, _ptr(x_next),
+                                                        ld_x, _ptr(acc_in), _ptr(acc_out), ld_acc, float(acc_scale), _stream()), 'peer_reduce_softmax')
+            else:
+                L.check(lib.b200rec_peer_reduce(_ptr(recv), self.world, self.rpp * d, d, self.it_rows, d, _ptr(x_next), ld_x,
+                                                _ptr(acc_in), _ptr(acc_out), ld_acc, float(acc_scale), _stream()), 'peer_reduce')
 
-    def push_transform(self, x, lin, par, t_dtype):
+    def push_scores(self, x, lin, par):
+        """S[par][it_r0 : it_r0 + rows] = w·x + b (fp32) on EVERY rank: the LightGAT source scores of the owned items.
+        `lin` = a (weight (1, K), bias (1,) or None) pair."""
+        M = x.shape[0]
+        if M == 0:
+            return
+        local = self.scores(par)[self.it_r0: self.it_r0 + M].view(M, 1)
+        ops.linear_raw(x, lin[0], lin[1], out=local, engine='simt')
+        if self.world > 1:
+            others = (C.c_void_p * (self.world - 1))(*[self.arena.bases[q] + self.off[f'S{par}'] for q in range(self.world) if q != self.rank])
+            with torch.cuda.device(self.device):
+                L.check(L.lib().b200rec_peer_push_floats(_ptr(local), M, others, self.world - 1, self.it_r0, _stream()), 'peer_push_floats')
+
+    def push_transform(self, x, lin, par, t_dtype, scaled=True):
         """T[par][it_r0 : it_r0 + rows] = dinv ∘ (W x + b) on EVERY rank — K1c with the all-gather in its epilogue.
-        `lin` = a Linear module or a (weight, bias) pair."""
+        `lin` = a Linear module or a (weight, bias) pair; `scaled=False` leaves out dinv (LightGAT)."""
         M, K = x.shape
         if M == 0:
             return
         w, b = lin if isinstance(lin, tuple) else (lin.weight, lin.bias)
         N = w.shape[0]
         esz = 2 if t_dtype == torch.bfloat16 else 4
+        row_scale = self.dinv_items_own if scaled else None
         dst = self.arena.ptrs(self.off[f'T{par}'], first=self.rank)
         y_off = self.it_r0 * N
         if K <= 128 and K % 32 == 0 and N <= 128 and x.stride(0) % 4 == 0 and x.data_ptr() % 16 == 0 and x.stride(1) == 1:
@@ -213,12 +258,12 @@ class PeerShard:
             packed = ops._packed_weight(wc, ldw, L.TC_TF32X3)
             bias = None if b is None else b.detach().contiguous().float()
             with torch.cuda.device(self.device), ops._timed('linear_shortk_push', (M, K, N, self.world)):
-                L.check(L.lib().b200rec_linear_shortk_push(_ptr(x), M, K, x.stride(0), _ptr(packed), N, _ptr(bias), _ptr(self.dinv_items_own), 0,
+                L.check(L.lib().b200rec_linear_shortk_push(_ptr(x), M, K, x.stride(0), _ptr(packed), N, _ptr(bias), _ptr(row_scale), 0,
                                                           dst, self.world, y_off, N, ops._dtype_code(t_dtype), _stream()), 'linear_shortk_push')
             return
         # widths the persistent kernel does not take: plain GEMM into the local table, then a copy kernel to the peers
         local = self.table(par, N, t_dtype)[self.it_r0: self.it_r0 + M]
-        ops.linear_raw(x, w, b, row_scale=self.dinv_items_own, out=local)
+        ops.linear_raw(x, w, b, row_scale=row_scale, out=local)
         if self.world > 1:
             if (N * esz) % 16:
                 raise NotImplementedError('the peer path needs rows of the message table that are multiples of 16 bytes')
@@ -322,8 +367,6 @@ def _steps(model, sh: PeerShard, userIds, itemIds, keep=None):
     from .neural_collaborative_filtering.util import run_mlp
     if torch.is_grad_enabled() and any(p.requires_grad for p in model.parameters()):
         raise NotImplementedError('partitioned GraphNCF propagation is inference-only; wrap the call in torch.no_grad()')
-    if model.concat or model.convType != 'LightGCN':
-        raise NotImplementedError('the partitioned path covers LightGCN with mean combine (concat / LightGAT: single GPU)')
     dev = sh.device
     L_ = len(model.gnn_convs)
     d = model.item_embeddings[0].weight.shape[0]
@@ -332,13 +375,23 @@ def _steps(model, sh: PeerShard, userIds, itemIds, keep=None):
     B = int(userIds.shape[0])
     if 2 * B > 2 * sh.batch_max:
         raise ValueError(f'batch of {B} pairs exceeds the partition\'s batch_max {sh.batch_max}')
+    concat, gat = model.concat, model.convType == 'LightGAT'
+    width = d * (L_ + 1) if concat else d                                           # combined embedding [x0 | ... | xL] or their mean
+    if B * width > sh.batch_max * sh.d_max:
+        raise ValueError(f'batch of {B} pairs of {width}-wide concatenated rows exceeds the partition\'s rows buffer (batch_max {sh.batch_max} '
+                         f'x d_max {sh.d_max} floats per side)')
     ie, ue = model.item_embeddings[0], model.user_embeddings[0]
     nu, ni = sh.users_rows, sh.it_rows
     iid, uid = itemIds.long().contiguous(), userIds.long().contiguous()
     empty = lambda n: torch.empty((n, d), dtype=torch.float32, device=dev)
     sh._trace_reset = True
     sh.stamp('start')
-    x0_items, x0_users = empty(ni), empty(nu)
+    if concat:                                                                       # owned rows of comb; x_l is its column block l
+        comb_items, comb_users = (torch.empty((n, width), dtype=torch.float32, device=dev) for n in (ni, nu))
+        x0_items, x0_users = comb_items[:, :d], comb_users[:, :d]
+        block = lambda comb, l: comb[:, d * l: d * (l + 1)]
+    else:
+        x0_items, x0_users = empty(ni), empty(nu)
 
     def embed():                                                                     # x0 = node embeddings of the owned rows (:300-301)
         if ni:
@@ -350,25 +403,37 @@ def _steps(model, sh: PeerShard, userIds, itemIds, keep=None):
     if L_ == 0:
         embed()
     if L_ > 0:
-        lin_u, lin_i, _ = model.gnn_convs[0].typed()
+        conv = model.gnn_convs[0]
+        lin_u, lin_i, _ = conv.typed()
         if model.message_dtype not in ('fp32', 'bf16'):
             raise ValueError("message_dtype must be 'fp32' or 'bf16'")
         t_dtype = torch.bfloat16 if (model.message_dtype == 'bf16' and d % 32 == 0 and d <= 128) else torch.float32
         t_users = torch.empty((max(nu, 1), d), dtype=t_dtype, device=dev)
-        acc_users, acc_items = empty(nu), empty(ni)
-        spare_u = empty(nu) if L_ > 1 else None
-        xi_next = empty(ni) if L_ > 1 else None
+        if not concat:
+            acc_users, acc_items = empty(nu), empty(ni)
+            spare_u = empty(nu) if L_ > 1 else None
+            xi_next = empty(ni) if L_ > 1 else None
+        if gat:                                                                      # LightGAT: source scores, no degree normalisation
+            att_u, att_i = conv.attention()
+            a_u, a_i = (att_u.weight[:, :d], None), (att_i.weight[:, :d], None)
+            ps_u = torch.empty((max(nu, 1), 1), dtype=torch.float32, device=dev)
+        dinv_users, dinv_items = (None, None) if gat else (sh.dinv_users, sh.dinv_items_all)
         main = torch.cuda.current_stream(dev)
         side = sh.side_stream()
         # Layer 0's messages straight from the node features: t0 = dinv ∘ (W_t (W_e f + b_e) + b_t) = dinv ∘ ((W_t W_e) f + (W_t b_e + b_t)) — composite
-        # weights formed once per weight version in float64.  So the first SpMM waits for ONE transform only; the embeddings x0 (needed from the
-        # first running-mean update on) and the broadcast of the item messages run on the side stream underneath it.
-        (Wci, bci), (Wcu, bcu) = _layer0_composites(model, ie, ue, lin_i, lin_u)
+        # weights formed once per weight version in float64 (LightGAT: also the scores a·x0 = (a W_e) f + a b_e).  So the first SpMM waits for ONE
+        # transform only; the embeddings x0 (needed from the first running-mean update on) and the broadcast of the item messages run on the side
+        # stream underneath it.
+        (Wci, bci), (Wcu, bcu), sc_i, sc_u = _layer0_composites(model, ie, ue, lin_i, lin_u, *((att_i, att_u) if gat else ()))
         if nu:
-            ops.linear_raw(sh.user_features_own, Wcu, bcu, row_scale=sh.dinv_users, out=t_users[:nu])
+            ops.linear_raw(sh.user_features_own, Wcu, bcu, row_scale=dinv_users, out=t_users[:nu])
+            if gat:
+                ops.linear_raw(sh.user_features_own, *sc_u, out=ps_u[:nu], engine='simt')
 
         def layer0_side():
-            sh.push_transform(sh.item_features_own, (Wci, bci), 0, t_dtype)
+            sh.push_transform(sh.item_features_own, (Wci, bci), 0, t_dtype, scaled=not gat)
+            if gat:
+                sh.push_scores(sh.item_features_own, sc_i, 0)
             sh.signal(CH_T0)
             embed()
 
@@ -384,9 +449,16 @@ def _steps(model, sh: PeerShard, userIds, itemIds, keep=None):
             sh.stamp(f'C{l} begin')
             sh.wait(CH_A0 + par)
             sh.stamp(f'C{l} partials arrived')
-            sh.reduce(par, d, x_next=None if last else xi_next, acc_in=x0_items if l == 0 else acc_items, acc_out=acc_items, acc_scale=scale)
+            if concat:
+                xi = block(comb_items, l + 1)
+                sh.reduce(par, d, x_next=xi, acc_in=None, acc_out=None, acc_scale=1.0, softmax=gat)
+            else:
+                xi = None if last else xi_next
+                sh.reduce(par, d, x_next=xi, acc_in=x0_items if l == 0 else acc_items, acc_out=acc_items, acc_scale=scale, softmax=gat)
             if not last:
-                sh.push_transform(xi_next, lin_i, 1 - par, t_dtype)
+                sh.push_transform(xi, lin_i, 1 - par, t_dtype, scaled=not gat)
+                if gat:
+                    sh.push_scores(xi, a_i, 1 - par)
                 sh.signal(CH_T0 + (1 - par))
             sh.stamp(f'C{l} end')
 
@@ -395,7 +467,8 @@ def _steps(model, sh: PeerShard, userIds, itemIds, keep=None):
             scale = 1.0 / (L_ + 1) if last else 1.0
             sh.stamp(f'A{l} begin')
             if nu:                                                                   # A_l: partial item rows -> owners' receive slots
-                ops.propagate_step(sh.index_items, t_users, dinv=sh.dinv_items_all, push=sh.push_spec(par, d))
+                ops.propagate_step(sh.index_items, t_users, dinv=dinv_items, push=sh.push_spec(par, d), att_src=ps_u if gat else None,
+                                   push_stats=sh.stats_offset(par) if gat else None)
             sh.signal(CH_A0 + par)
             sh.stamp(f'A{l} end')
             forked = torch.cuda.Event()
@@ -410,23 +483,29 @@ def _steps(model, sh: PeerShard, userIds, itemIds, keep=None):
             if l == 0:
                 main.wait_event(x0_ready)                                            # x0_users is B_0's running-mean input
             sh.stamp(f'B{l} table arrived')
+            xu = block(comb_users, l + 1) if concat else (None if last else spare_u)
             if nu:                                                                   # B_l: own user rows from the gathered table
-                ops.propagate_step(sh.index_users, sh.table(par, d, t_dtype), dinv=sh.dinv_users, x_next=None if last else spare_u,
-                                   acc_in=x0_users if l == 0 else acc_users, acc_out=acc_users, acc_scale=scale)
+                acc = {} if concat else dict(acc_in=x0_users if l == 0 else acc_users, acc_out=acc_users, acc_scale=scale)
+                ops.propagate_step(sh.index_users, sh.table(par, d, t_dtype), dinv=dinv_users, x_next=xu, att_src=sh.scores(par) if gat else None,
+                                   **acc)
             sh.stamp(f'B{l} end')
             if not last and nu:
-                ops.linear_raw(spare_u, lin_u.weight, lin_u.bias, row_scale=sh.dinv_users, out=t_users[:nu])
+                ops.linear_raw(xu, lin_u.weight, lin_u.bias, row_scale=dinv_users, out=t_users[:nu])
+                if gat:
+                    ops.linear_raw(xu, *a_u, out=ps_u[:nu], engine='simt')
         main.wait_event(joined)
         sh.stamp('layers joined')
+    if concat:
+        acc_items, acc_users = comb_items, comb_users
     if keep is not None:                        # tests: the owned rows of the combined embedding
         keep['items'], keep['users'] = acc_items, acc_users
-    sh.gather_rows(acc_items, sh.it_r0, ni, iid, 0, d)
-    sh.gather_rows(acc_users, sh.nI + sh.users_r0, nu, uid, B, d)
+    sh.gather_rows(acc_items, sh.it_r0, ni, iid, 0, width)
+    sh.gather_rows(acc_users, sh.nI + sh.users_r0, nu, uid, B, width)
     sh.signal(CH_R)
     yield
     sh.wait(CH_R)
     sh.stamp('batch rows arrived')
-    rows = sh.rows_view(2 * B, d)
+    rows = sh.rows_view(2 * B, width)
     if model.MLP is None:
         out = ops.rowdot(rows[B:], rows[:B])
     else:
@@ -439,18 +518,28 @@ def _steps(model, sh: PeerShard, userIds, itemIds, keep=None):
     return out
 
 
-def _layer0_composites(model, ie, ue, lin_i, lin_u):
-    """((W_i2u·W_item, W_i2u·b_item + b_i2u), (W_u2i·W_user, W_u2i·b_user + b_u2i)) as cached fp32 tensors (float64 products, rounded once)"""
-    def comp(lin, emb):
-        w = (lin.weight.detach().double() @ emb.weight.detach().double()).float().contiguous()
+def _layer0_composites(model, ie, ue, lin_i, lin_u, att_i=None, att_u=None):
+    """((W_i2u·W_item, W_i2u·b_item + b_i2u), (W_u2i·W_user, W_u2i·b_user + b_u2i), item score pair, user score pair) as cached fp32 tensors
+    (float64 products, rounded once).  With the LightGAT attention Linears a score pair is (a·W_emb, a·b_emb), a = the source half of the
+    attention weight (the scores a·x0 of layer 0); None otherwise."""
+    d = ie.weight.shape[0]
+
+    def comp(w_out, b_out, emb):
+        w = (w_out.detach().double() @ emb.weight.detach().double()).float().contiguous()
         eb = emb.bias.detach().double() if emb.bias is not None else torch.zeros(emb.weight.shape[0], dtype=torch.float64, device=w.device)
-        b = lin.weight.detach().double() @ eb
-        if lin.bias is not None:
-            b = b + lin.bias.detach().double()
+        b = w_out.detach().double() @ eb
+        if b_out is not None:
+            b = b + b_out.detach().double()
         return w, b.float().contiguous()
 
-    return model._peer_layer0.get((ie.weight, ie.bias, ue.weight, ue.bias, lin_i.weight, lin_i.bias, lin_u.weight, lin_u.bias),
-                                  lambda: (comp(lin_i, ie), comp(lin_u, ue)))
+    def build():
+        out = (comp(lin_i.weight, lin_i.bias, ie), comp(lin_u.weight, lin_u.bias, ue))
+        if att_i is None:
+            return out + (None, None)
+        return out + (comp(att_i.weight[:, :d], None, ie), comp(att_u.weight[:, :d], None, ue))
+
+    att = (None, None) if att_i is None else (att_i.weight, att_u.weight)
+    return model._peer_layer0.get((ie.weight, ie.bias, ue.weight, ue.bias, lin_i.weight, lin_i.bias, lin_u.weight, lin_u.bias) + att, build)
 
 
 def forward_peer(model, sh: PeerShard, userIds, itemIds, keep=None):

@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define B200REC_VERSION 206
+#define B200REC_VERSION 207
 
 typedef void* b200rec_stream_t; /* cudaStream_t */
 
@@ -352,12 +352,16 @@ typedef struct {
   float* partials_ml;   /* (n_slots, 2) scratch for the softmax state of multi-chunk rows */
   /* reduce-scatter fused into the epilogue (partitioned propagation): when push_parts > 0 a finished row r is not written to
    * x_next / acc_out but into the receive slot of its OWNER rank o = r / push_rows_per_part, i.e. to
-   * (float*)push_dst[o] + push_offset + (r - o * push_rows_per_part) * push_ld — push_dst are the peer-mapped arenas */
+   * (float*)push_dst[o] + push_offset + (r - o * push_rows_per_part) * push_ld — push_dst are the peer-mapped arenas.
+   * With att_src (LightGAT) the pushed row is NOT normalised: it is Σ exp(s - m)·w·t relative to the row's own max m, and its
+   * softmax state (m, l = Σ exp(s - m)) goes to (float*)push_dst[o] + push_stats_offset + 2 * (r - o * push_rows_per_part);
+   * b200rec_peer_reduce_softmax merges the slots.  push_stats_offset must then be a positive multiple of 2 (0 = not given). */
   void* push_dst[B200REC_PEER_MAX];
   int push_parts;
   int push_rows_per_part;
   int64_t push_offset;
   int64_t push_ld;
+  int64_t push_stats_offset;
 } b200rec_spmm_t;
 int b200rec_spmm(const b200rec_spmm_t* a, b200rec_stream_t stream);
 
@@ -497,9 +501,18 @@ int b200rec_peer_wait(const uint32_t* flags, int n_peers, int channel, uint32_t*
 /* x_next[r] = sum_{s < n_slots} recv[s * slot_stride + r * ld_recv ..] (slot order);  acc_out = (acc_in + x_next) * acc_scale */
 int b200rec_peer_reduce(const float* recv, int n_slots, int64_t slot_stride, int64_t ld_recv, int64_t rows, int d, float* x_next,
                         int64_t ld_x, const float* acc_in, float* acc_out, int64_t ld_acc, float acc_scale, b200rec_stream_t stream);
+/* LightGAT form of b200rec_peer_reduce: slot s holds an unnormalised row and its softmax state (m_s, l_s) at
+ * stats[s * stats_stride + 2 r ..].  In slot order, over the slots with l_s > 0 only (a slot nobody wrote is zero):
+ *   M = max m_s,   L = Σ l_s·exp(m_s - M),   x_next[r] = Σ recv_s[r]·exp(m_s - M) / (L + 1e-16)   (0 for a row without edges);
+ * acc_out = (acc_in + x_next) * acc_scale as above */
+int b200rec_peer_reduce_softmax(const float* recv, const float* stats, int n_slots, int64_t slot_stride, int64_t ld_recv, int64_t stats_stride,
+                                int64_t rows, int d, float* x_next, int64_t ld_x, const float* acc_in, float* acc_out, int64_t ld_acc,
+                                float acc_scale, b200rec_stream_t stream);
 /* copies src (rows, d) to (float*)dst[q] + dst_offset for every q < n_dst (dst: HOST array of device pointers) */
 int b200rec_peer_push_rows(const float* src, int64_t ld_src, int64_t rows, int d, void* const* dst, int n_dst, int64_t dst_offset,
                            int64_t ld_dst, b200rec_stream_t stream);
+/* copies n floats src[0 .. n) to (float*)dst[q] + dst_offset for every q < n_dst (one score per item row: LightGAT's source scores) */
+int b200rec_peer_push_floats(const float* src, int64_t n, void* const* dst, int n_dst, int64_t dst_offset, b200rec_stream_t stream);
 /* batch rows (models/gnn_ncf.py:354-357 on a partitioned embedding): for every j < n_ids with row0 <= ids[j] < row0 + rows,
  * row (dst_offset / ld_dst + j) of every destination receives table[ids[j] - row0] * scale */
 int b200rec_peer_gather_rows(const float* table, int64_t ld, int64_t row0, int64_t rows, const int64_t* ids, int64_t n_ids, int d,
