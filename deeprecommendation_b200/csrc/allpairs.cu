@@ -549,6 +549,10 @@ allpairs_merge_kernel(const float* __restrict__ part_val, const int* __restrict_
 // CTA = 64 users x 128-item tiles, a thread owns 4 users x 8 items = 32 accumulators and walks h through shared memory
 // (user rows resident, item tile transposed to h-major so that a warp's 16 item columns are conflict-free); per h and pair one FADD,
 // one FMNMX, one FFMA.  Same top-k epilogue / split lists / merge kernel as the tensor-core path.
+//
+// DOT = true is the dot-product model's form of the same kernel, score(u, i) = A[u]·B[i] (GraphNCF(use_dot_product=True) over a
+// partitioned graph, peer.recommend_peer): one FFMA per h and pair and no w2 / b2.  The top-k never needs the (nU x nI) score matrix,
+// which a GEMM + row-wise top-k would have to write (5 TB for one rank of BASELINE configs[4]).
 constexpr int RD_UT = 64, RD_IT = 128, RD_HC = 64, RD_THREADS = 256;
 
 struct ReluDotParams {
@@ -560,6 +564,7 @@ struct ReluDotParams {
   const int* seen_ptr; const int* seen_idx;
 };
 
+template <bool DOT>
 __global__ void __launch_bounds__(RD_THREADS, 1)
 allpairs_relu_dot_kernel(const ReluDotParams p) {
   extern __shared__ __align__(16) unsigned char rd_smem[];
@@ -580,7 +585,8 @@ allpairs_relu_dot_kernel(const ReluDotParams p) {
     const int r = (i * 4) / H1, c = (i * 4) % H1;
     reinterpret_cast<float4*>(sA)[i] = r < users_here ? __ldg(reinterpret_cast<const float4*>(p.A + (long long)(u0 + r) * H1 + c)) : make_float4(0.f, 0.f, 0.f, 0.f);
   }
-  for (int i = tid; i < H1; i += RD_THREADS) sW[i] = __ldg(p.w2 + i);
+  if constexpr (!DOT)
+    for (int i = tid; i < H1; i += RD_THREADS) sW[i] = __ldg(p.w2 + i);
   for (int i = tid; i < RD_UT * AP_KMAX; i += RD_THREADS) { sm_lv[i] = -INFINITY; sm_li[i] = -1; }
   if (tid < RD_UT) sm_thr[tid] = -INFINITY;
   __syncthreads();
@@ -622,7 +628,7 @@ allpairs_relu_dot_kernel(const ReluDotParams p) {
       const float* wt = sW + hc * RD_HC;
 #pragma unroll 4
       for (int h = 0; h < RD_HC; ++h) {
-        const float w = wt[h];
+        [[maybe_unused]] const float w = DOT ? 0.f : wt[h];
         float a[4], b[8];
 #pragma unroll
         for (int q = 0; q < 4; ++q) a[q] = at[q * 16 * H1 + h];
@@ -631,13 +637,16 @@ allpairs_relu_dot_kernel(const ReluDotParams p) {
 #pragma unroll
         for (int q = 0; q < 4; ++q)
 #pragma unroll
-          for (int j = 0; j < 8; ++j) acc[q][j] = fmaf(w, fmaxf(a[q] + b[j], 0.f), acc[q][j]);
+          for (int j = 0; j < 8; ++j) {
+            if constexpr (DOT) acc[q][j] = fmaf(a[q], b[j], acc[q][j]);
+            else acc[q][j] = fmaf(w, fmaxf(a[q] + b[j], 0.f), acc[q][j]);
+          }
       }
     }
 #pragma unroll
     for (int q = 0; q < 4; ++q)
 #pragma unroll
-      for (int j = 0; j < 8; ++j) sS[(ty + 16 * q) * RD_IT + tx + 16 * j] = acc[q][j] + p.b2;
+      for (int j = 0; j < 8; ++j) sS[(ty + 16 * q) * RD_IT + tx + 16 * j] = DOT ? acc[q][j] : acc[q][j] + p.b2;
     __syncthreads();
     // ---- tile epilogue: warp w owns users w, w + 8, ... ----
     for (int ul = warp; ul < users_here; ul += RD_THREADS / 32) {
@@ -828,24 +837,25 @@ static int rd_auto_splits(int64_t nU, int64_t nI) {
 
 extern "C" int b200rec_allpairs_relu_dot_splits(int64_t nU, int64_t nI) { return (nU <= 0 || nI <= 0) ? 1 : rd_auto_splits(nU, nI); }
 
-extern "C" int b200rec_allpairs_relu_dot_topk(const float* A, const float* B, int64_t nU, int64_t nI, int H1, const float* w2, float b2, int k,
-                                              int n_splits, const int* seen_ptr, const int* seen_idx, float* scores, int64_t lds, float* top_val,
-                                              int64_t* top_idx, void* workspace, size_t workspace_bytes, b200rec_stream_t stream) {
-  cudaStream_t st = (cudaStream_t)stream;
-  if (nU < 0 || nI < 0 || !w2 || (nU > 0 && nI > 0 && (!A || !B))) return b200rec_fail(B200REC_ERR_BAD_ARG, "allpairs_relu_dot: null operand");
-  if (H1 <= 0 || H1 > 256 || (H1 % 64)) return b200rec_fail(B200REC_ERR_UNSUPPORTED, "allpairs_relu_dot: H1 must be 64, 128, 192 or 256 (zero-pad)");
-  if (k < 0 || k > AP_KMAX) return b200rec_fail(B200REC_ERR_BAD_ARG, "allpairs_relu_dot: need 0 <= k <= 64");
-  if (k > 0 && (!top_val || !top_idx)) return b200rec_fail(B200REC_ERR_BAD_ARG, "allpairs_relu_dot: top-k outputs missing");
-  if (k == 0 && !scores) return b200rec_fail(B200REC_ERR_BAD_ARG, "allpairs_relu_dot: nothing to compute");
-  if (scores && lds < nI) return b200rec_fail(B200REC_ERR_BAD_ARG, "allpairs_relu_dot: lds too small");
-  if ((seen_ptr == nullptr) != (seen_idx == nullptr)) return b200rec_fail(B200REC_ERR_BAD_ARG, "allpairs_relu_dot: seen CSR needs both arrays");
-  if (nU > INT32_MAX / 2 || nI > INT32_MAX / 2) return b200rec_fail(B200REC_ERR_UNSUPPORTED, "allpairs_relu_dot: dims > 2^30");
-  if ((uintptr_t)A % 16 || (uintptr_t)B % 16) return b200rec_fail(B200REC_ERR_BAD_ARG, "allpairs_relu_dot: A / B must be 16-byte aligned");
+// the checks, split lists and merge of both instantiations; `what` names the entry point in the error messages
+template <bool DOT>
+static int rd_topk(const char* const (&what)[11], const float* A, const float* B, int64_t nU, int64_t nI, int H1, const float* w2, float b2, int k,
+                   int n_splits, const int* seen_ptr, const int* seen_idx, float* scores, int64_t lds, float* top_val, int64_t* top_idx,
+                   void* workspace, size_t workspace_bytes, cudaStream_t st) {
+  if (nU < 0 || nI < 0 || (!DOT && !w2) || (nU > 0 && nI > 0 && (!A || !B))) return b200rec_fail(B200REC_ERR_BAD_ARG, what[0]);
+  if (H1 <= 0 || H1 > 256 || (H1 % 64)) return b200rec_fail(B200REC_ERR_UNSUPPORTED, what[1]);
+  if (k < 0 || k > AP_KMAX) return b200rec_fail(B200REC_ERR_BAD_ARG, what[2]);
+  if (k > 0 && (!top_val || !top_idx)) return b200rec_fail(B200REC_ERR_BAD_ARG, what[3]);
+  if (k == 0 && !scores) return b200rec_fail(B200REC_ERR_BAD_ARG, what[4]);
+  if (scores && lds < nI) return b200rec_fail(B200REC_ERR_BAD_ARG, what[5]);
+  if ((seen_ptr == nullptr) != (seen_idx == nullptr)) return b200rec_fail(B200REC_ERR_BAD_ARG, what[6]);
+  if (nU > INT32_MAX / 2 || nI > INT32_MAX / 2) return b200rec_fail(B200REC_ERR_UNSUPPORTED, what[7]);
+  if ((uintptr_t)A % 16 || (uintptr_t)B % 16) return b200rec_fail(B200REC_ERR_BAD_ARG, what[8]);
   if (nU == 0) return B200REC_OK;
   if (n_splits <= 0) n_splits = nI > 0 ? rd_auto_splits(nU, nI) : 1;
-  if (n_splits > 128) return b200rec_fail(B200REC_ERR_BAD_ARG, "allpairs_relu_dot: at most 128 item splits");
+  if (n_splits > 128) return b200rec_fail(B200REC_ERR_BAD_ARG, what[9]);
   if (k > 0 && (!workspace || workspace_bytes < b200rec_allpairs_workspace(nU, k, n_splits) || (uintptr_t)workspace % 16))
-    return b200rec_fail(B200REC_ERR_WORKSPACE, "allpairs_relu_dot: workspace too small (b200rec_allpairs_workspace)");
+    return b200rec_fail(B200REC_ERR_WORKSPACE, what[10]);
   ReluDotParams p;
   p.A = A; p.B = B; p.w2 = w2; p.b2 = b2; p.nU = (int)nU; p.nI = (int)nI; p.H1 = H1; p.k = k; p.n_splits = n_splits;
   p.items_per_split = (int)(((nI + n_splits - 1) / n_splits + RD_IT - 1) / RD_IT * RD_IT);
@@ -856,9 +866,9 @@ extern "C" int b200rec_allpairs_relu_dot_topk(const float* A, const float* B, in
   if (nI > 0) {
     const size_t smem = rd_smem_bytes(H1);
     static B200recSmemOptIn opted;
-    B200REC_CUDA(b200rec_opt_in_smem(opted, allpairs_relu_dot_kernel, (int)rd_smem_bytes(256)));
+    B200REC_CUDA(b200rec_opt_in_smem(opted, allpairs_relu_dot_kernel<DOT>, (int)rd_smem_bytes(256)));
     dim3 grid((unsigned)((nU + RD_UT - 1) / RD_UT), (unsigned)n_splits);
-    allpairs_relu_dot_kernel<<<grid, RD_THREADS, smem, st>>>(p);
+    allpairs_relu_dot_kernel<DOT><<<grid, RD_THREADS, smem, st>>>(p);
     B200REC_CHECK_LAUNCH();
   } else if (k > 0) {
     B200REC_CUDA(cudaMemsetAsync(p.part_idx, 0xff, (size_t)nU * n_splits * k * sizeof(int), st));
@@ -868,4 +878,28 @@ extern "C" int b200rec_allpairs_relu_dot_topk(const float* A, const float* B, in
     B200REC_CHECK_LAUNCH();
   }
   return B200REC_OK;
+}
+
+extern "C" int b200rec_allpairs_relu_dot_topk(const float* A, const float* B, int64_t nU, int64_t nI, int H1, const float* w2, float b2, int k,
+                                              int n_splits, const int* seen_ptr, const int* seen_idx, float* scores, int64_t lds, float* top_val,
+                                              int64_t* top_idx, void* workspace, size_t workspace_bytes, b200rec_stream_t stream) {
+  static const char* const what[11] = {
+      "allpairs_relu_dot: null operand", "allpairs_relu_dot: H1 must be 64, 128, 192 or 256 (zero-pad)", "allpairs_relu_dot: need 0 <= k <= 64",
+      "allpairs_relu_dot: top-k outputs missing", "allpairs_relu_dot: nothing to compute", "allpairs_relu_dot: lds too small",
+      "allpairs_relu_dot: seen CSR needs both arrays", "allpairs_relu_dot: dims > 2^30", "allpairs_relu_dot: A / B must be 16-byte aligned",
+      "allpairs_relu_dot: at most 128 item splits", "allpairs_relu_dot: workspace too small (b200rec_allpairs_workspace)"};
+  return rd_topk<false>(what, A, B, nU, nI, H1, w2, b2, k, n_splits, seen_ptr, seen_idx, scores, lds, top_val, top_idx, workspace, workspace_bytes,
+                        (cudaStream_t)stream);
+}
+
+extern "C" int b200rec_allpairs_dot_topk(const float* A, const float* B, int64_t nU, int64_t nI, int H, int k, int n_splits, const int* seen_ptr,
+                                         const int* seen_idx, float* scores, int64_t lds, float* top_val, int64_t* top_idx, void* workspace,
+                                         size_t workspace_bytes, b200rec_stream_t stream) {
+  static const char* const what[11] = {
+      "allpairs_dot: null operand", "allpairs_dot: H must be 64, 128, 192 or 256 (zero-pad)", "allpairs_dot: need 0 <= k <= 64",
+      "allpairs_dot: top-k outputs missing", "allpairs_dot: nothing to compute", "allpairs_dot: lds too small",
+      "allpairs_dot: seen CSR needs both arrays", "allpairs_dot: dims > 2^30", "allpairs_dot: A / B must be 16-byte aligned",
+      "allpairs_dot: at most 128 item splits", "allpairs_dot: workspace too small (b200rec_allpairs_workspace)"};
+  return rd_topk<true>(what, A, B, nU, nI, H, nullptr, 0.f, k, n_splits, seen_ptr, seen_idx, scores, lds, top_val, top_idx, workspace, workspace_bytes,
+                       (cudaStream_t)stream);
 }

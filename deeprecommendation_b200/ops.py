@@ -1294,6 +1294,40 @@ def allpairs_relu_dot_raw(A, B, w2, b2, k, *, return_scores=False, seen=None, n_
     return val, idx, scores
 
 
+def allpairs_dot_topk_raw(A, B, k, *, return_scores=False, seen=None, n_splits=0):
+    """score(u, i) = A[u]·B[i] for every pair + the k best columns per row — b200rec_allpairs_dot_topk (exact fp32, the dot form of the
+    relu_dot kernel).  A (nU, H), B (nI, H) fp32 with H <= 256; widths that are not a multiple of 64 are zero-padded here.  Returns
+    (top_val (nU, k), top_idx (nU, k) int64, scores (nU, nI) | None); `seen` as for `allpairs_topk_raw`."""
+    _require_cuda(A, B)
+    nU, H = A.shape
+    nI = B.shape[0]
+    if B.shape[1] != H:
+        raise ValueError('allpairs_dot: A and B disagree on the width')
+    Hp = max(64, (H + 63) // 64 * 64)
+    if Hp > 256:
+        raise NotImplementedError(f'all-pairs dot kernel: embedding width {H} > 256')
+    dev = A.device
+    pad = lambda t: t.float().contiguous() if H == Hp else torch.nn.functional.pad(t.float(), (0, Hp - H)).contiguous()
+    A, B = pad(A), pad(B)
+    lib = L.lib()
+    if n_splits <= 0:
+        n_splits = lib.b200rec_allpairs_relu_dot_splits(nU, nI)            # same tiling as relu_dot
+    val = torch.empty((nU, k), dtype=torch.float32, device=dev) if k > 0 else None
+    idx = torch.empty((nU, k), dtype=torch.int64, device=dev) if k > 0 else None
+    scores = torch.empty((nU, nI), dtype=torch.float32, device=dev) if return_scores else None
+    wsb = lib.b200rec_allpairs_workspace(nU, k, n_splits) if k > 0 else 0
+    ws = torch.empty(wsb, dtype=torch.uint8, device=dev) if wsb else None
+    sp = si = None
+    if seen is not None:
+        sp, si = seen[0].contiguous().int(), seen[1].contiguous().int()
+        if sp.numel() != nU + 1:
+            raise ValueError('allpairs: seen_ptr must have nU + 1 entries')
+    with _on(dev), _timed('allpairs_dot', (nU, nI, Hp, k)):
+        L.check(lib.b200rec_allpairs_dot_topk(_ptr(A), _ptr(B), nU, nI, Hp, k, n_splits, _ptr(sp), _ptr(si), _ptr(scores), nI, _ptr(val), _ptr(idx),
+                                              _ptr(ws), wsb, _stream()), 'allpairs_dot_topk')
+    return val, idx, scores
+
+
 def mlp_allpairs_topk(row_emb, col_emb, weights, biases, k, *, rows_first=True, precision='fp32', seen=None, return_scores=False,
                       n_splits=0):
     """Scores `MLP(cat(row_emb[u], col_emb[i]))` (rows_first) or `MLP(cat(col_emb[i], row_emb[u]))` for EVERY (u, i) and keeps

@@ -77,6 +77,11 @@ class _LocalIndex(GraphIndex):
         self.e1, self.e2 = int(col.numel()), 0
         self.chunk_size = chunk
         self.symmetric, self.w_bwd, self._hash = False, None, None
+        if self.num_nodes == 0:                      # a rank without rows of this type (more ranks than users): no SpMM ever runs on it
+            empty = torch.zeros(0, dtype=torch.int32, device=row_ptr.device)
+            self.n_chunks = self.n_multi = self.n_slots = 0
+            self.chunk_row = self.chunk_start = self.chunk_slot = self.multi_row = self.multi_first_slot = self.multi_n_slots = empty
+            return
         self._build_plan()
 
 
@@ -186,15 +191,18 @@ class UserPartitionedGraph:
         return (local >= 0) & (local < self.users.rows), local
 
 
-def partition_graph(graph, group=None, scheme: str = 'peer', d_max: int = 128, batch_max: int = 8192):
+def partition_graph(graph, group=None, scheme: str = 'peer', d_max: int = 128, batch_max: int = 8192, catalogue_width: int = 0):
     """'peer' (default): users partitioned, the exchange written as this library's own kernels over peer-mapped memory (peer.py);
-    'reduce' / 'gather': the same partitions with NCCL collectives issued from Python (kept as the comparison baseline)."""
+    'reduce' / 'gather': the same partitions with NCCL collectives issued from Python (kept as the comparison baseline).
+    `catalogue_width` (scheme 'peer' only): floats per item row of the catalogue section of `peer.recommend_peer`."""
     if scheme not in ('peer', 'reduce', 'gather'):
         raise ValueError(scheme)
+    if catalogue_width and scheme != 'peer':
+        raise ValueError("catalogue_width: only scheme 'peer' serves recommend_peer")
     get_index(graph)                                   # (resets a stale partition of an edited graph)
     if scheme == 'peer':
         from .peer import partition_graph_peer
-        pg = partition_graph_peer(graph, group, d_max=d_max, batch_max=batch_max)
+        pg = partition_graph_peer(graph, group, d_max=d_max, batch_max=batch_max, catalogue_width=catalogue_width)
     else:
         pg = UserPartitionedGraph(graph, group) if scheme == 'reduce' else PartitionedGraph(graph, group)
     try:

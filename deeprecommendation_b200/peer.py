@@ -30,6 +30,17 @@ concat=True: every rank keeps its owned rows of comb = [x0 | x1 | ... | xL]; eac
 dimension) and the batch rows travel (L+1)·d wide.  signal / wait are epoch flags inside the arenas (release / acquire at system scope; waits time out into an
 error flag instead of hanging the GPU), counted on the device so that a captured CUDA graph can be replayed.
 
+Whole-catalogue top-k (`recommend_peer`): the same propagation (`_propagate`, shared with the forward), then
+
+    cat   every owner pushes its final item rows into the section `cat` of EVERY rank (itself included) at rows it_r0 ..;  signal(C)
+    score wait(C);  the owned users' rows against cat[:nI] — K5 / relu_dot through ops.mlp_allpairs_topk, or the dot form of relu_dot
+    close signal(D);  wait(D)
+
+C orders the pushes before any rank reads the table.  D orders every rank's scoring before the next call of any rank writes `cat` again:
+without it a fast rank's next push would overwrite rows a slow rank is still scoring from, and with L = 0 there are no layer flags in
+between that could order it.  The propagation sections are ordered exactly as for the forward (a recommend ends with all ranks past D, a
+stronger state than the end of a forward), so forwards and recommends can follow each other in any order on the same epoch counters.
+
 The arenas are cudaMalloc'd by libb200rec and exchanged as CUDA IPC handles through torch.distributed (plumbing).
 `emulated_shards` builds all P shards inside ONE process (plain device buffers, the same kernels and addresses) so that the
 exchange logic is covered by the single-GPU test-suite; there the ranks advance in lock step, segment by segment.
@@ -44,10 +55,11 @@ import torch
 
 from . import _lib as L
 from . import ops
+from .derived import Derived
 from .graph import get_index
 from .ops import _ptr, _stream
 
-CH_T0, CH_T1, CH_A0, CH_A1, CH_R, CH_E = 0, 1, 2, 3, 4, 5
+CH_T0, CH_T1, CH_A0, CH_A1, CH_R, CH_E, CH_C, CH_D = 0, 1, 2, 3, 4, 5, 6, 7
 _CTRL_BYTES = 4096                 # flags uint32[16][16] (1 KB) | counters uint32[32] | err int32
 _OFF_COUNTERS = L.PEER_CHANNELS * L.PEER_MAX * 4
 _OFF_ERR = _OFF_COUNTERS + 2 * L.PEER_CHANNELS * 4
@@ -143,7 +155,7 @@ class PeerShard:
     """What rank `rank` keeps of a user-partitioned graph + the arena layout (identical on every rank)."""
 
     def __init__(self, *, rank, world, nI, nU, d_max, rpp, users_r0, users_rows, index_users, index_items, dinv_users, dinv_items_all,
-                 item_features_own, user_features_own, arena, batch_max, edges_total, edges_own):
+                 item_features_own, user_features_own, arena, batch_max, edges_total, edges_own, catalogue_width=0):
         self.rank, self.world, self.nI, self.nU, self.rpp = rank, world, int(nI), int(nU), int(rpp)
         self.N = self.nI + self.nU
         self.users_r0, self.users_rows = int(users_r0), int(users_rows)
@@ -155,15 +167,17 @@ class PeerShard:
         self.item_features_own, self.user_features_own = item_features_own, user_features_own
         self.arena, self.d_max, self.batch_max = arena, int(d_max), int(batch_max)
         self.edges_total, self.edges_own = int(edges_total), int(edges_own)
-        self.off = self.layout(world, self.rpp, self.d_max, self.batch_max)
+        self.catalogue_width = int(catalogue_width)
+        self.off = self.layout(world, self.rpp, self.d_max, self.batch_max, self.catalogue_width)
         self.device = arena.buf.device
         self._flag_ptrs = arena.ptrs(0)
         self._counters = arena.buf[_OFF_COUNTERS:].data_ptr()
         self._err = arena.view(_OFF_ERR, (1,), torch.int32)
         self.table_rows = world * self.rpp
+        self._seen = Derived(1)                                        # seen CSR of every owned user (recommend_peer, users=None)
 
     @staticmethod
-    def layout(world, rpp, d_max, batch_max):
+    def layout(world, rpp, d_max, batch_max, catalogue_width=0):
         off, cur = {}, _CTRL_BYTES
         slab = _align(world * rpp * d_max * 4)
         for name in ('recv0', 'recv1', 'T0', 'T1'):
@@ -175,6 +189,9 @@ class PeerShard:
         for name, nbytes in (('S0', world * rpp * 4), ('S1', world * rpp * 4), ('stats0', world * rpp * 8), ('stats1', world * rpp * 8)):
             off[name] = cur
             cur += _align(nbytes)
+        if catalogue_width:                 # recommend_peer: the final item rows of ALL items, (P * rpp, catalogue_width) fp32
+            off['cat'] = cur
+            cur += _align(world * rpp * catalogue_width * 4)
         off['total'] = cur
         return off
 
@@ -316,7 +333,7 @@ def _rows_per_part(nI, world):
     return max(1, (int(nI) + world - 1) // world)
 
 
-def shard_from_full(graph, rank, world, arena, d_max, batch_max=8192):
+def shard_from_full(graph, rank, world, arena, d_max, batch_max=8192, catalogue_width=0):
     """Shard of rank `rank` cut out of the full neighbour index (every rank builds the ~10 ms full index and keeps its slices;
     graphs that do not fit one GPU are built per rank instead: `bench.py --workload graph5`)."""
     from .parallel import RowPartition, _LocalIndex, column_slice_csr, split_rows
@@ -339,50 +356,83 @@ def shard_from_full(graph, rank, world, arena, d_max, batch_max=8192):
     return PeerShard(rank=rank, world=world, nI=nI, nU=N - nI, d_max=d_max, rpp=rpp, users_r0=users.r0, users_rows=users.rows,
                      index_users=index_users, index_items=index_items, dinv_users=dinv_users, dinv_items_all=dinv_items,
                      item_features_own=graph.item_features[i0: min(i0 + rpp, nI)], user_features_own=graph.user_features[users.r0:users.r1],
-                     arena=arena, batch_max=batch_max, edges_total=full.e1 + full.e2, edges_own=int(index_users.col.numel() + lcol.numel()))
+                     arena=arena, batch_max=batch_max, edges_total=full.e1 + full.e2, edges_own=int(index_users.col.numel() + lcol.numel()),
+                     catalogue_width=catalogue_width)
 
 
-def partition_graph_peer(graph, group=None, d_max=128, batch_max=8192):
-    """One process per GPU: allocates + exchanges the arenas and cuts this rank's shard.  `d_max` = largest node_emb served."""
+def partition_graph_peer(graph, group=None, d_max=128, batch_max=8192, catalogue_width=0):
+    """One process per GPU: allocates + exchanges the arenas and cuts this rank's shard.  `d_max` = largest node_emb served;
+    `catalogue_width` = floats per item row of the catalogue section that `recommend_peer` needs (`catalogue_width(model)`; 0 = none)."""
     import torch.distributed as dist
     world = dist.get_world_size(group)
     nI = int(graph.item_features.shape[0])
-    nbytes = PeerShard.layout(world, _rows_per_part(nI, world), d_max, batch_max)['total']
+    nbytes = PeerShard.layout(world, _rows_per_part(nI, world), d_max, batch_max, catalogue_width)['total']
     arena = PeerArena.ipc(nbytes, group, device=graph.item_features.device)
-    return shard_from_full(graph, dist.get_rank(group), world, arena, d_max, batch_max)
+    return shard_from_full(graph, dist.get_rank(group), world, arena, d_max, batch_max, catalogue_width)
 
 
-def emulated_shards(graph, world, d_max=128, batch_max=8192):
-    """all P shards in ONE process (single-GPU tests of the exchange logic; run with `forward_emulated`)"""
+def emulated_shards(graph, world, d_max=128, batch_max=8192, catalogue_width=0):
+    """all P shards in ONE process (single-GPU tests of the exchange logic; run with `forward_emulated` / `recommend_emulated`)"""
     nI = int(graph.item_features.shape[0])
-    nbytes = PeerShard.layout(world, _rows_per_part(nI, world), d_max, batch_max)['total']
+    nbytes = PeerShard.layout(world, _rows_per_part(nI, world), d_max, batch_max, catalogue_width)['total']
     arenas = PeerArena.emulated(nbytes, world, graph.item_features.device)
-    return [shard_from_full(graph, q, world, arenas[q], d_max, batch_max) for q in range(world)]
+    return [shard_from_full(graph, q, world, arenas[q], d_max, batch_max, catalogue_width) for q in range(world)]
 
 
 # ----------------------------------------------------------------------------------------------------------------------
+def _widths(model, sh: PeerShard):
+    """(node_emb d, width of a combined row) after the checks every partitioned call makes"""
+    if torch.is_grad_enabled() and any(p.requires_grad for p in model.parameters()):
+        raise NotImplementedError('partitioned GraphNCF propagation is inference-only; wrap the call in torch.no_grad()')
+    d = model.item_embeddings[0].weight.shape[0]
+    if d > sh.d_max or d % 4:
+        raise ValueError(f'node_emb {d} does not fit the arena of this partition (d_max {sh.d_max}) or is not a multiple of 4')
+    return d, (d * (len(model.gnn_convs) + 1) if model.concat else d)             # combined embedding [x0 | ... | xL] or their mean
+
+
 def _steps(model, sh: PeerShard, userIds, itemIds, keep=None):
     """Generator: GraphNCF.forward on shard `sh` (inference).  It yields right before every cross-rank wait, so that an emulation can
     advance all ranks in lock step; a real rank just runs it to the end.  Returns the (B, 1) scores."""
     from .neural_collaborative_filtering.util import run_mlp
-    if torch.is_grad_enabled() and any(p.requires_grad for p in model.parameters()):
-        raise NotImplementedError('partitioned GraphNCF propagation is inference-only; wrap the call in torch.no_grad()')
-    dev = sh.device
-    L_ = len(model.gnn_convs)
-    d = model.item_embeddings[0].weight.shape[0]
-    if d > sh.d_max or d % 4:
-        raise ValueError(f'node_emb {d} does not fit the arena of this partition (d_max {sh.d_max}) or is not a multiple of 4')
+    d, width = _widths(model, sh)
     B = int(userIds.shape[0])
     if 2 * B > 2 * sh.batch_max:
         raise ValueError(f'batch of {B} pairs exceeds the partition\'s batch_max {sh.batch_max}')
-    concat, gat = model.concat, model.convType == 'LightGAT'
-    width = d * (L_ + 1) if concat else d                                           # combined embedding [x0 | ... | xL] or their mean
     if B * width > sh.batch_max * sh.d_max:
         raise ValueError(f'batch of {B} pairs of {width}-wide concatenated rows exceeds the partition\'s rows buffer (batch_max {sh.batch_max} '
                          f'x d_max {sh.d_max} floats per side)')
-    ie, ue = model.item_embeddings[0], model.user_embeddings[0]
     nu, ni = sh.users_rows, sh.it_rows
     iid, uid = itemIds.long().contiguous(), userIds.long().contiguous()
+    acc_items, acc_users = yield from _propagate(model, sh, d, width)
+    if keep is not None:                        # tests: the owned rows of the combined embedding
+        keep['items'], keep['users'] = acc_items, acc_users
+    sh.gather_rows(acc_items, sh.it_r0, ni, iid, 0, width)
+    sh.gather_rows(acc_users, sh.nI + sh.users_r0, nu, uid, B, width)
+    sh.signal(CH_R)
+    yield
+    sh.wait(CH_R)
+    sh.stamp('batch rows arrived')
+    rows = sh.rows_view(2 * B, width)
+    if model.MLP is None:
+        out = ops.rowdot(rows[B:], rows[:B])
+    else:
+        out = run_mlp(model.MLP, rows[:B], rows[B:], training=False)               # item first (gnn_ncf.py:361)
+    sh.stamp('end')
+    if len(model.gnn_convs) == 0:               # no layer barrier protected `rows` against the next call's writers
+        sh.signal(CH_E)
+        yield
+        sh.wait(CH_E)
+    return out
+
+
+def _propagate(model, sh: PeerShard, d, width):
+    """Generator (part of `_steps` / `_recommend_steps`, same yields): the L layers on shard `sh`.  Returns the owned rows of the combined
+    embedding, (items (it_rows, width), users (users_rows, width)): the running mean, or comb = [x0 | ... | xL] with concat."""
+    dev = sh.device
+    L_ = len(model.gnn_convs)
+    concat, gat = model.concat, model.convType == 'LightGAT'
+    ie, ue = model.item_embeddings[0], model.user_embeddings[0]
+    nu, ni = sh.users_rows, sh.it_rows
     empty = lambda n: torch.empty((n, d), dtype=torch.float32, device=dev)
     sh._trace_reset = True
     sh.stamp('start')
@@ -497,25 +547,7 @@ def _steps(model, sh: PeerShard, userIds, itemIds, keep=None):
         sh.stamp('layers joined')
     if concat:
         acc_items, acc_users = comb_items, comb_users
-    if keep is not None:                        # tests: the owned rows of the combined embedding
-        keep['items'], keep['users'] = acc_items, acc_users
-    sh.gather_rows(acc_items, sh.it_r0, ni, iid, 0, width)
-    sh.gather_rows(acc_users, sh.nI + sh.users_r0, nu, uid, B, width)
-    sh.signal(CH_R)
-    yield
-    sh.wait(CH_R)
-    sh.stamp('batch rows arrived')
-    rows = sh.rows_view(2 * B, width)
-    if model.MLP is None:
-        out = ops.rowdot(rows[B:], rows[:B])
-    else:
-        out = run_mlp(model.MLP, rows[:B], rows[B:], training=False)               # item first (gnn_ncf.py:361)
-    sh.stamp('end')
-    if L_ == 0:                                 # no layer barrier protected `rows` against the next call's writers
-        sh.signal(CH_E)
-        yield
-        sh.wait(CH_E)
-    return out
+    return acc_items, acc_users
 
 
 def _layer0_composites(model, ie, ue, lin_i, lin_u, att_i=None, att_u=None):
@@ -555,6 +587,165 @@ def forward_emulated(model, shards, userIds, itemIds, keep=None):
     """all ranks of `emulated_shards` in lock step on one stream; returns the list of per-rank outputs"""
     keep = keep if keep is not None else [None] * len(shards)
     gens = [_steps(model, sh, userIds, itemIds, keep[q]) for q, sh in enumerate(shards)]
+    outs = [None] * len(shards)
+    live = list(range(len(shards)))
+    while live:
+        for q in list(live):
+            try:
+                next(gens[q])
+            except StopIteration as stop:
+                outs[q] = stop.value
+                live.remove(q)
+    return outs
+
+
+# ----------------------------------------------------------------------------------------------------------------------
+# whole-catalogue top-k on the partitioned graph
+# ----------------------------------------------------------------------------------------------------------------------
+def _dot_width(width):
+    return max(64, (int(width) + 63) // 64 * 64)
+
+
+def catalogue_width(model):
+    """Floats per item row of the catalogue section (`catalogue_width=` of the partition builders) that `recommend_peer` needs for `model`:
+    the combined width (L+1)·d with concat, else d; for a dot-product model padded to a multiple of 64, the operand width of the dot kernel."""
+    d = model.item_embeddings[0].weight.shape[0]
+    width = d * (len(model.gnn_convs) + 1) if model.concat else d
+    return _dot_width(width) if model.MLP is None else width
+
+
+def served_rows(users, nI, users_r0, users_rows):
+    """(node ids int64, local rows int64) of the entries of `users` (global user NODE ids) that fall in the range [nI + users_r0,
+    nI + users_r0 + users_rows) of a rank, in request order"""
+    users = users.long()
+    local = users - (nI + users_r0)
+    mine = (local >= 0) & (local < users_rows)
+    return users[mine], local[mine]
+
+
+def seen_csr(row_ptr, col, rows, n_items):
+    """CSR (ptr int32 (n+1), idx int32 ascending per row) of the sources of `rows` of a CSR whose sources are item ids < `n_items`: the
+    `ignore_seen` sets of a shard's users (rows of `index_users`; neighbour rows are in interaction order, so they are sorted here).
+    The sort key is row · n_items + item.  (GraphIndex.seen_items multiplies by `num_nodes`, which on a shard's local user index is the
+    number of OWNED users: item ids can exceed it, and then the keys of neighbouring rows overlap.)"""
+    rows = rows.long()
+    dev = rows.device
+    start, end = row_ptr[rows].long(), row_ptr[rows + 1].long()
+    cnt = end - start
+    ptr = torch.zeros(rows.numel() + 1, dtype=torch.int64, device=dev)
+    ptr[1:] = torch.cumsum(cnt, 0)
+    total = int(ptr[-1])
+    r = torch.repeat_interleave(torch.arange(rows.numel(), device=dev), cnt)
+    within = torch.arange(total, device=dev) - ptr[:-1][r]
+    key = torch.sort(r * int(n_items) + col[start[r] + within].long()).values
+    return ptr.int(), (key - r * int(n_items)).int()
+
+
+def _recommend_steps(model, sh: PeerShard, k=10, users=None, precision='fp32', ignore_seen=True, return_scores=False, chunk_users=None):
+    """Generator (yields like `_steps`): `recommend_peer` on shard `sh`."""
+    from .neural_collaborative_filtering.util import mlp_parameters
+    if model.training:
+        raise NotImplementedError('recommend_peer is an inference call: model.eval() first')
+    d, width = _widths(model, sh)
+    if precision not in ('fp32', 'bf16'):
+        raise ValueError("precision must be 'fp32' or 'bf16'")
+    if not 1 <= int(k) <= 64:
+        raise ValueError(f'k = {k}: the all-pairs kernels keep 1 to 64 items per user')
+    dot = model.MLP is None
+    if dot and width > 256:
+        raise NotImplementedError(f'dot-product scoring of {width}-wide combined rows: the all-pairs dot kernel takes at most 256 floats per row')
+    if not dot:                                    # the all-pairs limits, checked before any rank signals
+        weights, biases, _ = mlp_parameters(model.MLP)
+        if len(weights) not in (2, 3) or weights[0].shape[0] > 256 or (len(weights) == 3 and weights[1].shape[0] > 128):
+            raise NotImplementedError('all-pairs scoring supports MLPs of 1 or 2 hidden layers, the first at most 256 and the second at most 128 wide')
+    cw = catalogue_width(model)
+    if sh.catalogue_width < cw:
+        raise ValueError(f'recommend_peer needs a catalogue section of {cw} floats per item row; this partition has {sh.catalogue_width} '
+                         f'(build it with catalogue_width={cw})')
+    dev, nI = sh.device, sh.nI
+    if users is None:
+        nodes = torch.arange(nI + sh.users_r0, nI + sh.users_r0 + sh.users_rows, device=dev)
+        local = None
+    else:
+        nodes, local = served_rows(users.to(dev), nI, sh.users_r0, sh.users_rows)
+    n = int(nodes.numel())
+    seen = None
+    if ignore_seen:
+        rp, col = sh.index_users.row_ptr, sh.index_users.col
+        if local is None:
+            seen = sh._seen.get((rp, col), lambda: seen_csr(rp, col, torch.arange(sh.users_rows, device=dev), nI))
+        else:
+            seen = seen_csr(rp, col, local, nI)
+        if seen[1].numel() == 0:                   # nobody has seen anything (an empty idx array would reach the kernels as NULL)
+            seen = None
+
+    acc_items, acc_users = yield from _propagate(model, sh, d, width)
+
+    # the final item rows of every owner -> the catalogue section of every rank (itself included), rows it_r0 ..
+    cat = sh.arena.view(sh.off['cat'], (sh.table_rows, cw))
+    if cw > width:                                 # the dot kernel's zero padding: only this rank writes these columns
+        cat[:, width:].zero_()
+    if sh.it_rows:
+        with torch.cuda.device(dev):
+            L.check(L.lib().b200rec_peer_push_rows(_ptr(acc_items), acc_items.stride(0), sh.it_rows, width, sh.arena.ptrs(sh.off['cat']), sh.world,
+                                                   sh.it_r0 * cw, cw, _stream()), 'peer_push_rows')
+    sh.signal(CH_C)
+    sh.stamp('catalogue pushed')
+    yield
+    sh.wait(CH_C)
+    sh.stamp('catalogue arrived')
+
+    items = cat[:nI]
+    val = torch.full((n, k), float('-inf'), dtype=torch.float32, device=dev)
+    idx = torch.full((n, k), -1, dtype=torch.int64, device=dev)
+    scores = torch.empty((n, nI), dtype=torch.float32, device=dev) if return_scores else None
+    step = n if not chunk_users else int(chunk_users)
+    for s in range(0, n, max(step, 1)):
+        e = min(s + step, n)
+        rows = acc_users[s:e] if local is None else acc_users[local[s:e]]
+        sc = None if seen is None else (seen[0][s:e + 1], seen[1])     # absolute offsets into the shard's idx array
+        if dot:
+            v, i, sc_out = ops.allpairs_dot_topk_raw(rows if cw == width else torch.nn.functional.pad(rows, (0, cw - width)), items, k,
+                                                     return_scores=return_scores, seen=sc)
+        else:
+            v, i, sc_out = ops.mlp_allpairs_topk(rows, items, weights, biases, k, rows_first=False, precision=precision, seen=sc,
+                                                 return_scores=return_scores)
+        val[s:e], idx[s:e] = v, i
+        if return_scores:
+            scores[s:e] = sc_out
+    sh.stamp('scored')
+
+    # closing barrier: the next call's catalogue push must not overwrite a table a slower rank still scores from
+    sh.signal(CH_D)
+    yield
+    sh.wait(CH_D)
+    return (nodes, val, idx, scores) if return_scores else (nodes, val, idx)
+
+
+def recommend_peer(model, sh: PeerShard, k=10, users=None, precision='fp32', ignore_seen=True, return_scores=False, chunk_users=None):
+    """Top-k items over the WHOLE catalogue for the users this rank owns — `GraphNCF.recommend` on a partitioned graph.  Every rank of the
+    group calls it (with the same arguments); the propagation runs again on every call.
+
+    users          global user NODE ids (nI .. N-1) or None = every owned user.  A rank serves the ids of its range, in request order.
+    precision      'fp32' / 'bf16' as in GraphNCF.recommend (two-hidden-layer MLPs: the tensor-core operand split; the exact kernels of
+                   one-hidden-layer MLPs and of dot-product models ignore it).
+    ignore_seen    leave out the items a user is connected to in the graph.
+    chunk_users    score at most this many users per kernel call (bounds the per-user tables and workspace on large shards).
+
+    Returns (user_nodes int64 (n,), val (n, k) fp32, idx (n, k) int64 item node ids[, scores (n, nI)]), rows padded with (-inf, -1).  Nothing
+    is gathered across ranks: the union of the ranks' `user_nodes` is the request.  The partition needs a catalogue section of
+    `catalogue_width(model)` floats per item row (ValueError otherwise)."""
+    gen = _recommend_steps(model, sh, k, users, precision, ignore_seen, return_scores, chunk_users)
+    try:
+        while True:
+            next(gen)
+    except StopIteration as stop:
+        return stop.value
+
+
+def recommend_emulated(model, shards, **kw):
+    """`recommend_peer` on all ranks of `emulated_shards` in lock step on one stream; returns the list of per-rank results"""
+    gens = [_recommend_steps(model, sh, **kw) for sh in shards]
     outs = [None] * len(shards)
     live = list(range(len(shards)))
     while live:

@@ -58,7 +58,7 @@ def create_graph_local(u_local, items, ratings, n_local_users, nI, item_features
                      user2item_edge_attr=attr_u, item2user_edge_attr=attr_i)
 
 
-def shard_from_local(graph_local, *, rank, world, nI, nU, users_r0, arena, d_max, batch_max, reduce_items=None, edges_total=None):
+def shard_from_local(graph_local, *, rank, world, nI, nU, users_r0, arena, d_max, batch_max, reduce_items=None, edges_total=None, catalogue_width=0):
     """PeerShard of a rank from the graph of its own interactions (`create_graph_local`)."""
     from .parallel import _LocalIndex
     from .peer import PeerShard, _rows_per_part
@@ -86,12 +86,14 @@ def shard_from_local(graph_local, *, rank, world, nI, nU, users_r0, arena, d_max
     return PeerShard(rank=rank, world=world, nI=nI, nU=nU, d_max=d_max, rpp=rpp, users_r0=users_r0, users_rows=n_local, index_users=index_users,
                      index_items=index_items, dinv_users=dinv_users, dinv_items_all=dinv_items,
                      item_features_own=graph_local.item_features[i0: min(i0 + rpp, nI)], user_features_own=graph_local.user_features,
-                     arena=arena, batch_max=batch_max, edges_total=own if edges_total is None else edges_total, edges_own=own)
+                     arena=arena, batch_max=batch_max, edges_total=own if edges_total is None else edges_total, edges_own=own,
+                     catalogue_width=catalogue_width)
 
 
 def build_shard(u_local, items, ratings, *, nI, nU, users_r0, n_local_users, item_features, user_features_local, group=None, d_max=64,
-                batch_max=8192, edges_total=None):
-    """One process per GPU: the PeerShard of this rank from its own interactions + the arena exchange (collectives at build time only)."""
+                batch_max=8192, edges_total=None, catalogue_width=0):
+    """One process per GPU: the PeerShard of this rank from its own interactions + the arena exchange (collectives at build time only).
+    `catalogue_width` > 0 adds the catalogue section of `peer.recommend_peer`."""
     import torch.distributed as dist
     from .peer import PeerArena, PeerShard, _rows_per_part
     world, rank = dist.get_world_size(group), dist.get_rank(group)
@@ -100,7 +102,7 @@ def build_shard(u_local, items, ratings, *, nI, nU, users_r0, n_local_users, ite
         dist.all_reduce(t, group=group)
 
     g = create_graph_local(u_local, items, ratings, n_local_users, nI, item_features, user_features_local, reduce_items if world > 1 else None)
-    nbytes = PeerShard.layout(world, _rows_per_part(nI, world), d_max, batch_max)['total']
+    nbytes = PeerShard.layout(world, _rows_per_part(nI, world), d_max, batch_max, catalogue_width)['total']
     arena = PeerArena.ipc(nbytes, group, device=u_local.device)
     return shard_from_local(g, rank=rank, world=world, nI=nI, nU=nU, users_r0=users_r0, arena=arena, d_max=d_max, batch_max=batch_max,
-                            reduce_items=reduce_items if world > 1 else None, edges_total=edges_total)
+                            reduce_items=reduce_items if world > 1 else None, edges_total=edges_total, catalogue_width=catalogue_width)

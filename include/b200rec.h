@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define B200REC_VERSION 207
+#define B200REC_VERSION 208
 
 typedef void* b200rec_stream_t; /* cudaStream_t */
 
@@ -154,6 +154,13 @@ int b200rec_allpairs_relu_dot_splits(int64_t nU, int64_t nI);
 int b200rec_allpairs_relu_dot_topk(const float* A, const float* B, int64_t nU, int64_t nI, int H1, const float* w2, float b2, int k, int n_splits,
                                    const int* seen_ptr, const int* seen_idx, float* scores, int64_t lds, float* top_val, int64_t* top_idx,
                                    void* workspace, size_t workspace_bytes, b200rec_stream_t stream);
+/* Dot-product models in all-pairs mode: score(u,i) = sum_h A[u,h]·B[i,h], the same kernel's exact FP32 form (one FFMA per h and pair), with
+ * the same tiling, top-k / `seen` / split-list semantics and workspace query; b200rec_allpairs_relu_dot_splits gives its automatic split
+ * count.  The (nU, nI) scores are never materialised unless `scores` is given.  A (nU, H), B (nI, H) contiguous fp32, H in {64,128,192,256}
+ * (zero-pad). */
+int b200rec_allpairs_dot_topk(const float* A, const float* B, int64_t nU, int64_t nI, int H, int k, int n_splits, const int* seen_ptr,
+                              const int* seen_idx, float* scores, int64_t lds, float* top_val, int64_t* top_idx, void* workspace,
+                              size_t workspace_bytes, b200rec_stream_t stream);
 int b200rec_topk_rows(const float* scores, int64_t rows, int64_t cols, int64_t ld, int k, float* out_val, int64_t* out_idx,
                       b200rec_stream_t stream);
 
