@@ -12,7 +12,7 @@ OK, ERR_CUDA, ERR_BAD_ARG, ERR_UNSUPPORTED, ERR_WORKSPACE = 0, 1, 2, 3, 4
 F32, BF16 = 0, 1
 ATT_NET, ATT_DOT = 0, 1
 TC_TF32X3, TC_BF16, TC_BF16X3 = 0, 1, 2
-ABI_VERSION = 208          # B200REC_VERSION of include/b200rec.h these bindings were written against (checked when the library is loaded)
+ABI_VERSION = 209          # B200REC_VERSION of include/b200rec.h these bindings were written against (checked when the library is loaded)
 AP_BF16, AP_BF16X2 = 0, 1
 MLP_MAX_LAYERS = 8
 PEER_MAX, PEER_CHANNELS, PEER_HANDLE_BYTES = 16, 16, 64
@@ -149,6 +149,9 @@ SIGNATURES = {
     'b200rec_peer_push_floats': (c_int, [c_vp, c_i64, C.POINTER(c_vp), c_int, c_i64, c_vp]),
     'b200rec_peer_push_rows': (c_int, [c_vp, c_i64, c_i64, c_int, C.POINTER(c_vp), c_int, c_i64, c_i64, c_vp]),
     'b200rec_device_timestamp': (c_int, [c_vp, c_vp]),
+    'b200rec_peer_scale_rows': (c_int, [c_vp, c_i64, c_i64, c_int, c_vp, c_i64, c_vp, c_f, c_vp, c_i64, c_vp, c_i64, c_vp]),
+    'b200rec_peer_rows_to_owned': (c_int, [c_vp, c_i64, c_vp, c_vp, c_i64, c_i64, c_i64, c_int, c_f, c_vp, c_i64, c_vp]),
+    'b200rec_peer_mask_targets': (c_int, [c_vp, c_vp, c_i64, c_vp, c_i64, c_i64, c_i64, c_i64, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     'b200rec_peer_gather_rows': (c_int, [c_vp, c_i64, c_i64, c_i64, c_vp, c_i64, c_int, c_f, C.POINTER(c_vp), c_int, c_i64, c_i64, c_vp]),
 }
 

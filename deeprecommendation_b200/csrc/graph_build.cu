@@ -436,6 +436,37 @@ __global__ void mask_targets_kernel(const int64_t* __restrict__ positions, long 
   }
 }
 
+// partitioned training (peer.py): the batch targets on one rank.  Entry i counts when first[i] == i (the first entry of its pair in the
+// batch; GraphIndex.masked takes each position once).  Every rank takes one off the degree of item iid[i]; the rank that owns user uid[i]
+// (node0 <= uid < node0 + rows) finds the pair in its local hash (vals = CSR entry, local_pos = the entry's interaction position), sets
+// that position's skip bit and takes one off the user's degree.  Ids outside the graph and pairs the owner does not find are counted in
+// *n_missing.
+__global__ void peer_mask_targets_kernel(const int64_t* __restrict__ uid, const int64_t* __restrict__ iid, long long n, const int64_t* __restrict__ first,
+                                         long long n_items, long long n_nodes, long long node0, long long rows,
+                                         const unsigned long long* __restrict__ keys, const int* __restrict__ vals, unsigned long long cap_mask,
+                                         const int* __restrict__ local_pos, unsigned* __restrict__ skip_bits, int* __restrict__ deg_users,
+                                         int* __restrict__ deg_items, int* __restrict__ n_missing) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int64_t u = uid[i], it = iid[i];
+  if (u < n_items || u >= n_nodes || it < 0 || it >= n_items) { atomicAdd(n_missing, 1); return; }
+  if (first[i] != i) return;
+  atomicSub(deg_items + it, 1);
+  const long long lu = u - node0;
+  if (lu < 0 || lu >= rows) return;
+  const unsigned long long key = ((unsigned long long)u << 32) | (unsigned long long)(it & 0xffffffffLL);
+  unsigned long long h = mix64(key) & cap_mask;
+  while (true) {
+    const unsigned long long k = keys[h];
+    if (k == key) break;
+    if (k == HASH_EMPTY) { atomicAdd(n_missing, 1); return; }
+    h = (h + 1) & cap_mask;
+  }
+  const int p = local_pos[vals[h]];
+  atomicOr(skip_bits + (p >> 5), 1u << (p & 31));
+  atomicSub(deg_users + lu, 1);
+}
+
 }  // namespace b200rec
 
 using namespace b200rec;
@@ -629,6 +660,20 @@ extern "C" int b200rec_mask_targets(const int64_t* positions, int64_t n, int64_t
   if (n < 0 || n_edges < 0 || !skip_bits || !deg || !u2i || !i2u) return b200rec_fail(B200REC_ERR_BAD_ARG, "mask_targets: bad argument");
   if (n == 0) return B200REC_OK;
   mask_targets_kernel<<<grid1d(n), 256, 0, (cudaStream_t)stream>>>(positions, n, n_edges, u2i, i2u, skip_bits, deg);
+  B200REC_CHECK_LAUNCH();
+  return B200REC_OK;
+}
+
+extern "C" int b200rec_peer_mask_targets(const int64_t* uid, const int64_t* iid, int64_t n, const int64_t* first, int64_t n_items, int64_t n_nodes,
+                                         int64_t node0, int64_t rows, const uint64_t* keys, const int* vals, int64_t capacity, const int* local_pos,
+                                         uint32_t* skip_bits, int* deg_users, int* deg_items, int* n_missing, b200rec_stream_t stream) {
+  if (n < 0 || !skip_bits || !deg_items || !n_missing || (n > 0 && (!uid || !iid || !first)) ||
+      (rows > 0 && (!keys || !vals || !local_pos || !deg_users || capacity <= 0 || (capacity & (capacity - 1)))))
+    return b200rec_fail(B200REC_ERR_BAD_ARG, "peer_mask_targets: bad argument");
+  if (n == 0) return B200REC_OK;
+  peer_mask_targets_kernel<<<grid1d(n), 256, 0, (cudaStream_t)stream>>>(uid, iid, n, first, n_items, n_nodes, node0, rows, (const unsigned long long*)keys,
+                                                                       vals, (unsigned long long)capacity - 1, local_pos, skip_bits, deg_users, deg_items,
+                                                                       n_missing);
   B200REC_CHECK_LAUNCH();
   return B200REC_OK;
 }

@@ -16,6 +16,9 @@
 //     flag word after the producing kernel, an acquire spin (bounded by a timeout that raises an error flag instead of hanging
 //     the GPU) before the consuming kernel.  Epochs are counted on the device, so a captured CUDA graph can be replayed.
 //   * peer_gather_rows_kernel pushes the batch rows a rank owns into every rank's (2B, d) buffer (replaces an all-reduce).
+//   * training (peer.py): peer_rows_to_owned_kernel sums the batch rows' gradient onto the owned rows in batch order and
+//     peer_scale_rows_kernel applies dropout multipliers / degree scaling and accumulates partial gradients; the backward's exchanges
+//     are the forward's kernels on the reverse-edge weights.
 #include <math.h>
 #include <stdio.h>
 #include <string.h>
@@ -185,6 +188,51 @@ __global__ void __launch_bounds__(256) peer_gather_rows_kernel(const float* __re
   }
 }
 
+// training (peer.py, _train_backward): out = scale · x ∘ mask ∘ row_scale[r] (+ add) elementwise over a (rows, d) block; mask / row_scale /
+// add may be null.  The conv-dropout multipliers, the degree scaling of a gradient and the accumulation of partial gradients.  out may alias
+// x or add.
+__global__ void __launch_bounds__(256) peer_scale_rows_kernel(const float* x, long long ld_x, int rows, int d4, const float* mask, long long ld_m,
+                                                              const float* row_scale, float scale, const float* add, long long ld_add, float* out,
+                                                              long long ld_out) {
+  const long long total = (long long)rows * d4;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const int r = (int)(i / d4), c = (int)(i - (long long)r * d4) * 4;
+    float4 v = *reinterpret_cast<const float4*>(x + (long long)r * ld_x + c);
+    if (mask) {
+      const float4 m = *reinterpret_cast<const float4*>(mask + (long long)r * ld_m + c);
+      v = make_float4(v.x * m.x, v.y * m.y, v.z * m.z, v.w * m.w);
+    }
+    const float s = row_scale ? scale * row_scale[r] : scale;
+    v = make_float4(v.x * s, v.y * s, v.z * s, v.w * s);
+    if (add) {
+      const float4 a = *reinterpret_cast<const float4*>(add + (long long)r * ld_add + c);
+      v = make_float4(v.x + a.x, v.y + a.y, v.z + a.z, v.w + a.w);
+    }
+    *reinterpret_cast<float4*>(out + (long long)r * ld_out + c) = v;
+  }
+}
+
+// training: the gradient of the batch rows onto the owned rows they were gathered from, without atomics.  sorted / perm = the batch ids
+// sorted stably and their batch positions, so that the entries of one id are adjacent and in batch order.  One warp per sorted entry; the
+// first entry of an id this rank owns (row0 <= id < row0 + rows) writes out[id - row0] = scale · Σ g[j] over that id's entries, in batch
+// order.  Rows no entry names are not written.
+__global__ void __launch_bounds__(256) peer_rows_to_owned_kernel(const float* __restrict__ g, long long ld_g, const long long* __restrict__ sorted,
+                                                                 const long long* __restrict__ perm, int n, long long row0, long long rows, int d4,
+                                                                 float scale, float* __restrict__ out, long long ld_out) {
+  const int w = (int)(((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+  if (w >= n) return;
+  const long long id = sorted[w], local = id - row0;
+  if (local < 0 || local >= rows || (w > 0 && sorted[w - 1] == id)) return;
+  for (int c4 = lane; c4 < d4; c4 += 32) {
+    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+    for (int s = w; s < n && sorted[s] == id; ++s) {
+      const float4 v = *reinterpret_cast<const float4*>(g + perm[s] * ld_g + 4 * c4);
+      acc = make_float4(acc.x + v.x, acc.y + v.y, acc.z + v.z, acc.w + v.w);
+    }
+    *reinterpret_cast<float4*>(out + local * ld_out + 4 * c4) = make_float4(acc.x * scale, acc.y * scale, acc.z * scale, acc.w * scale);
+  }
+}
+
 // device-side tracing: one thread writes %globaltimer (ns) — a marker between the kernels of a captured forward, so that the phases of a
 // rank (and the time it spends waiting for its peers) can be read back after a CUDA-graph replay
 __global__ void device_timestamp_kernel(unsigned long long* slot) { *slot = globaltimer_ns(); }
@@ -325,6 +373,33 @@ extern "C" int b200rec_peer_gather_rows(const float* table, int64_t ld, int64_t 
   const int grid = (int)((n_ids * 32 + 255) / 256);
   peer_gather_rows_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(table, ld, row0, rows, reinterpret_cast<const long long*>(ids), (int)n_ids, d / 4,
                                                                   scale, pp, n_dst, dst_offset, ld_dst);
+  B200REC_CHECK_LAUNCH();
+  return B200REC_OK;
+}
+
+extern "C" int b200rec_peer_scale_rows(const float* x, int64_t ld_x, int64_t rows, int d, const float* mask, int64_t ld_m, const float* row_scale,
+                                       float scale, const float* add, int64_t ld_add, float* out, int64_t ld_out, b200rec_stream_t stream) {
+  if (rows == 0) return B200REC_OK;
+  auto a16 = [](const void* p) { return ((uintptr_t)p % 16) == 0; };
+  if (!x || !out || rows < 0 || rows > INT32_MAX || d <= 0 || (d % 4) || (ld_x % 4) || (ld_out % 4) || !a16(x) || !a16(out) ||
+      (mask && (!a16(mask) || (ld_m % 4))) || (add && (!a16(add) || (ld_add % 4))))
+    return b200rec_fail(B200REC_ERR_BAD_ARG, "peer_scale_rows: operands must allow 128-bit access (d, leading dims multiples of 4)");
+  const long long total = rows * (long long)(d / 4);
+  const int grid = (int)std::min<long long>((total + 255) / 256, (long long)b200rec_num_sms() * 8);
+  peer_scale_rows_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(x, ld_x, (int)rows, d / 4, mask, ld_m, row_scale, scale, add, ld_add, out, ld_out);
+  B200REC_CHECK_LAUNCH();
+  return B200REC_OK;
+}
+
+extern "C" int b200rec_peer_rows_to_owned(const float* g, int64_t ld_g, const int64_t* sorted, const int64_t* perm, int64_t n, int64_t row0,
+                                          int64_t rows, int d, float scale, float* out, int64_t ld_out, b200rec_stream_t stream) {
+  if (n == 0 || rows == 0) return B200REC_OK;
+  if (!g || !sorted || !perm || !out || n < 0 || n > INT32_MAX / 32 || rows < 0 || d <= 0 || (d % 4) || (ld_g % 4) || (ld_out % 4) ||
+      ((uintptr_t)g % 16) || ((uintptr_t)out % 16))
+    return b200rec_fail(B200REC_ERR_BAD_ARG, "peer_rows_to_owned: operands must allow 128-bit access");
+  const int grid = (int)((n * 32 + 255) / 256);
+  peer_rows_to_owned_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(g, ld_g, reinterpret_cast<const long long*>(sorted),
+                                                                    reinterpret_cast<const long long*>(perm), (int)n, row0, rows, d / 4, scale, out, ld_out);
   B200REC_CHECK_LAUNCH();
   return B200REC_OK;
 }

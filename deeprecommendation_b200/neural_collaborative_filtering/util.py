@@ -29,10 +29,11 @@ def mlp_parameters(mlp: nn.Sequential):
     return [m.weight for m in lin], [m.bias for m in lin], (drops[0] if drops else 0.0)
 
 
-def run_mlp(mlp: nn.Sequential, in0, in1, idx0=None, idx1=None, training=False):
+def run_mlp(mlp: nn.Sequential, in0, in1, idx0=None, idx1=None, training=False, generator=None):
     """MLP([in0[idx0], in1[idx1]]) -> (B, 1).  Eval (or inert dropout): one fused kernel, activations stay in shared
     memory.  Training with dropout p > 0: layer-by-layer through the CUDA linear kernel with torch's Bernoulli mask in
-    between (the reference's Philox stream cannot be bit-matched anyway, SURVEY.md §7.3)."""
+    between (the reference's Philox stream cannot be bit-matched anyway, SURVEY.md §7.3).  `generator`: draw the masks from
+    it instead of torch's default generator (partitioned training: the same masks on every rank)."""
     weights, biases, p = mlp_parameters(mlp)
     if not (training and p > 0.0):
         return ops.mlp_tower(in0, in1, weights, biases, idx0, idx1)
@@ -42,7 +43,10 @@ def run_mlp(mlp: nn.Sequential, in0, in1, idx0=None, idx1=None, training=False):
     for n, (w, b) in enumerate(zip(weights, biases)):
         x = ops.linear(x, w, b, relu=n < last)
         if n < last:
-            x = torch.nn.functional.dropout(x, p, training=True)
+            if generator is None:
+                x = torch.nn.functional.dropout(x, p, training=True)
+            else:
+                x = x * torch.empty_like(x).bernoulli_(1.0 - p, generator=generator).div_(1.0 - p)
     return x
 
 

@@ -619,6 +619,36 @@ def rowdot(in0, in1, idx0=None, idx1=None):
     return out
 
 
+def scale_rows_raw(x, *, mask=None, row_scale=None, scale=1.0, add=None, out=None):
+    """out = scale · x ∘ mask ∘ row_scale[:, None] (+ add) on (rows, d) fp32 blocks — b200rec_peer_scale_rows (partitioned training).
+    `out` may be `x` or `add`."""
+    _require_cuda(x, mask, row_scale, add, out)
+    rows, d = x.shape
+    if out is None:
+        out = torch.empty((rows, d), dtype=torch.float32, device=x.device)
+    for t in (x, mask, add, out):
+        if t is not None and (t.shape != (rows, d) or t.dtype != torch.float32 or t.stride(1) != 1):
+            raise ValueError('scale_rows: operands must be (rows, d) fp32 blocks with unit column stride')
+    if row_scale is not None:
+        row_scale = row_scale.contiguous().float()
+    ld = lambda t: (t.stride(0) if rows > 1 else d) if t is not None else 0
+    with _on(x.device):
+        L.check(L.lib().b200rec_peer_scale_rows(_ptr(x), ld(x), rows, d, _ptr(mask), ld(mask), _ptr(row_scale), float(scale), _ptr(add), ld(add),
+                                                _ptr(out), ld(out), _stream()), 'peer_scale_rows')
+    return out
+
+
+def rows_to_owned_raw(g, ids, row0, rows, scale, out):
+    """out[ids[j] - row0] = scale · Σ_j g[j] for the ids in [row0, row0 + rows), duplicates summed in batch order (no atomics) —
+    b200rec_peer_rows_to_owned.  Rows no id names are left as they are."""
+    _require_cuda(g, ids, out)
+    sorted_ids, perm = torch.sort(ids.long(), stable=True)
+    with _on(g.device):
+        L.check(L.lib().b200rec_peer_rows_to_owned(_ptr(g), g.stride(0), _ptr(sorted_ids), _ptr(perm), ids.numel(), int(row0), int(rows), g.shape[1],
+                                                   float(scale), _ptr(out), out.stride(0) if rows > 1 else out.shape[1], _stream()), 'peer_rows_to_owned')
+    return out
+
+
 # ------------------------------------------------------------------------------------------------------------------
 # K2 attention pooling
 # ------------------------------------------------------------------------------------------------------------------

@@ -68,21 +68,39 @@ class RowPartition:
 
 
 class _LocalIndex(GraphIndex):
-    """GraphIndex over a set of owned rows only (no edge lists / hash: inference-side object)."""
+    """GraphIndex over a set of owned rows only (no edge lists).  `w_bwd` = weight of the reverse edge of every entry (the backward of
+    the partitioned training, peer.py); `pair_hash` is built on first use."""
 
-    def __init__(self, row_ptr, col, w, pos, dinv_own, chunk):
+    def __init__(self, row_ptr, col, w, pos, dinv_own, chunk, w_bwd=None):
         self.row_ptr, self.col, self.w, self.pos = row_ptr, col, w, pos
         self.dinv = dinv_own
         self.num_nodes = int(row_ptr.numel() - 1)
         self.e1, self.e2 = int(col.numel()), 0
         self.chunk_size = chunk
-        self.symmetric, self.w_bwd, self._hash = False, None, None
+        self.symmetric, self.w_bwd, self._hash = False, w_bwd, None
         if self.num_nodes == 0:                      # a rank without rows of this type (more ranks than users): no SpMM ever runs on it
             empty = torch.zeros(0, dtype=torch.int32, device=row_ptr.device)
             self.n_chunks = self.n_multi = self.n_slots = 0
             self.chunk_row = self.chunk_start = self.chunk_slot = self.multi_row = self.multi_first_slot = self.multi_n_slots = empty
             return
         self._build_plan()
+
+    def pair_hash(self, node0):
+        """(keys int64, vals int32, capacity) of the pair hash (source row node0 + r, column) -> CSR entry of this index's entries (the
+        `b200rec_pairhash_build` format; a shard's user index: user node -> item).  Identical pairs keep their first entry, which is
+        their first interaction position: a row's entries are in position order.  Built on first use."""
+        if self._hash is None:
+            from . import _lib as L
+            from .ops import _ptr, _stream
+            dev, n = self.row_ptr.device, int(self.col.numel())
+            rows = torch.repeat_interleave(torch.arange(self.num_nodes, device=dev), (self.row_ptr[1:] - self.row_ptr[:-1]).long()) + int(node0)
+            edges = torch.stack((rows, self.col.long()))
+            cap = 1 << max(4, (2 * n - 1).bit_length())
+            keys, vals = torch.empty(cap, dtype=torch.int64, device=dev), torch.empty(cap, dtype=torch.int32, device=dev)
+            with torch.cuda.device(dev):
+                L.check(L.lib().b200rec_pairhash_build(_ptr(edges), n, _ptr(keys), _ptr(vals), cap, _stream()), 'pairhash_build')
+            self._hash = (keys, vals, cap)
+        return self._hash
 
 
 class PartitionedGraph:
@@ -191,18 +209,22 @@ class UserPartitionedGraph:
         return (local >= 0) & (local < self.users.rows), local
 
 
-def partition_graph(graph, group=None, scheme: str = 'peer', d_max: int = 128, batch_max: int = 8192, catalogue_width: int = 0):
+def partition_graph(graph, group=None, scheme: str = 'peer', d_max: int = 128, batch_max: int = 8192, catalogue_width: int = 0,
+                    grad_floats: int = 0):
     """'peer' (default): users partitioned, the exchange written as this library's own kernels over peer-mapped memory (peer.py);
     'reduce' / 'gather': the same partitions with NCCL collectives issued from Python (kept as the comparison baseline).
-    `catalogue_width` (scheme 'peer' only): floats per item row of the catalogue section of `peer.recommend_peer`."""
+    `catalogue_width` (scheme 'peer' only): floats per item row of the catalogue section of `peer.recommend_peer`.
+    `grad_floats` (scheme 'peer' only): floats per rank of the gradient section of partitioned training (`peer.grad_floats(model)`)."""
     if scheme not in ('peer', 'reduce', 'gather'):
         raise ValueError(scheme)
     if catalogue_width and scheme != 'peer':
         raise ValueError("catalogue_width: only scheme 'peer' serves recommend_peer")
+    if grad_floats and scheme != 'peer':
+        raise ValueError("grad_floats: only scheme 'peer' trains on a partitioned graph")
     get_index(graph)                                   # (resets a stale partition of an edited graph)
     if scheme == 'peer':
         from .peer import partition_graph_peer
-        pg = partition_graph_peer(graph, group, d_max=d_max, batch_max=batch_max, catalogue_width=catalogue_width)
+        pg = partition_graph_peer(graph, group, d_max=d_max, batch_max=batch_max, catalogue_width=catalogue_width, grad_floats=grad_floats)
     else:
         pg = UserPartitionedGraph(graph, group) if scheme == 'reduce' else PartitionedGraph(graph, group)
     try:

@@ -41,6 +41,12 @@ without it a fast rank's next push would overwrite rows a slow rank is still sco
 between that could order it.  The propagation sections are ordered exactly as for the forward (a recommend ends with all ranks past D, a
 stronger state than the end of a forward), so forwards and recommends can follow each other in any order on the same epoch counters.
 
+Training (`forward_peer` with grad, `train_emulated`; LightGCN, mean combine): the forward above on one stream with per-shard target masking
+and dropout (`_train_forward`), then a collective backward (`_train_backward`) that runs the same exchanges in reverse on the reverse-edge weights
+`w_bwd` — C' pushes dinv ∘ G of the owned items into T[par] (the all-gather), A' pushes partial item gradients into the owners' recv[par] (the
+reduce-scatter) — and ends with the partial parameter gradients pushed into every rank's `grad` section and summed there in rank order (channel G),
+so every rank gets the same bits.  A missing-pair count crosses channel M before any data moves.  DESIGN.md §7 has the exchange table.
+
 The arenas are cudaMalloc'd by libb200rec and exchanged as CUDA IPC handles through torch.distributed (plumbing).
 `emulated_shards` builds all P shards inside ONE process (plain device buffers, the same kernels and addresses) so that the
 exchange logic is covered by the single-GPU test-suite; there the ranks advance in lock step, segment by segment.
@@ -59,10 +65,12 @@ from .derived import Derived
 from .graph import get_index
 from .ops import _ptr, _stream
 
-CH_T0, CH_T1, CH_A0, CH_A1, CH_R, CH_E, CH_C, CH_D = 0, 1, 2, 3, 4, 5, 6, 7
-_CTRL_BYTES = 4096                 # flags uint32[16][16] (1 KB) | counters uint32[32] | err int32
+CH_T0, CH_T1, CH_A0, CH_A1, CH_R, CH_E, CH_C, CH_D, CH_M, CH_G = 0, 1, 2, 3, 4, 5, 6, 7, 8, 9
+_CTRL_BYTES = 4096                 # flags uint32[16][16] (1 KB) | counters uint32[32] | err int32 | ... | missing int32[16] at 2 KB
 _OFF_COUNTERS = L.PEER_CHANNELS * L.PEER_MAX * 4
 _OFF_ERR = _OFF_COUNTERS + 2 * L.PEER_CHANNELS * 4
+_OFF_MISSING = 2048                # training: slot q = the number of batch pairs rank q could not find among its edges
+MLP_DROPOUT_SEED = 0x5eed          # initial state of every shard's MLP dropout generator (the same on every rank)
 WAIT_TIMEOUT_NS = 10_000_000_000
 TRACE = os.environ.get('B200REC_PEER_TRACE', '0') == '1'
 
@@ -74,6 +82,10 @@ class _Raw:
 
 def _align(n, a=256):
     return (int(n) + a - 1) // a * a
+
+
+def _round4(n):
+    return (int(n) + 3) // 4 * 4
 
 
 class PeerArena:
@@ -155,7 +167,8 @@ class PeerShard:
     """What rank `rank` keeps of a user-partitioned graph + the arena layout (identical on every rank)."""
 
     def __init__(self, *, rank, world, nI, nU, d_max, rpp, users_r0, users_rows, index_users, index_items, dinv_users, dinv_items_all,
-                 item_features_own, user_features_own, arena, batch_max, edges_total, edges_own, catalogue_width=0):
+                 item_features_own, user_features_own, arena, batch_max, edges_total, edges_own, catalogue_width=0, grad_floats=0,
+                 deg_users=None, deg_items_all=None, n_positions=0, symmetric=False):
         self.rank, self.world, self.nI, self.nU, self.rpp = rank, world, int(nI), int(nU), int(rpp)
         self.N = self.nI + self.nU
         self.users_r0, self.users_rows = int(users_r0), int(users_rows)
@@ -168,7 +181,13 @@ class PeerShard:
         self.arena, self.d_max, self.batch_max = arena, int(d_max), int(batch_max)
         self.edges_total, self.edges_own = int(edges_total), int(edges_own)
         self.catalogue_width = int(catalogue_width)
-        self.off = self.layout(world, self.rpp, self.d_max, self.batch_max, self.catalogue_width)
+        self.grad_floats = int(grad_floats)
+        # training (_train_forward / _train_backward): unmasked in-degrees of the owned users and of ALL items, the number of interaction positions the local
+        # indexes' `pos` refer to (skip bitmap size), and whether the reverse weights w_bwd describe the same edges (binary=False graphs)
+        self.deg_users, self.deg_items_all = deg_users, deg_items_all
+        self.n_positions, self.symmetric = int(n_positions), bool(symmetric)
+        self._mlp_generator = None
+        self.off = self.layout(world, self.rpp, self.d_max, self.batch_max, self.catalogue_width, self.grad_floats)
         self.device = arena.buf.device
         self._flag_ptrs = arena.ptrs(0)
         self._counters = arena.buf[_OFF_COUNTERS:].data_ptr()
@@ -177,7 +196,7 @@ class PeerShard:
         self._seen = Derived(1)                                        # seen CSR of every owned user (recommend_peer, users=None)
 
     @staticmethod
-    def layout(world, rpp, d_max, batch_max, catalogue_width=0):
+    def layout(world, rpp, d_max, batch_max, catalogue_width=0, grad_floats=0):
         off, cur = {}, _CTRL_BYTES
         slab = _align(world * rpp * d_max * 4)
         for name in ('recv0', 'recv1', 'T0', 'T1'):
@@ -192,8 +211,20 @@ class PeerShard:
         if catalogue_width:                 # recommend_peer: the final item rows of ALL items, (P * rpp, catalogue_width) fp32
             off['cat'] = cur
             cur += _align(world * rpp * catalogue_width * 4)
+        if grad_floats:                     # training: one slot of grad_floats fp32 (rounded up to 4) per rank, summed in rank order
+            off['grad'] = cur
+            cur += _align(world * _round4(grad_floats) * 4)
         off['total'] = cur
         return off
+
+    @property
+    def mlp_generator(self):
+        """generator of the MLP dropout masks in training: seeded with MLP_DROPOUT_SEED on every rank and advanced by the same draws, so
+        that every rank drops the same units of the (identical) batch MLP"""
+        if self._mlp_generator is None:
+            self._mlp_generator = torch.Generator(device=self.device)
+            self._mlp_generator.manual_seed(MLP_DROPOUT_SEED)
+        return self._mlp_generator
 
     # ---- exchange primitives ---------------------------------------------------------------------------------------------
     def signal(self, channel):
@@ -333,7 +364,7 @@ def _rows_per_part(nI, world):
     return max(1, (int(nI) + world - 1) // world)
 
 
-def shard_from_full(graph, rank, world, arena, d_max, batch_max=8192, catalogue_width=0):
+def shard_from_full(graph, rank, world, arena, d_max, batch_max=8192, catalogue_width=0, grad_floats=0):
     """Shard of rank `rank` cut out of the full neighbour index (every rank builds the ~10 ms full index and keeps its slices;
     graphs that do not fit one GPU are built per rank instead: `bench.py --workload graph5`)."""
     from .parallel import RowPartition, _LocalIndex, column_slice_csr, split_rows
@@ -347,36 +378,40 @@ def shard_from_full(graph, rank, world, arena, d_max, batch_max=8192, catalogue_
     dinv_users = full.dinv[nI + users.r0: nI + users.r1].contiguous()
     dinv_items = full.dinv[:nI].contiguous()
     index_users = _LocalIndex((rp[nI + users.r0: nI + users.r1 + 1] - k0).contiguous(), full.col[k0:k1].contiguous(), cut(full.w), cut(full.pos),
-                              dinv_users, full.chunk_size)
+                              dinv_users, full.chunk_size, w_bwd=cut(full.w_bwd))
     head = lambda a: None if a is None else a[:k_items]
-    lrp, lcol, lw, lpos = column_slice_csr(rp[:nI + 1], full.col[:k_items], nI + users.r0, nI + users.r1, head(full.w), head(full.pos))
-    index_items = _LocalIndex(lrp, lcol, lw, lpos, dinv_items, full.chunk_size)
+    lrp, lcol, lw, lpos, lwb = column_slice_csr(rp[:nI + 1], full.col[:k_items], nI + users.r0, nI + users.r1, head(full.w), head(full.pos),
+                                                head(full.w_bwd))
+    index_items = _LocalIndex(lrp, lcol, lw, lpos, dinv_items, full.chunk_size, w_bwd=lwb)
     rpp = _rows_per_part(nI, world)
     i0 = min(rank * rpp, nI)
     return PeerShard(rank=rank, world=world, nI=nI, nU=N - nI, d_max=d_max, rpp=rpp, users_r0=users.r0, users_rows=users.rows,
                      index_users=index_users, index_items=index_items, dinv_users=dinv_users, dinv_items_all=dinv_items,
                      item_features_own=graph.item_features[i0: min(i0 + rpp, nI)], user_features_own=graph.user_features[users.r0:users.r1],
                      arena=arena, batch_max=batch_max, edges_total=full.e1 + full.e2, edges_own=int(index_users.col.numel() + lcol.numel()),
-                     catalogue_width=catalogue_width)
+                     catalogue_width=catalogue_width, grad_floats=grad_floats, deg_users=full.deg[nI + users.r0: nI + users.r1].contiguous(),
+                     deg_items_all=full.deg[:nI].contiguous(), n_positions=full.e1, symmetric=full.symmetric)
 
 
-def partition_graph_peer(graph, group=None, d_max=128, batch_max=8192, catalogue_width=0):
+def partition_graph_peer(graph, group=None, d_max=128, batch_max=8192, catalogue_width=0, grad_floats=0):
     """One process per GPU: allocates + exchanges the arenas and cuts this rank's shard.  `d_max` = largest node_emb served;
-    `catalogue_width` = floats per item row of the catalogue section that `recommend_peer` needs (`catalogue_width(model)`; 0 = none)."""
+    `catalogue_width` = floats per item row of the catalogue section that `recommend_peer` needs (`catalogue_width(model)`; 0 = none);
+    `grad_floats` = floats per rank of the gradient section that training needs (`grad_floats(model)`; 0 = none)."""
     import torch.distributed as dist
     world = dist.get_world_size(group)
     nI = int(graph.item_features.shape[0])
-    nbytes = PeerShard.layout(world, _rows_per_part(nI, world), d_max, batch_max, catalogue_width)['total']
+    nbytes = PeerShard.layout(world, _rows_per_part(nI, world), d_max, batch_max, catalogue_width, grad_floats)['total']
     arena = PeerArena.ipc(nbytes, group, device=graph.item_features.device)
-    return shard_from_full(graph, dist.get_rank(group), world, arena, d_max, batch_max, catalogue_width)
+    return shard_from_full(graph, dist.get_rank(group), world, arena, d_max, batch_max, catalogue_width, grad_floats)
 
 
-def emulated_shards(graph, world, d_max=128, batch_max=8192, catalogue_width=0):
-    """all P shards in ONE process (single-GPU tests of the exchange logic; run with `forward_emulated` / `recommend_emulated`)"""
+def emulated_shards(graph, world, d_max=128, batch_max=8192, catalogue_width=0, grad_floats=0):
+    """all P shards in ONE process (single-GPU tests of the exchange logic; run with `forward_emulated` / `recommend_emulated` /
+    `train_emulated`)"""
     nI = int(graph.item_features.shape[0])
-    nbytes = PeerShard.layout(world, _rows_per_part(nI, world), d_max, batch_max, catalogue_width)['total']
+    nbytes = PeerShard.layout(world, _rows_per_part(nI, world), d_max, batch_max, catalogue_width, grad_floats)['total']
     arenas = PeerArena.emulated(nbytes, world, graph.item_features.device)
-    return [shard_from_full(graph, q, world, arenas[q], d_max, batch_max, catalogue_width) for q in range(world)]
+    return [shard_from_full(graph, q, world, arenas[q], d_max, batch_max, catalogue_width, grad_floats) for q in range(world)]
 
 
 # ----------------------------------------------------------------------------------------------------------------------
@@ -574,13 +609,16 @@ def _layer0_composites(model, ie, ue, lin_i, lin_u, att_i=None, att_u=None):
     return model._peer_layer0.get((ie.weight, ie.bias, ue.weight, ue.bias, lin_i.weight, lin_i.bias, lin_u.weight, lin_u.bias) + att, build)
 
 
-def forward_peer(model, sh: PeerShard, userIds, itemIds, keep=None):
-    gen = _steps(model, sh, userIds, itemIds, keep)
-    try:
-        while True:
-            next(gen)
-    except StopIteration as stop:
-        return stop.value
+def forward_peer(model, sh: PeerShard, userIds, itemIds, keep=None, mask_targets=True):
+    """GraphNCF.forward on a partitioned graph; every rank of the group calls it with the same batch and gets the same (B, 1) scores.
+
+    With grad off this is the inference forward (`model.training` is not looked at).  With grad on it is the training forward: the
+    scores carry a grad_fn, and `loss.backward()`, called by every rank, leaves the gradient of that loss in every parameter's `.grad`,
+    bit-identical on all ranks.  `model.training` then switches on target masking (`mask_targets`) and dropout, as on one GPU.  The
+    partition needs a gradient section of `grad_floats(model)` floats (ValueError otherwise)."""
+    if torch.is_grad_enabled() and any(p.requires_grad for p in model.parameters()):
+        return _head(model, sh, _PeerTrainFn.apply(model, sh, userIds, itemIds, mask_targets, keep, *_train_params(model).values()))
+    return _run(_steps(model, sh, userIds, itemIds, keep))
 
 
 def forward_emulated(model, shards, userIds, itemIds, keep=None):
@@ -756,3 +794,366 @@ def recommend_emulated(model, shards, **kw):
                 outs[q] = stop.value
                 live.remove(q)
     return outs
+
+
+# ----------------------------------------------------------------------------------------------------------------------
+# training on the partitioned graph (LightGCN, mean combine)
+# ----------------------------------------------------------------------------------------------------------------------
+def _train_params(model):
+    """{name: parameter} of the embedding and conv parameters, in the order of the flat gradient vector.  The MLP is not among them: every
+    rank runs it on the same batch rows under ordinary autograd, so its gradients are already the same on every rank."""
+    return {n: p for n, p in model.named_parameters() if n.startswith(('item_embeddings.', 'user_embeddings.', 'gnn_convs.'))}
+
+
+def _slot(p):
+    return _round4(p.numel())                       # every parameter starts 16-byte aligned in the flat vector
+
+
+def grad_floats(model):
+    """Floats per rank of the gradient section (`grad_floats=` of the partition builders) that training `model` needs: the embedding and
+    conv parameters, each padded to a multiple of 4"""
+    return sum(_slot(p) for p in _train_params(model).values())
+
+
+def _train_check(model, sh: PeerShard, B):
+    """node_emb d after the checks of a training call (all made before any rank signals)"""
+    if model.convType != 'LightGCN':
+        raise NotImplementedError(f"partitioned training covers convType='LightGCN', not convType={model.convType!r} (train it on one GPU)")
+    if model.concat:
+        raise NotImplementedError('partitioned training covers the mean combine, not concat=True (train it on one GPU)')
+    for name in ('node_dropout', 'message_dropout'):
+        if getattr(model, name) is not None and getattr(model, name) > 0.0:
+            raise NotImplementedError(f'partitioned training does not support {name} (train it on one GPU)')
+    if not sh.symmetric:
+        raise NotImplementedError('partitioned training needs a binary=False graph: its backward multiplies by the reverse-edge weights of the same '
+                                  'index, and edge masking has the same restriction on one GPU')
+    d = model.item_embeddings[0].weight.shape[0]
+    if d > sh.d_max or d % 4:
+        raise ValueError(f'node_emb {d} does not fit the arena of this partition (d_max {sh.d_max}) or is not a multiple of 4')
+    if B > sh.batch_max:
+        raise ValueError(f'batch of {B} pairs exceeds the partition\'s batch_max {sh.batch_max}')
+    need = grad_floats(model)
+    if sh.grad_floats < need:
+        raise ValueError(f'training needs a gradient section of {need} floats per rank; this partition has {sh.grad_floats} '
+                         f'(build it with grad_floats={need})')
+    return d
+
+
+def _mask_batch(sh: PeerShard, uid, iid):
+    """(skip bitmap, masked dinv of the owned users, masked dinv of ALL items, count of pairs this rank could not find) for the batch targets.
+    Identical pairs of the batch count once (GraphIndex.masked: one interaction position each).  Every rank takes the item degrees down
+    from the batch alone; the owner of a pair's user finds its position in its local pair hash and masks it in both local indexes."""
+    dev, B, lib = sh.device, int(uid.numel()), L.lib()
+    skip = torch.zeros((sh.n_positions + 31) // 32 + 1, dtype=torch.int32, device=dev)
+    deg_u, deg_i = sh.deg_users.clone(), sh.deg_items_all.clone()
+    dinv_u, dinv_i = torch.empty(sh.users_rows, dtype=torch.float32, device=dev), torch.empty(sh.nI, dtype=torch.float32, device=dev)
+    cap = 1 << max(4, (2 * B - 1).bit_length())
+    keys, vals = torch.empty(cap, dtype=torch.int64, device=dev), torch.empty(cap, dtype=torch.int32, device=dev)
+    first = torch.empty(B, dtype=torch.int64, device=dev)
+    missing = torch.zeros(1, dtype=torch.int32, device=dev)
+    pairs = torch.stack((uid, iid))
+    hk, hv, hcap = sh.index_users.pair_hash(sh.nI + sh.users_r0)
+    with torch.cuda.device(dev):
+        st = _stream()
+        # first[j] = the first batch entry holding the pair of entry j (a batch-local hash; every pair is found)
+        L.check(lib.b200rec_pairhash_build(_ptr(pairs), B, _ptr(keys), _ptr(vals), cap, st), 'pairhash_build')
+        L.check(lib.b200rec_pairhash_lookup(_ptr(uid), _ptr(iid), B, _ptr(keys), _ptr(vals), cap, _ptr(first), _ptr(missing), st), 'pairhash_lookup')
+        L.check(lib.b200rec_peer_mask_targets(_ptr(uid), _ptr(iid), B, _ptr(first), sh.nI, sh.N, sh.nI + sh.users_r0, sh.users_rows, _ptr(hk), _ptr(hv),
+                                              hcap, _ptr(sh.index_users.pos), _ptr(skip), _ptr(deg_u), _ptr(deg_i), _ptr(missing), st), 'peer_mask_targets')
+        if sh.users_rows:
+            L.check(lib.b200rec_dinv(_ptr(deg_u), sh.users_rows, _ptr(dinv_u), st), 'dinv')
+        L.check(lib.b200rec_dinv(_ptr(deg_i), sh.nI, _ptr(dinv_i), st), 'dinv')
+    return skip, dinv_u, dinv_i, missing
+
+
+def _train_forward(model, sh: PeerShard, userIds, itemIds, mask_targets, keep=None):
+    """Generator (yields like `_steps`): the training forward of GraphNCF on shard `sh` up to the batch rows.  Returns ((2B, d) batch rows,
+    item rows first, the same on every rank; what the backward needs).  Layer 0 runs as two steps, x0 = W_e f + b_e and
+    t0 = drop(dinv ∘ (W_t x0 + b_t)), like the single-GPU training path; each row's conv-dropout mask is drawn by its owner."""
+    B = int(userIds.shape[0])
+    d = _train_check(model, sh, B)
+    dev, nI = sh.device, sh.nI
+    uid, iid = userIds.to(dev).long().contiguous(), itemIds.to(dev).long().contiguous()
+    L_ = len(model.gnn_convs)
+    ie, ue = model.item_embeddings[0], model.user_embeddings[0]
+    nu, ni = sh.users_rows, sh.it_rows
+    empty = lambda n: torch.empty((n, d), dtype=torch.float32, device=dev)
+    skip, dinv_u, dinv_i = None, sh.dinv_users, sh.dinv_items_all
+    if model.training and mask_targets:
+        skip, dinv_u, dinv_i, missing = _mask_batch(sh, uid, iid)
+        # every rank learns every rank's count before any data moves, so that a batch with a non-edge fails on all ranks alike
+        with torch.cuda.device(dev):
+            L.check(L.lib().b200rec_peer_push_floats(_ptr(missing), 1, sh.arena.ptrs(0), sh.world, _OFF_MISSING // 4 + sh.rank, _stream()),
+                    'peer_push_floats')
+        sh.signal(CH_M)
+        yield
+        sh.wait(CH_M)
+        if sum(sh.arena.view(_OFF_MISSING, (sh.world,), torch.int32).tolist()):
+            raise KeyError('batch pairs that are not edges of the graph (pos_df.loc raises KeyError in the reference, gnn_ncf.py:370)')
+    dinv_i_own = dinv_i[sh.it_r0: sh.it_r0 + ni]
+    x0_i, x0_u = empty(ni), empty(nu)
+    if ni:
+        ops.linear_raw(sh.item_features_own, ie.weight, ie.bias, out=x0_i)
+    if nu:
+        ops.linear_raw(sh.user_features_own, ue.weight, ue.bias, out=x0_u)
+    xs_i, xs_u, masks_i, masks_u = [], [], [], []
+    acc_i, acc_u = x0_i, x0_u
+    if L_ > 0:
+        lin_u, lin_i, p = model.gnn_convs[0].typed()
+        p = p if model.training else 0.0
+        acc_i, acc_u = empty(ni), empty(nu)
+        t_u = empty(max(nu, 1))
+
+        def transform(x, lin, rs, out):              # out = drop(rs ∘ (W x + b)); returns the dropout multipliers (0 or 1/(1-p)) or None
+            if x.shape[0] == 0:
+                return None
+            ops.linear_raw(x, lin.weight, lin.bias, row_scale=rs, out=out)
+            if p <= 0.0:
+                return None
+            m = torch.empty_like(out).bernoulli_(1.0 - p).div_(1.0 - p)
+            ops.scale_rows_raw(out, mask=m, out=out)
+            return m
+
+        def publish(x, par):                         # the owned item messages into T[par] of every rank
+            local = sh.table(par, d, torch.float32)[sh.it_r0: sh.it_r0 + ni]
+            m = transform(x, lin_i, dinv_i_own, local)
+            _push_table_rows(sh, local, par, d)
+            return m
+
+        x_i, x_u = x0_i, x0_u
+        masks_u.append(transform(x_u, lin_u, dinv_u, t_u[:nu]))
+        masks_i.append(publish(x_i, 0))
+        sh.signal(CH_T0)
+        for l in range(L_):
+            par, last = l & 1, l == L_ - 1
+            scale = 1.0 / (L_ + 1) if last else 1.0
+            xs_i.append(x_i)
+            xs_u.append(x_u)
+            if nu:                                   # A_l: partial item rows -> owners' receive slots
+                ops.spmm_raw(sh.index_items, t_u, w=sh.index_items.w, dinv=dinv_i, skip_bits=skip, push=sh.push_spec(par, d))
+            sh.signal(CH_A0 + par)
+            yield
+            sh.wait(CH_A0 + par)                     # C_l: owned item rows, then their messages for the next layer
+            xi_next = None if last else empty(ni)
+            sh.reduce(par, d, x_next=xi_next, acc_in=x0_i if l == 0 else acc_i, acc_out=acc_i, acc_scale=scale)
+            if not last:
+                masks_i.append(publish(xi_next, 1 - par))
+                sh.signal(CH_T0 + (1 - par))
+            sh.wait(CH_T0 + par)                     # B_l: owned user rows from the gathered table
+            xu_next = None if last else empty(nu)
+            if nu:
+                ops.spmm_raw(sh.index_users, sh.table(par, d, torch.float32), w=sh.index_users.w, dinv=dinv_u, skip_bits=skip, x_next=xu_next,
+                             acc_in=x0_u if l == 0 else acc_u, acc_out=acc_u, acc_scale=scale)
+            if not last:
+                masks_u.append(transform(xu_next, lin_u, dinv_u, t_u[:nu]))
+            x_i, x_u = xi_next, xu_next
+    sh.gather_rows(acc_i, sh.it_r0, ni, iid, 0, d)
+    sh.gather_rows(acc_u, nI + sh.users_r0, nu, uid, B, d)
+    sh.signal(CH_R)
+    yield
+    sh.wait(CH_R)
+    rows = sh.rows_view(2 * B, d).clone()
+    if L_ == 0:                                      # no layer barrier protects `rows` against the next call's writers
+        sh.signal(CH_E)
+        yield
+        sh.wait(CH_E)
+    if keep is not None:                             # tests: the owned combined rows and the conv-dropout multipliers of every layer
+        keep.update(items=acc_i, users=acc_u, masks_items=masks_i, masks_users=masks_u)
+    return rows, dict(uid=uid, iid=iid, d=d, skip=skip, dinv_u=dinv_u, dinv_i_own=dinv_i_own, xs_i=xs_i, xs_u=xs_u, masks_i=masks_i,
+                      masks_u=masks_u)
+
+
+def _push_table_rows(sh: PeerShard, local, par, d):
+    """rows it_r0 .. of the local T[par] into T[par] of every other rank"""
+    if local.shape[0] == 0 or sh.world == 1:
+        return
+    others = (C.c_void_p * (sh.world - 1))(*[sh.arena.bases[q] + sh.off[f'T{par}'] for q in range(sh.world) if q != sh.rank])
+    with torch.cuda.device(sh.device):
+        L.check(L.lib().b200rec_peer_push_rows(_ptr(local), d, local.shape[0], d, others, sh.world - 1, sh.it_r0 * d, d, _stream()), 'peer_push_rows')
+
+
+def _train_backward(model, sh: PeerShard, saved, g_rows):
+    """Generator (yields like `_steps`): the backward of `_train_forward` on shard `sh` for the gradient `g_rows` of its batch rows (the same
+    on every rank).  Returns {name: gradient} of the embedding and conv parameters, summed over the ranks in rank order (bit-identical on
+    every rank).  Per layer l = L-1 .. 0, with G_l the gradient of the owned rows x_l and par = l & 1:
+
+        C'  s_i = dinv_i ∘ G_{l+1,i} of the owned items -> T[par] of every rank;  g_t_u = K3(index_users, w_bwd, T[par])
+        A'  K3(index_items, w_bwd, dinv_u ∘ G_{l+1,u}) -> the owners' recv[par];  g_t_i = the P slots summed in rank order
+        G_l = G_L + (dinv ∘ mask ∘ g_t) W;   partial dW += (dinv ∘ mask ∘ g_t)ᵀ x_l,  db += its column sums
+
+    It starts after the forward's CH_R barrier, when every exchange section is free, and ends with the gradient exchange on CH_G."""
+    d, uid, iid = saved['d'], saved['uid'], saved['iid']
+    B = int(uid.numel())
+    dev = sh.device
+    L_ = len(model.gnn_convs)
+    nu, ni = sh.users_rows, sh.it_rows
+    params = _train_params(model)
+    need = grad_floats(model)
+    flat = torch.zeros(need, dtype=torch.float32, device=dev)
+    views, o = {}, 0
+    for name, p in params.items():
+        views[id(p)] = flat[o: o + p.numel()].view((1, -1) if p.dim() == 1 else p.shape)
+        o += _slot(p)
+    ones = torch.ones((1, max(nu, ni, 1)), dtype=torch.float32, device=dev)
+
+    def add_grad(p, g):                              # slot of p += g
+        v = views[id(p)]
+        ops.scale_rows_raw(g.view(v.shape), add=v, out=v)
+
+    def transform_backward(gt, m, rs, lin, x, base):
+        if gt.shape[0] == 0:
+            return base
+        g_lin = torch.empty_like(gt)
+        ops.scale_rows_raw(gt, mask=m, row_scale=rs, out=g_lin)
+        add_grad(lin.weight, ops.linear_raw(g_lin.t(), x.t()))
+        if lin.bias is not None:
+            add_grad(lin.bias, ops.linear_raw(ones[:, :gt.shape[0]], g_lin.t()))
+        out = ops.linear_raw(g_lin, lin.weight.t())
+        ops.scale_rows_raw(out, add=base, out=out)
+        return out
+
+    g = g_rows.contiguous().float()
+    G_i, G_u = torch.zeros((ni, d), dtype=torch.float32, device=dev), torch.zeros((nu, d), dtype=torch.float32, device=dev)
+    ops.rows_to_owned_raw(g[:B], iid, sh.it_r0, ni, 1.0 / (L_ + 1), G_i)
+    ops.rows_to_owned_raw(g[B:], uid, sh.nI + sh.users_r0, nu, 1.0 / (L_ + 1), G_u)
+    if L_ > 0:
+        lin_u, lin_i, _ = model.gnn_convs[0].typed()
+        skip, dinv_u, dinv_i_own = saved['skip'], saved['dinv_u'], saved['dinv_i_own']
+        base_i, base_u = G_i, G_u                    # what every x_l receives from the mean
+        s_u = torch.empty((max(nu, 1), d), dtype=torch.float32, device=dev)
+        for l in reversed(range(L_)):
+            par = l & 1
+            local = sh.table(par, d, torch.float32)[sh.it_r0: sh.it_r0 + ni]
+            if ni:
+                ops.scale_rows_raw(G_i, row_scale=dinv_i_own, out=local)
+            _push_table_rows(sh, local, par, d)
+            sh.signal(CH_T0 + par)
+            if nu:
+                ops.scale_rows_raw(G_u, row_scale=dinv_u, out=s_u[:nu])
+                ops.spmm_raw(sh.index_items, s_u, w=sh.index_items.w_bwd, dinv=None, skip_bits=skip, push=sh.push_spec(par, d))
+            sh.signal(CH_A0 + par)
+            yield
+            sh.wait(CH_T0 + par)
+            gt_u = torch.empty((nu, d), dtype=torch.float32, device=dev)
+            if nu:
+                ops.spmm_raw(sh.index_users, sh.table(par, d, torch.float32), w=sh.index_users.w_bwd, dinv=None, skip_bits=skip, x_next=gt_u)
+            sh.wait(CH_A0 + par)
+            gt_i = torch.empty((ni, d), dtype=torch.float32, device=dev)
+            sh.reduce(par, d, x_next=gt_i, acc_in=None, acc_out=None, acc_scale=1.0)
+            G_u = transform_backward(gt_u, saved['masks_u'][l], dinv_u, lin_u, saved['xs_u'][l], base_u)
+            G_i = transform_backward(gt_i, saved['masks_i'][l], dinv_i_own, lin_i, saved['xs_i'][l], base_i)
+    for n, G, f, emb in ((ni, G_i, sh.item_features_own, model.item_embeddings[0]), (nu, G_u, sh.user_features_own, model.user_embeddings[0])):
+        if n:
+            ops.linear_raw(G.t(), f.t(), out=views[id(emb.weight)])
+            if emb.bias is not None:
+                ops.linear_raw(ones[:, :n], G.t(), out=views[id(emb.bias)])
+    # the partial gradients -> slot `rank` of every rank's gradient section; every rank sums the P slots in rank order
+    stride = _round4(sh.grad_floats)
+    with torch.cuda.device(dev):
+        L.check(L.lib().b200rec_peer_push_rows(_ptr(flat), need, 1, need, sh.arena.ptrs(sh.off['grad']), sh.world, sh.rank * stride, need, _stream()),
+                'peer_push_rows')
+    sh.signal(CH_G)
+    yield
+    sh.wait(CH_G)
+    total = torch.empty(need, dtype=torch.float32, device=dev)
+    slots = sh.arena.view(sh.off['grad'], (sh.world * stride,))
+    with torch.cuda.device(dev):
+        L.check(L.lib().b200rec_peer_reduce(_ptr(slots), sh.world, stride, need, 1, need, _ptr(total), need, None, None, need, 1.0, _stream()),
+                'peer_reduce')
+    out, o = {}, 0
+    for name, p in params.items():
+        out[name] = total[o: o + p.numel()].view(p.shape)
+        o += _slot(p)
+    return out
+
+
+class _RowDotFn(torch.autograd.Function):
+    """(B, 1) row-wise dot products of the batch rows (the dot-product head, gnn_ncf.py:365) with a gradient"""
+
+    @staticmethod
+    def forward(ctx, a, b):
+        ctx.save_for_backward(a, b)
+        return ops.rowdot(a, b)
+
+    @staticmethod
+    def backward(ctx, g):
+        a, b = ctx.saved_tensors
+        return g * b, g * a
+
+
+def _head(model, sh: PeerShard, rows):
+    """scores of the (2B, d) batch rows (items first) under autograd; the MLP's dropout masks come from the shard's generator"""
+    from .neural_collaborative_filtering.util import run_mlp
+    B = rows.shape[0] // 2
+    if model.MLP is None:
+        return _RowDotFn.apply(rows[B:], rows[:B])
+    return run_mlp(model.MLP, rows[:B], rows[B:], training=model.training, generator=sh.mlp_generator)
+
+
+def _run(gen):
+    try:
+        while True:
+            next(gen)
+    except StopIteration as stop:
+        return stop.value
+
+
+class _PeerTrainFn(torch.autograd.Function):
+    """(embedding and conv parameters) -> the (2B, d) batch rows of a partitioned propagation.  backward is collective: every rank runs it."""
+
+    @staticmethod
+    def forward(ctx, model, sh, userIds, itemIds, mask_targets, keep, *params):
+        rows, saved = _run(_train_forward(model, sh, userIds, itemIds, mask_targets, keep))
+        ctx.state = (model, sh, saved)
+        return rows
+
+    @staticmethod
+    def backward(ctx, g):
+        model, sh, saved = ctx.state
+        ctx.state = None
+        grads = _run(_train_backward(model, sh, saved, g))
+        return (None,) * 6 + tuple(grads.values())
+
+
+def _lockstep(gens):
+    """runs the generators of all emulated ranks segment by segment; when one rank raises, the others still run to their end (or their own
+    error), and the error is raised when every rank raised the same kind"""
+    outs, errs = [None] * len(gens), [None] * len(gens)
+    live = list(range(len(gens)))
+    with torch.no_grad():
+        while live:
+            for q in list(live):
+                try:
+                    next(gens[q])
+                except StopIteration as stop:
+                    outs[q] = stop.value
+                    live.remove(q)
+                except Exception as e:              # noqa: BLE001 (re-raised below)
+                    errs[q] = e
+                    live.remove(q)
+    failed = [e for e in errs if e is not None]
+    if failed:
+        if len(failed) == len(errs) and all(type(e) is type(failed[0]) for e in failed):
+            raise failed[0]
+        raise RuntimeError(f'emulated ranks failed differently: {errs}') from failed[0]
+    return outs
+
+
+def train_emulated(model, shards, userIds, itemIds, loss_fn, mask_targets=True, keep=None):
+    """One training step's forward and backward on all ranks of `emulated_shards` in lock step.  `loss_fn(out)` maps a rank's (B, 1) scores
+    to its scalar loss.  Returns, per rank, (scores, {parameter name: gradient}); nothing is written to `.grad`."""
+    keep = keep if keep is not None else [None] * len(shards)
+    fwd = _lockstep([_train_forward(model, sh, userIds, itemIds, mask_targets, keep[q]) for q, sh in enumerate(shards)])
+    own = _train_params(model)
+    head = {n: p for n, p in model.named_parameters() if n not in own and p.requires_grad}
+    outs, g_rows, head_grads = [], [], []
+    for q, sh in enumerate(shards):
+        rows = fwd[q][0].requires_grad_()
+        with torch.enable_grad():
+            out = _head(model, sh, rows)
+            gs = torch.autograd.grad(loss_fn(out), [rows] + list(head.values()), allow_unused=True)
+        outs.append(out.detach())
+        g_rows.append(gs[0])
+        head_grads.append({n: g for n, g in zip(head, gs[1:]) if g is not None})
+    bwd = _lockstep([_train_backward(model, sh, fwd[q][1], g_rows[q]) for q, sh in enumerate(shards)])
+    return [(outs[q], {**bwd[q], **head_grads[q]}) for q in range(len(shards))]

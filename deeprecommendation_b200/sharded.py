@@ -58,8 +58,10 @@ def create_graph_local(u_local, items, ratings, n_local_users, nI, item_features
                      user2item_edge_attr=attr_u, item2user_edge_attr=attr_i)
 
 
-def shard_from_local(graph_local, *, rank, world, nI, nU, users_r0, arena, d_max, batch_max, reduce_items=None, edges_total=None, catalogue_width=0):
-    """PeerShard of a rank from the graph of its own interactions (`create_graph_local`)."""
+def shard_from_local(graph_local, *, rank, world, nI, nU, users_r0, arena, d_max, batch_max, reduce_items=None, edges_total=None, catalogue_width=0,
+                     grad_floats=0):
+    """PeerShard of a rank from the graph of its own interactions (`create_graph_local`).  The local indexes keep the local graph's reverse
+    weights `w_bwd` and its interaction positions, so that training can mask the batch targets of the owned users."""
     from .parallel import _LocalIndex
     from .peer import PeerShard, _rows_per_part
     dev = graph_local.item_features.device
@@ -76,10 +78,11 @@ def shard_from_local(graph_local, *, rank, world, nI, nU, users_r0, arena, d_max
     k_items = int(rp[nI])
     dinv_users = idx.dinv[nI:].contiguous()
     index_items = _LocalIndex(rp[:nI + 1].contiguous(), (idx.col[:k_items] - nI).contiguous(), idx.w[:k_items].contiguous(), idx.pos[:k_items].contiguous(),
-                              dinv_items, idx.chunk_size)
+                              dinv_items, idx.chunk_size, w_bwd=idx.w_bwd[:k_items].contiguous())
     index_users = _LocalIndex((rp[nI:] - k_items).contiguous(), idx.col[k_items:].contiguous(), idx.w[k_items:].contiguous(), idx.pos[k_items:].contiguous(),
-                              dinv_users, idx.chunk_size)
+                              dinv_users, idx.chunk_size, w_bwd=idx.w_bwd[k_items:].contiguous())
     own = int(idx.e1 + idx.e2)
+    deg_users, n_positions, symmetric = idx.deg[nI:].contiguous(), idx.e1, idx.symmetric
     del idx
     rpp = _rows_per_part(nI, world)
     i0 = min(rank * rpp, nI)
@@ -87,13 +90,14 @@ def shard_from_local(graph_local, *, rank, world, nI, nU, users_r0, arena, d_max
                      index_items=index_items, dinv_users=dinv_users, dinv_items_all=dinv_items,
                      item_features_own=graph_local.item_features[i0: min(i0 + rpp, nI)], user_features_own=graph_local.user_features,
                      arena=arena, batch_max=batch_max, edges_total=own if edges_total is None else edges_total, edges_own=own,
-                     catalogue_width=catalogue_width)
+                     catalogue_width=catalogue_width, grad_floats=grad_floats, deg_users=deg_users, deg_items_all=deg_items,
+                     n_positions=n_positions, symmetric=symmetric)
 
 
 def build_shard(u_local, items, ratings, *, nI, nU, users_r0, n_local_users, item_features, user_features_local, group=None, d_max=64,
-                batch_max=8192, edges_total=None, catalogue_width=0):
+                batch_max=8192, edges_total=None, catalogue_width=0, grad_floats=0):
     """One process per GPU: the PeerShard of this rank from its own interactions + the arena exchange (collectives at build time only).
-    `catalogue_width` > 0 adds the catalogue section of `peer.recommend_peer`."""
+    `catalogue_width` > 0 adds the catalogue section of `peer.recommend_peer`, `grad_floats` > 0 the gradient section of training."""
     import torch.distributed as dist
     from .peer import PeerArena, PeerShard, _rows_per_part
     world, rank = dist.get_world_size(group), dist.get_rank(group)
@@ -102,7 +106,8 @@ def build_shard(u_local, items, ratings, *, nI, nU, users_r0, n_local_users, ite
         dist.all_reduce(t, group=group)
 
     g = create_graph_local(u_local, items, ratings, n_local_users, nI, item_features, user_features_local, reduce_items if world > 1 else None)
-    nbytes = PeerShard.layout(world, _rows_per_part(nI, world), d_max, batch_max, catalogue_width)['total']
+    nbytes = PeerShard.layout(world, _rows_per_part(nI, world), d_max, batch_max, catalogue_width, grad_floats)['total']
     arena = PeerArena.ipc(nbytes, group, device=u_local.device)
     return shard_from_local(g, rank=rank, world=world, nI=nI, nU=nU, users_r0=users_r0, arena=arena, d_max=d_max, batch_max=batch_max,
-                            reduce_items=reduce_items if world > 1 else None, edges_total=edges_total, catalogue_width=catalogue_width)
+                            reduce_items=reduce_items if world > 1 else None, edges_total=edges_total, catalogue_width=catalogue_width,
+                            grad_floats=grad_floats)

@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define B200REC_VERSION 208
+#define B200REC_VERSION 209
 
 typedef void* b200rec_stream_t; /* cudaStream_t */
 
@@ -524,6 +524,24 @@ int b200rec_peer_push_floats(const float* src, int64_t n, void* const* dst, int 
  * row (dst_offset / ld_dst + j) of every destination receives table[ids[j] - row0] * scale */
 int b200rec_peer_gather_rows(const float* table, int64_t ld, int64_t row0, int64_t rows, const int64_t* ids, int64_t n_ids, int d,
                              float scale, void* const* dst, int n_dst, int64_t dst_offset, int64_t ld_dst, b200rec_stream_t stream);
+
+/* ---- training on the partitioned graph (peer.py: train_emulated / forward_peer with grad) ---------------------------------
+ * out = scale · x ∘ mask ∘ row_scale[r] (+ add), elementwise over (rows, d); mask, row_scale and add may be NULL, out may alias x or add.
+ * d and the leading dimensions multiples of 4, pointers 16-byte aligned. */
+int b200rec_peer_scale_rows(const float* x, int64_t ld_x, int64_t rows, int d, const float* mask, int64_t ld_m, const float* row_scale,
+                            float scale, const float* add, int64_t ld_add, float* out, int64_t ld_out, b200rec_stream_t stream);
+/* sorted / perm (n int64): batch ids sorted stably and their batch positions.  For every id with row0 <= id < row0 + rows:
+ * out[id - row0] = scale · Σ g[j] over the batch positions j of that id, summed in batch order (deterministic, no atomics).  Rows no
+ * id names are not written. */
+int b200rec_peer_rows_to_owned(const float* g, int64_t ld_g, const int64_t* sorted, const int64_t* perm, int64_t n, int64_t row0, int64_t rows,
+                               int d, float scale, float* out, int64_t ld_out, b200rec_stream_t stream);
+/* the batch targets (uid[i] user node, iid[i] item) on one rank, for the entries with first[i] == i (first entry of an identical pair):
+ * deg_items[iid] -= 1 on every rank; the owner of the user (node0 <= uid < node0 + rows) looks the pair up in its pair hash (keys / vals
+ * as from b200rec_pairhash_build over its CSR entries; capacity a power of two), sets bit local_pos[entry] of skip_bits and does
+ * deg_users[uid - node0] -= 1.  *n_missing += 1 for a pair the owner does not find and for ids outside [0, n_items) / [n_items, n_nodes). */
+int b200rec_peer_mask_targets(const int64_t* uid, const int64_t* iid, int64_t n, const int64_t* first, int64_t n_items, int64_t n_nodes,
+                              int64_t node0, int64_t rows, const uint64_t* keys, const int* vals, int64_t capacity, const int* local_pos,
+                              uint32_t* skip_bits, int* deg_users, int* deg_items, int* n_missing, b200rec_stream_t stream);
 
 /* tracing aid: *slot = %globaltimer (ns) when the stream reaches this point (one 1-thread kernel; usable inside a captured graph) */
 int b200rec_device_timestamp(uint64_t* slot, b200rec_stream_t stream);
